@@ -18,6 +18,8 @@ rank collects its own 2^30-element block, no data-path collective (SURVEY.md §8
             crate itself cannot be built here) on a bounded sample of the same workload
 
 `--impl reference` times that CPU restatement alone, as the reference arm.
+`--dump-outputs DIR` writes a seeded sample of config 2's result after its timed steps, so that two builds can be
+compared output for output (the inputs come from fixed seeds).
 """
 import argparse
 import ctypes as C
@@ -26,6 +28,8 @@ import os
 import sys
 import threading
 import time
+
+sys.dont_write_bytecode = True  # the benchmark writes nothing into the tree it runs from (which may be read-only)
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
@@ -283,6 +287,26 @@ def emit_line(obj):
     os.write(_json_fd if _json_fd is not None else 1, (json.dumps(obj) + "\n").encode())
 
 
+DUMP_SAMPLE = 1 << 21  # over all ranks: 8 MiB of f32 results + 16 MiB of f64 positions
+
+
+def dump_outputs(out_dir, tout, rank, world):
+    """Config 2's result as the last timed collect left it: DIR/zip_map_out.npy (float32) and the positions it was read at,
+    DIR/zip_map_out_index.npy (float64, exact below 2^53).  All of it when it has at most DUMP_SAMPLE / world elements,
+    otherwise that many positions drawn with a fixed seed.  Under torchrun every rank writes its own block, suffixed _rank<r>."""
+    import torch
+    n, k = tout.numel(), DUMP_SAMPLE // world
+    if n <= k:
+        idx = np.arange(n)
+    else:
+        idx = np.unique(np.random.default_rng(0x5EED00D0).integers(0, n, k))
+    got = tout[torch.from_numpy(idx).to(tout.device)].cpu().numpy()
+    suffix = f"_rank{rank}" if world > 1 else ""
+    os.makedirs(out_dir, exist_ok=True)
+    np.save(os.path.join(out_dir, f"zip_map_out{suffix}.npy"), got)
+    np.save(os.path.join(out_dir, f"zip_map_out_index{suffix}.npy"), idx.astype(np.float64))
+
+
 class Bench:
     """What every section needs: the context and its stream, the communicator, timing, buffers."""
 
@@ -353,7 +377,8 @@ def main():
     keep_stdout_for_json()
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=20)
+    ap.add_argument("--steps", type=int, default=20, help="timed steps of every GPU measurement (the 4096x4096 transpose counts "
+                                                          "one pass over its 16 rotating buffers as a step)")
     ap.add_argument("--warmup", type=int, default=3)
     ap.add_argument("--impl", default="b200", choices=["b200", "reference"])
     ap.add_argument("--log2-elems", type=int, default=30, help="elements per GPU (default 2^30 = the BASELINE config)")
@@ -361,7 +386,11 @@ def main():
     ap.add_argument("--no-e2e", action="store_true")
     ap.add_argument("--no-cpu", action="store_true")
     ap.add_argument("--e2e-steps", type=int, default=0)
+    ap.add_argument("--dump-outputs", metavar="DIR", help="after the timed steps, write a seeded sample of config 2's result "
+                                                          "(float32) and its positions (float64) to DIR as .npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     args.warmup = max(args.warmup, 3) if args.impl == "b200" else args.warmup
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
@@ -399,6 +428,8 @@ def main():
     ms_step, launches = B.time_launches(lambda: view.collect(out=st_out, flags=F.COLLECT_ASYNC), args.steps, args.warmup)
     clocks.stop()
     kernel_ran = ctx.last_kernel()
+    if args.dump_outputs:  # before the sections below overwrite tout and ta
+        dump_outputs(args.dump_outputs, tout, rank, world)
     alg_bytes = 12 * n
     per_gpu = alg_bytes / (ms_step * 1e-3) / 1e9
     value = per_gpu * world
@@ -528,7 +559,7 @@ def bench_ops(B, ta, tout):
     torch, ctx, peak, args = B.torch, B.ctx, B.peak, B.args
     dev_array, out_storage, time_launches = B.dev_array, B.out_storage, B.time_launches
     ops = {}
-    steps = max(5, min(args.steps, 20))
+    steps = args.steps
 
     def line(name, alg_bytes, ms, plan, **extra):
         gbs = alg_bytes / (ms * 1e-3) / 1e9
@@ -656,7 +687,7 @@ def bench_scaling_ops(B, ta, tout):
     torch, ctx, comm, world, rank, peak = B.torch, B.ctx, B.comm, B.world, B.rank, B.peak
     dev_array, out_storage, time_launches = B.dev_array, B.out_storage, B.time_launches
     rows = {}
-    steps = 8
+    steps = B.args.steps
 
     def row(name, alg_bytes, ms, n1_ms, kernel, nvlink_in_bytes=0, **extra):
         gbs = alg_bytes / (ms * 1e-3) / 1e9
@@ -725,7 +756,7 @@ def bench_scaling_ops(B, ta, tout):
     src_rep = dev_array(usize, n_src, rep, "f32")
     v_all = dev_array(usize, n3, tidx_all, usize).compose(src_rep)
     p_all = v_all.prepare(out=out_storage(tout[:n3], F.F32), flags=F.COLLECT_ASYNC)
-    n1_ms, _ = time_launches(p_all.run, 5, 2, collective=False)
+    n1_ms, _ = time_launches(p_all.run, steps, 2, collective=False)
     ilo, ihi = sharding.shard_bounds(n3, world, rank)
     tidx = tidx_all[ilo:ihi]
     idx = dev_array(usize, ihi - ilo, tidx, usize)
@@ -735,7 +766,7 @@ def bench_scaling_ops(B, ta, tout):
     p3 = v3.prepare(out=o3, flags=F.COLLECT_ASYNC)
     p3.run(); ctx.sync()
     assert torch.equal(tout[: ihi - ilo], want3), "sharded gather (replicated source) mismatch"
-    ms, _ = time_launches(p3.run, 5, 2)
+    ms, _ = time_launches(p3.run, steps, 2)
     row("c3_compose_source_replicated", 16 * n3, ms, n1_ms, v3.describe(), note="indices and result sharded, 4 GiB source replicated: no exchange")
     if world > 1:
         block = n_src // world
@@ -745,7 +776,7 @@ def bench_scaling_ops(B, ta, tout):
         pp = vp.prepare(out=o3, flags=F.COLLECT_ASYNC)
         pp.run(); ctx.sync()
         assert torch.equal(tout[: ihi - ilo], want3), "peer-mapped gather mismatch"
-        ms_peer, _ = time_launches(pp.run, 5, 2)
+        ms_peer, _ = time_launches(pp.run, steps, 2)
         row("c3_compose_source_sharded_peer_mapped", 16 * n3, ms_peer, n1_ms, vp.describe(), nvlink_in_bytes=4 * (ihi - ilo) * (world - 1) // world,
             note="the gather kernel reads each element from the owning GPU over NVLink (32-byte sectors on the wire)")
         v2 = idx.compose(dev_array(usize, n_src, full_buf, "f32"))
@@ -757,7 +788,7 @@ def bench_scaling_ops(B, ta, tout):
             p2.run()
         ag_then_gather(); ctx.sync()
         assert torch.equal(tout[: ihi - ilo], want3), "all-gather + gather mismatch"
-        ms_ag, _ = time_launches(ag_then_gather, 5, 2)
+        ms_ag, _ = time_launches(ag_then_gather, steps, 2)
         row("c3_compose_source_sharded_allgather_first", 16 * n3, ms_ag, n1_ms, v2.describe(), nvlink_in_bytes=4 * block * (world - 1),
             note="mdim_allgather (NCCL) of the 4 GiB source, then a local gather: the north star's route")
         route = sharding.choose_compose_route(ihi - ilo, 4 * n_src, world)
