@@ -50,11 +50,11 @@ static bool sig_matches(const EvalVariant& v, const char* sig, int sig_len) {
     return true;
 }
 
-int find_static_signature(const char* sig, int sig_len, int slot_bytes, int vec, int vpt, int need_maxr, int wide) {
+int find_static_signature(const char* sig, int sig_len, int slot_bytes, int vec, int need_maxr, int wide) {
     if (wide) return -1;  // signatures are instantiated with 32-bit coordinates only
     const std::vector<EvalVariant>& R = registry();
     for (size_t i = 0; i < R.size(); ++i)
-        if (R[i].slot_bytes == slot_bytes && R[i].vec == vec && R[i].vpt == vpt && R[i].maxr >= need_maxr && !R[i].wide && sig_matches(R[i], sig, sig_len))
+        if (R[i].slot_bytes == slot_bytes && R[i].vec == vec && R[i].maxr >= need_maxr && !R[i].wide && sig_matches(R[i], sig, sig_len))
             return (int)i;
     return -1;
 }
@@ -65,13 +65,13 @@ static const EvalVariant* select_variant(const Plan& p, bool force_interp) {
     const EvalVariant* best = nullptr;
     if (p.static_id >= 0 && !p.wide && !force_interp) {
         for (const EvalVariant& v : R) {
-            if (v.slot_bytes != p.slot_bytes || v.vec != p.vec || v.vpt != p.vpt || v.wide || v.maxr < need || !sig_matches(v, p.sig, p.sig_len)) continue;
+            if (v.slot_bytes != p.slot_bytes || v.vec != p.vec || v.wide || v.maxr < need || !sig_matches(v, p.sig, p.sig_len)) continue;
             if (!best || v.maxr < best->maxr) best = &v;
         }
         if (best) return best;
     }
     for (const EvalVariant& v : R) {
-        if (v.sig || v.slot_bytes != p.slot_bytes || v.vec != p.vec || v.vpt != p.vpt || v.wide != p.wide || v.maxr < need || v.max_depth < p.max_depth) continue;
+        if (v.sig || v.slot_bytes != p.slot_bytes || v.vec != p.vec || v.wide != p.wide || v.maxr < need || v.max_depth < p.max_depth) continue;
         if (!best || v.maxr < best->maxr || (v.maxr == best->maxr && v.max_depth < best->max_depth)) best = &v;
     }
     return best;
@@ -125,20 +125,16 @@ int launch_eval(mdim_ctx* ctx, const Plan& p, void* out, ErrWord* err, bool expl
     if (!(p.flags & (MDIM_COLLECT_NO_STATIC | MDIM_COLLECT_NO_JIT))) jit = jit_kernel_for(p, &jit_level);
     snprintf(ctx->last_kernel, sizeof ctx->last_kernel, "%s", jit ? (jit_level == 2 ? "mdim_jit_kernel[ops+shape]" : "mdim_jit_kernel[ops]") : v->name);
     Program q = p.prog;
-    static const bool no256 = [] { const char* e = getenv("MDIM_NO_VEC256"); return e && e[0] == '1'; }();
-    if (p.vec256_ok && !no256 && ((uintptr_t)out % 32) == 0) q.flags |= PF_VEC256;
+    if (p.vec256_ok && ((uintptr_t)out % 32) == 0) q.flags |= PF_VEC256;
     if (nowait && !explain) q.flags |= PF_NOWAIT;
     if (explain) {
         q.flags |= PF_EXPLAIN;
         q.explain_pos = explain_pos;
-        g0 = explain_pos / ((uint64_t)p.vec * (uint64_t)p.vpt);
+        g0 = explain_pos / (uint64_t)p.vec;
         g1 = g0 + 1;
         grid = 1;
     } else {
-        const uint64_t blocks = (g1 + kEvalThreads - 1) / kEvalThreads;
-        uint64_t cap = 0x7fffffffull;
-        if (ctx->eval_waves > 0) cap = (uint64_t)ctx->sm_count * ctx->eval_ctas_per_sm * ctx->eval_waves;
-        grid = (int)std::min<uint64_t>(blocks, cap);
+        grid = (int)std::min<uint64_t>((g1 + kEvalThreads - 1) / kEvalThreads, 0x7fffffffull);
     }
     if (jit) {
         unsigned long long a0 = g0, a1 = g1;
@@ -161,8 +157,7 @@ int launch_plan(mdim_ctx* ctx, const Plan& p, void* out, ErrWord* err) {
         case KK_TRANSPOSE: {
             // Not persistent: far more CTAs than fit at once, so the hardware scheduler balances the tail.
             // Measured (B200, 16384^2 f32): 8/SM (resident set) 5.71 TB/s, 64/SM 6.18, 128/SM 6.32, one CTA per tile 6.35.
-            const int per_sm = ctx->tr_ctas_cap > 0 ? ctx->tr_ctas_cap : 128;
-            const uint64_t cap = (uint64_t)ctx->sm_count * per_sm;
+            const uint64_t cap = (uint64_t)ctx->sm_count * 128;
             const int grid = (int)std::min<uint64_t>(p.tr.n_tiles, std::max<uint64_t>(cap, 1));
             TransposePlan tr = p.tr;
             tr.nowait = nowait;
@@ -279,18 +274,12 @@ int mdim_init(int device, mdim_ctx** out) {
     ctx->cc_major = prop.major;
     ctx->cc_minor = prop.minor;
     ctx->hbm = prop.totalGlobalMem;
-    ctx->eval_ctas_per_sm = env_int("MDIM_EVAL_CTAS_PER_SM", 8);
-    ctx->eval_waves = env_int("MDIM_EVAL_WAVES", 0);
-    ctx->tr_ctas_cap = env_int("MDIM_TR_CTAS_PER_SM", 0);
     ctx->dep_tracking = env_int("MDIM_DEP_TRACK", 1) != 0;
     ctx->host_chunk_bytes = (size_t)std::max(1, env_int("MDIM_HOST_CHUNK_MB", 128)) << 20;
     bool ok = cudaSetDevice(device) == cudaSuccess && cudaStreamCreateWithFlags(&ctx->own_stream, cudaStreamNonBlocking) == cudaSuccess &&
               cudaMalloc(&ctx->d_err, sizeof(ErrWord) * kErrSlots) == cudaSuccess &&
               cudaMallocHost(&ctx->h_err, sizeof(ErrWord) * kErrSlots) == cudaSuccess;
     if (ok) {
-        // Random gathers fetch whole L2 lines unless the fetch granularity is lowered (a per-device hint).
-        const int l2_fetch = env_int("MDIM_L2_FETCH", 0);
-        if (l2_fetch > 0) cudaDeviceSetLimit(cudaLimitMaxL2FetchGranularity, (size_t)l2_fetch);
         ctx->stream = ctx->own_stream;
         for (int i = 0; i < kErrSlots; ++i) { memset(&ctx->h_err[i], 0, sizeof(ErrWord)); ctx->h_err[i].pos = ~0ull; }
         ok = cudaMemcpy(ctx->d_err, ctx->h_err, sizeof(ErrWord) * kErrSlots, cudaMemcpyHostToDevice) == cudaSuccess;

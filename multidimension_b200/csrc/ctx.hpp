@@ -42,9 +42,6 @@ struct mdim_ctx {
     size_t hbm = 0;
     mdim_error_info last;
     mdim::HostPipe pipe;
-    int eval_ctas_per_sm = 8;
-    int eval_waves = 0;  // 0 = one trip per thread (non-persistent)
-    int tr_ctas_cap = 0;                               // MDIM_TR_CTAS_PER_SM
     uint64_t pos_base = 0;  // applied to collects issued while a host collect is chunking
     // Dependency-aware launches (launch.cuh): byte ranges touched by the kernels launched on own_stream since the last one
     // that waited for its predecessor.  A launch that conflicts with none of them skips the wait.

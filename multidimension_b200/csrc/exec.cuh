@@ -33,9 +33,6 @@
 // specialiser (jit.cu) can instead point it at a `constexpr Program` generated for one concrete shape, which
 // turns every stride into an immediate, drops zero strides and length-1 axes, and makes every divider a
 // compile-time constant.  Pointers, offsets and immediates always come from the real program.
-#ifndef MDIM_STORE_STREAMING
-#define MDIM_STORE_STREAMING true  // st.global.cs (evict-first): nothing re-reads the output
-#endif
 #ifndef MDIM_SHAPE_OF
 #define MDIM_SHAPE_OF(P) (P)
 #endif
@@ -236,7 +233,8 @@ template <class S, int V, bool CACHED> MDIM_FN void ld_vector(const void* base, 
     }
 }
 
-template <class S, int V> MDIM_FN void st_vector(void* base, uint64_t idx, int esize, const S (&d)[V], bool cs, bool w256 = false) {
+// Wide stores are streaming (st.global.cs, evict-first): nothing re-reads the output.
+template <class S, int V> MDIM_FN void st_vector(void* base, uint64_t idx, int esize, const S (&d)[V], bool w256 = false) {
     if constexpr (V * sizeof(S) == 32 && (sizeof(S) == 4 || sizeof(S) == 8)) {
         if (w256 && esize == (int)sizeof(S)) {
             uint32_t r[8];
@@ -247,7 +245,7 @@ template <class S, int V> MDIM_FN void st_vector(void* base, uint64_t idx, int e
 #pragma unroll
                 for (int i = 0; i < 4; ++i) { r[2 * i] = (uint32_t)d[i]; r[2 * i + 1] = (uint32_t)((uint64_t)d[i] >> 32); }
             }
-            st256((char*)base + idx * esize, r, cs);
+            st256((char*)base + idx * esize, r, true);
             return;
         }
     }
@@ -255,7 +253,7 @@ template <class S, int V> MDIM_FN void st_vector(void* base, uint64_t idx, int e
         char* p = (char*)base + idx * 4;
         if constexpr (V % 4 == 0) {
 #pragma unroll
-            for (int i = 0; i < V; i += 4) st128(p + i * 4, (uint32_t)d[i], (uint32_t)d[i + 1], (uint32_t)d[i + 2], (uint32_t)d[i + 3], cs);
+            for (int i = 0; i < V; i += 4) st128(p + i * 4, (uint32_t)d[i], (uint32_t)d[i + 1], (uint32_t)d[i + 2], (uint32_t)d[i + 3], true);
         } else if constexpr (V == 2) {
             st64(p, (uint32_t)d[0], (uint32_t)d[1]);
         } else {
@@ -267,7 +265,7 @@ template <class S, int V> MDIM_FN void st_vector(void* base, uint64_t idx, int e
             if constexpr (V % 2 == 0) {
 #pragma unroll
                 for (int i = 0; i < V; i += 2)
-                    st128(p + i * 8, (uint32_t)d[i], (uint32_t)(d[i] >> 32), (uint32_t)d[i + 1], (uint32_t)(d[i + 1] >> 32), cs);
+                    st128(p + i * 8, (uint32_t)d[i], (uint32_t)(d[i] >> 32), (uint32_t)d[i + 1], (uint32_t)(d[i + 1] >> 32), true);
             } else {
                 st64(p, (uint32_t)d[0], (uint32_t)(d[0] >> 32));
             }
@@ -851,13 +849,13 @@ MDIM_FN uint32_t fast_div(uint32_t n, uint32_t mul, uint32_t shr) {
 // One output vector: decode (Index::from_usize peels the LAST component first, src/index.rs:116-120,
 // src/lib.rs:38-39), evaluate, store at its to_usize position (row-major, src/index.rs:109-114).
 // Program axis 0 is the vector axis, so the decode runs a = 0, 1, ...: dec_len[a] is the decode length
-// of axis a (axis 0 counted in thread trips of V * VPT elements; 1 for reduction / unused axes) and
+// of axis a (axis 0 counted in vectors of V elements; 1 for reduction / unused axes) and
 // dec_scale[a] turns the decoded count back into an element coordinate.
-template <class Sig, class S, int V, int MAXD, bool WIDE, int MAXR, int VPT>
+template <class Sig, class S, int V, int MAXD, bool WIDE, int MAXR>
 MDIM_FN void eval_vector(const Program& P, void* out, ErrWord* err, uint64_t g) {
     using coord_t = typename CoordTraits<WIDE>::coord_t;
     ThreadState<WIDE, MAXR> ts;
-    ts.pos0 = g * (uint64_t)(V * VPT);
+    ts.pos0 = g * (uint64_t)V;
     ts.mask = (1u << V) - 1u;
     ts.red_k = 0;
     ts.rk = 0;
@@ -873,22 +871,14 @@ MDIM_FN void eval_vector(const Program& P, void* out, ErrWord* err, uint64_t g) 
     }
     ts.c[MAXR - 1] = rem * (coord_t)MDIM_SHAPE_OF(P).dec_scale[MAXR - 1];
     S st[MAXD][V];
+    if constexpr (Sig::n > 0) run_static<Sig, 0, 0, Sig::n, S, V, MAXD, WIDE, MAXR>(P, err, st, ts);
+    else run_interp<S, V, MAXD, WIDE, MAXR>(P, err, st, ts);
+    st_vector<S, V>(out, ts.pos0, esize_of(MDIM_SHAPE_OF(P).out_dtype), st[0], (P.flags & PF_VEC256) != 0);
+    if (MDIM_SHAPE_OF(P).n_out > 1) {  // a tuple-typed root: value k of the final stack is scalar leaf k, stored to its own run
 #pragma unroll
-    for (int j = 0; j < VPT; ++j) {  // VPT consecutive vectors along the vector axis share one decode
-        if constexpr (Sig::n > 0) run_static<Sig, 0, 0, Sig::n, S, V, MAXD, WIDE, MAXR>(P, err, st, ts);
-        else run_interp<S, V, MAXD, WIDE, MAXR>(P, err, st, ts);
-        st_vector<S, V>(out, ts.pos0, esize_of(MDIM_SHAPE_OF(P).out_dtype), st[0], MDIM_STORE_STREAMING, (P.flags & PF_VEC256) != 0);
-        if (MDIM_SHAPE_OF(P).n_out > 1) {  // a tuple-typed root: value k of the final stack is scalar leaf k, stored to its own run
-#pragma unroll
-            for (int k = 1; k < MDIM_MAX_OUTS; ++k)
-                if (k < MAXD && k < MDIM_SHAPE_OF(P).n_out)
-                    st_vector<S, V>(P.out_more[k - 1], ts.pos0, esize_of(MDIM_SHAPE_OF(P).out_dtypes[k]), st[k < MAXD ? k : 0], MDIM_STORE_STREAMING, false);
-        }
-        if constexpr (VPT > 1) {
-            ts.c[0] += (coord_t)V;
-            ts.pos0 += (uint64_t)V;
-            ts.mask = (1u << V) - 1u;
-        }
+        for (int k = 1; k < MDIM_MAX_OUTS; ++k)
+            if (k < MAXD && k < MDIM_SHAPE_OF(P).n_out)
+                st_vector<S, V>(P.out_more[k - 1], ts.pos0, esize_of(MDIM_SHAPE_OF(P).out_dtypes[k]), st[k < MAXD ? k : 0]);
     }
 }
 

@@ -7,12 +7,10 @@ namespace mdim {
 template <class Sig> constexpr const SigInstr* sig_code() { if constexpr (Sig::n > 0) return Sig::code; else return nullptr; }
 
 static const EvalVariant kVariants[] = {
-#define X4(Sig, S, V, MAXD, WIDE, MAXR, VPT) \
-    {#Sig, (int)sizeof(S), V, MAXD, WIDE ? 1 : 0, MAXR, VPT, sig_code<Sig>(), Sig::n, &k_eval<Sig, S, V, MAXD, WIDE, MAXR, VPT>},
-#define X(Sig, S, V, MAXD, WIDE, MAXR) X4(Sig, S, V, MAXD, WIDE, MAXR, 1)
+#define X(Sig, S, V, MAXD, WIDE, MAXR) \
+    {#Sig, (int)sizeof(S), V, MAXD, WIDE ? 1 : 0, MAXR, sig_code<Sig>(), Sig::n, &k_eval<Sig, S, V, MAXD, WIDE, MAXR>},
 #include "variants_s64_interp.inc"
 #undef X
-#undef X4
 };
 
 const EvalVariant* eval_variants_s64_interp(int* n) {

@@ -335,8 +335,6 @@ template <bool FAST> static bool launch_regs(const FoldRowsPlan& R, void* out, c
 }  // namespace
 
 const char* launch_fold_rows(const FoldRowsPlan& R, void* out, int sm_count, cudaStream_t stream) {
-    static const int env_warps = [] { const char* e = getenv("MDIM_FOLD_WARPS"); return e ? atoi(e) : 0; }();
-    static const int env_stages = [] { const char* e = getenv("MDIM_FOLD_STAGES"); return e ? atoi(e) : 0; }();
     // column chunk: the whole row when a 32-row tile of it fits 64 KB (and always for the fused form,
     // which needs the whole row resident); else 256 columns per item
     int ch = (int)R.row_len;
@@ -347,20 +345,14 @@ const char* launch_fold_rows(const FoldRowsPlan& R, void* out, int sm_count, cud
     if (max_tiles < 1) max_tiles = 1;
     // Measured on B200 (profiles/): warps hide each other's latency better than stages do — six warps with
     // one tile each beat three warps with two — so fill the warps first, then deepen the rings.
-    const int max_warps = kFoldThreads / 32;
-    int n_warps = env_warps > 0 ? env_warps : std::min(max_warps, max_tiles);
-    if (n_warps > max_warps) n_warps = max_warps;
-    if (n_warps > max_tiles) n_warps = max_tiles;
-    int stages = env_stages > 0 ? env_stages : std::min(8, std::min(4, max_tiles / n_warps));
-    if (stages * n_warps > max_tiles) stages = max_tiles / n_warps;
-    if (stages < 1) stages = 1;
+    const int n_warps = std::min(kFoldThreads / 32, max_tiles);
+    const int stages = std::min(4, max_tiles / n_warps);
     const size_t smem = kBarBytes + (size_t)n_warps * stages * tile_bytes;
     const uint64_t n_blocks = (R.n_rows + kRowsPerTile - 1) / kRowsPerTile;
     // Not one resident CTA per SM but up to 16 queued per SM (each warp then folds ~2 tiles): the hardware scheduler
     // evens out the tail.  Measured on B200, config 4a: 6 724 GB/s (x1) -> 6 892 (x4) -> 7 047 (x16) -> 6 983 (x64);
     // a pure read stream reaches 7 570 (scripts/probe/read_bw.cu).
-    static const int grid_mult = [] { const char* e = getenv("MDIM_FOLD_GRID_MULT"); return e && atoi(e) > 0 ? atoi(e) : 16; }();
-    int grid = (int)std::min<uint64_t>((n_blocks + n_warps - 1) / n_warps, (uint64_t)sm_count * grid_mult);
+    int grid = (int)std::min<uint64_t>((n_blocks + n_warps - 1) / n_warps, (uint64_t)sm_count * 16);
     if (grid < 1) grid = 1;
     // bank-conflict-free skew needs the dense row pitch to be a multiple of 8 sixteen-byte chunks
     const int skew = ((ch / 4) % 8 == 0) ? 1 : 0;

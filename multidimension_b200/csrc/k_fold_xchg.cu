@@ -21,7 +21,6 @@
 // Every CTA of the grid is co-resident (grid <= occupancy x SMs), so waiting on peers cannot starve a CTA that has not run.
 // Spins are bounded (~2 s): a rank that never arrives becomes MDIM_ERR_NCCL on the others, not a hung GPU.
 #include <cuda.h>
-#include <stdlib.h>
 #include <string.h>
 
 #include <algorithm>
@@ -294,9 +293,8 @@ template <bool EXCHANGE> XchgKernel pick_kernel(int dtype, int op) {
 int launch_fold_xchg(const FoldXchgArgs& A, int dtype, int op, int sm_count, cudaStream_t stream) {
     if (((uintptr_t)A.rows & 15) || (A.pitch_bytes & 15) || (A.row_bytes & 15) || ((uintptr_t)A.out & 15) || !A.n_rows || !A.row_bytes) return -1;
     FoldXchgArgs B = A;
-    // two ranks: one hop; more: owners (two hops, 2 (N-1)/N rows per GPU over NVLink instead of N-1).  MDIM_XCHG_ONE_SHOT=0/1 forces either.
-    static const int forced = [] { const char* e = getenv("MDIM_XCHG_ONE_SHOT"); return e ? atoi(e) : -1; }();
-    B.one_shot = forced >= 0 ? forced : (A.world <= 2);
+    // two ranks: one hop; more: owners (two hops, 2 (N-1)/N rows per GPU over NVLink instead of N-1)
+    B.one_shot = A.world <= 2;
     B.wide = !(((uintptr_t)A.rows & 31) || (A.pitch_bytes & 31));
     XchgKernel fn = pick_kernel<true>(dtype, op);
     if (!fn) return -1;

@@ -6,8 +6,8 @@
 //
 //   out[batch, a, b]  (b has out stride 1)   =   src[batch', b, a]  (a has src stride 1)
 //
-// One CTA moves one tile of TB B-rows x TAC chunks (16 bytes each) of A; the default is 64 rows x 16 chunks, i.e.
-// 64x64 4-byte or 64x32 8-byte elements, 16 KB of shared memory, both global directions 128-bit and coalesced:
+// One CTA moves one tile of TB = 64 B-rows x TAC = 16 chunks (16 bytes each) of A, i.e. 64x64 4-byte or 64x32 8-byte
+// elements, 16 KB of shared memory, both global directions 128-bit and coalesced:
 //   load : each thread reads 16 B along A (a warp covers 2 source rows x 256 B) and writes them
 //          with ONE 16-byte shared store at row b, chunk (a_chunk ^ swz(b));
 //   store: each thread assembles 16 B along B from CH scalar shared loads (one per source row) and
@@ -29,7 +29,7 @@ namespace mdim {
 // Resident CTAs per SM the register allocation aims for.  6 (40 registers) lets all four loads of a thread issue before
 // the first shared store; with 8 (32 registers) they go out two at a time.  Measured at 4096^2 on rotating buffers:
 // 8 -> 5 675 GB/s, 7 -> same code as 8, 6 -> 5 750, 5 -> 5 646.
-constexpr int tr_min_ctas(int smem_bytes) { return 227 * 1024 / (smem_bytes + 1024) > 6 ? 6 : 227 * 1024 / (smem_bytes + 1024); }
+constexpr int kTrMinCtas = 6;
 
 // Address of element `e` of the source.  PEER: the Array is cut into equal blocks of peer_block elements, block p in
 // the HBM of GPU p (mapped into this process with CUDA IPC); the owner is e / peer_block, estimated in f32 and
@@ -46,8 +46,9 @@ __device__ __forceinline__ const char* tr_src(const TransposePlan& T, int64_t e)
     }
 }
 
-template <int ES, bool VEC, int TAC, int TB, bool PEER>
-__global__ void __launch_bounds__(kTrThreads, tr_min_ctas(TB * TAC * 16)) k_transpose(const __grid_constant__ TransposePlan T, void* __restrict__ out_v) {
+template <int ES, bool VEC, bool PEER>
+__global__ void __launch_bounds__(kTrThreads, kTrMinCtas) k_transpose(const __grid_constant__ TransposePlan T, void* __restrict__ out_v) {
+    constexpr int TAC = kTrTileChunks, TB = kTrTileRows;
     constexpr int CH = 16 / ES;            // elements per 16-byte chunk
     constexpr int EW = ES / 4;             // 32-bit words per element
     constexpr int TA = TAC * CH;           // tile extent along A (elements); TAC chunks = TAC*16 bytes per source run
@@ -70,18 +71,11 @@ __global__ void __launch_bounds__(kTrThreads, tr_min_ctas(TB * TAC * 16)) k_tran
     const int bq_lo = lane & 7, a_lo = lane >> 3;
 
     for (uint64_t tile = blockIdx.x; tile < T.n_tiles; tile += gridDim.x) {
-        uint64_t ta, tb, batch;
-        if (T.a_fastest) {  // neighbouring CTAs read neighbouring pieces of the same source rows
-            ta = tile % T.tiles_a;
-            const uint64_t r = tile / T.tiles_a;
-            tb = r % T.tiles_b;
-            batch = r / T.tiles_b;
-        } else {            // neighbouring CTAs write neighbouring pieces of the same output rows
-            tb = tile % T.tiles_b;
-            const uint64_t r = tile / T.tiles_b;
-            ta = r % T.tiles_a;
-            batch = r / T.tiles_a;
-        }
+        // neighbouring CTAs write neighbouring pieces of the same output rows
+        const uint64_t tb = tile % T.tiles_b;
+        const uint64_t r = tile / T.tiles_b;
+        const uint64_t ta = r % T.tiles_a;
+        uint64_t batch = r / T.tiles_a;
         int64_t src_base = T.src_offset, out_base = 0;
 #pragma unroll
         for (int k = kMaxRank - 1; k >= 0; --k) {
@@ -162,102 +156,6 @@ __global__ void __launch_bounds__(kTrThreads, tr_min_ctas(TB * TAC * 16)) k_tran
         }
         __syncthreads();
     }
-}
-
-// ---- pipelined form (aligned operands): cp.async multi-stage ring ------------------------------------
-// Same tile geometry and swizzle as above, but the global -> shared leg is `cp.async.cg` (16 bytes per
-// request, straight into its swizzled slot, no registers) issued kStages-1 tiles ahead, so every CTA
-// keeps 32 KB of loads in flight while it drains the current tile; one __syncthreads per tile.
-constexpr int kTrStages = 3;
-
-__device__ __forceinline__ void cp_async16(void* smem_dst, const void* gmem_src, bool valid) {
-    const uint32_t d = (uint32_t)__cvta_generic_to_shared(smem_dst);
-    const int n = valid ? 16 : 0;  // src-size 0: the slot is zero-filled and the source is not read
-    asm volatile("cp.async.cg.shared.global [%0], [%1], 16, %2;" ::"r"(d), "l"(gmem_src), "r"(n) : "memory");
-}
-
-template <int ES>
-__global__ void __launch_bounds__(kTrThreads) k_transpose_pipe(const __grid_constant__ TransposePlan T, void* __restrict__ out_v) {
-    constexpr int CH = 16 / ES, EW = ES / 4, TA = 16 * CH, TB = 64, PA = TA / 32;
-    extern __shared__ __align__(16) uint32_t ring[];  // kTrStages x (TB x 64 words)
-    pdl_entry(T.nowait != 0);
-    const char* __restrict__ src = (const char*)T.src;
-    char* __restrict__ out = (char*)out_v;
-    const int tid = threadIdx.x;
-    const int aq = tid & 15, br = tid >> 4;
-    const int lane = tid & 31, w = tid >> 5;
-    const int bq_lo = lane & 7, a_lo = lane >> 3;
-
-    auto locate = [&](uint64_t tile, int64_t& src_base, int64_t& out_base, uint64_t& a0, uint64_t& b0) {
-        const uint64_t tb = tile % T.tiles_b;
-        uint64_t r = tile / T.tiles_b;
-        const uint64_t ta = r % T.tiles_a;
-        uint64_t batch = r / T.tiles_a;
-        src_base = T.src_offset; out_base = 0;
-#pragma unroll
-        for (int k = kMaxRank - 1; k >= 0; --k) {
-            if (k < T.n_batch) {
-                const uint64_t c = batch % T.batch_len[k];
-                batch /= T.batch_len[k];
-                src_base += (int64_t)c * T.batch_src_stride[k];
-                out_base += (int64_t)c * T.batch_out_stride[k];
-            }
-        }
-        a0 = ta * TA; b0 = tb * TB;
-    };
-    auto issue = [&](uint64_t tile, int stage) {
-        int64_t src_base, out_base; uint64_t a0, b0;
-        locate(tile, src_base, out_base, a0, b0);
-        uint32_t* sm = ring + stage * (TB * 64);
-#pragma unroll
-        for (int p = 0; p < 4; ++p) {
-            const int b_l = p * 16 + br;
-            const uint64_t b = b0 + b_l, a = a0 + (uint64_t)aq * CH;
-            const bool valid = b < T.len_b && a < T.len_a;
-            const int64_t e = valid ? src_base + (int64_t)b * T.src_stride_b + (int64_t)a : T.src_offset;
-            const int chunk = aq ^ ((b_l / CH) & 7);
-            cp_async16(sm + b_l * 64 + chunk * 4, src + e * ES, valid);
-        }
-    };
-
-    const uint64_t stride = gridDim.x;
-    uint64_t next = blockIdx.x;  // next tile to issue
-#pragma unroll
-    for (int s = 0; s < kTrStages - 1; ++s) {
-        if (next < T.n_tiles) issue(next, s);
-        asm volatile("cp.async.commit_group;" ::: "memory");
-        next += stride;
-    }
-    int it = 0;
-    for (uint64_t tile = blockIdx.x; tile < T.n_tiles; tile += stride, ++it) {
-        asm volatile("cp.async.wait_group %0;" ::"n"(kTrStages - 2) : "memory");
-        __syncthreads();  // tile `it` has landed for every thread, and stage (it-1) % kTrStages is drained
-        if (next < T.n_tiles) issue(next, (it + kTrStages - 1) % kTrStages);
-        asm volatile("cp.async.commit_group;" ::: "memory");
-        next += stride;
-
-        int64_t src_base, out_base; uint64_t a0, b0;
-        locate(tile, src_base, out_base, a0, b0);
-        const uint32_t* smem = ring + (it % kTrStages) * (TB * 64);
-#pragma unroll
-        for (int p = 0; p < 4; ++p) {
-            const int a_l = 4 * (w + 8 * (p % PA)) + a_lo;
-            const int bq = bq_lo + 8 * (p / PA);
-            uint32_t wds[4];
-#pragma unroll
-            for (int i = 0; i < CH; ++i) {
-                const int b_l = bq * CH + i;
-                const int word = b_l * 64 + (((a_l / CH) ^ (bq & 7)) * 4) + (a_l % CH) * EW;
-                if constexpr (ES == 4) wds[i] = smem[word];
-                else { const uint2 t = *reinterpret_cast<const uint2*>(&smem[word]); wds[2 * i] = t.x; wds[2 * i + 1] = t.y; }
-            }
-            const uint64_t a = a0 + a_l, b = b0 + (uint64_t)bq * CH;
-            const int64_t e = out_base + (int64_t)a * T.out_stride_a + (int64_t)b;
-            if (a < T.len_a && b < T.len_b)
-                asm volatile("st.global.cs.v4.u32 [%0], {%1,%2,%3,%4};" ::"l"(out + e * ES), "r"(wds[0]), "r"(wds[1]), "r"(wds[2]), "r"(wds[3]) : "memory");
-        }
-    }
-    asm volatile("cp.async.wait_group 0;" ::: "memory");
 }
 
 // ---- tensor-map TMA form (round 2) ---------------------------------------------------------------------------------
@@ -399,26 +297,19 @@ static bool transpose_vec_ok(const TransposePlan& T, const void* out) {
     return vec;
 }
 
-// Measured on B200 (round 1): the cp.async ring is SLOWER than the plain register-staged kernel at 8 CTAs/SM
-// (5.30 vs 5.61 TB/s at 16384^2), so it is opt-in.
-static bool use_pipe() {
-    static const bool on = [] { const char* e = getenv("MDIM_TR_PIPE"); return e && e[0] == '1'; }();
-    return on;
-}
-
-template <int ES, bool VEC, int TAC, int TB, bool PEER>
+template <int ES, bool VEC, bool PEER>
 static void launch_tr1(const TransposePlan& T, void* out, int grid, cudaStream_t stream) {
-    constexpr int smem = TB * TAC * 16;
-    static const bool once = [] { return cudaFuncSetAttribute(k_transpose<ES, VEC, TAC, TB, PEER>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem) == cudaSuccess; }();
+    constexpr int smem = kTrTileRows * kTrTileChunks * 16;
+    static const bool once = [] { return cudaFuncSetAttribute(k_transpose<ES, VEC, PEER>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem) == cudaSuccess; }();
     (void)once;
-    launch_pdl(k_transpose<ES, VEC, TAC, TB, PEER>, dim3(grid), dim3(kTrThreads), smem, stream, T, out);
+    launch_pdl(k_transpose<ES, VEC, PEER>, dim3(grid), dim3(kTrThreads), smem, stream, T, out);
 }
 
-template <int ES, int TAC, int TB>
+template <int ES>
 static void launch_tr(const TransposePlan& T, void* out, int grid, bool vec, cudaStream_t stream) {
     const bool peer = T.n_peers > 1;
-    if (vec) { if (peer) launch_tr1<ES, true, TAC, TB, true>(T, out, grid, stream); else launch_tr1<ES, true, TAC, TB, false>(T, out, grid, stream); }
-    else { if (peer) launch_tr1<ES, false, TAC, TB, true>(T, out, grid, stream); else launch_tr1<ES, false, TAC, TB, false>(T, out, grid, stream); }
+    if (vec) { if (peer) launch_tr1<ES, true, true>(T, out, grid, stream); else launch_tr1<ES, true, false>(T, out, grid, stream); }
+    else { if (peer) launch_tr1<ES, false, true>(T, out, grid, stream); else launch_tr1<ES, false, false>(T, out, grid, stream); }
 }
 
 // ---- host side of the TMA form ---------------------------------------------------------------------------------------
@@ -482,9 +373,8 @@ static bool launch_transpose_tma(const TransposePlan& T, void* out, cudaStream_t
     for (int k = 0; k < T.n_batch; ++k) { n_tiles *= T.batch_len[k]; A.batch_len[k] = (uint32_t)T.batch_len[k]; }
     if (n_tiles == 0 || n_tiles > 0x7fffffffull) return false;
     A.tiles_a = (uint32_t)tiles_a; A.tiles_b = (uint32_t)tiles_b; A.n_tiles = (uint32_t)n_tiles; A.n_batch = T.n_batch; A.nowait = T.nowait;
-    // tile order: A-fastest measured +2.5 % at 4096^2 and -0.5 % at 16384^2 (profiles/r2_tr_tma_probe.md); MDIM_TR_ORDER overrides
-    const char* ord = getenv("MDIM_TR_ORDER");
-    A.a_fastest = ord ? atoi(ord) : (2 * T.len_a * T.len_b * (uint64_t)es <= (512ull << 20) ? 1 : 0);
+    // tile order: A-fastest measured +2.5 % at 4096^2 and -0.5 % at 16384^2 (profiles/r2_tr_tma_probe.md)
+    A.a_fastest = 2 * T.len_a * T.len_b * (uint64_t)es <= (512ull << 20) ? 1 : 0;
     CUtensorMap dm;
     if (!tma_encode(&dm, out, es, T.len_b, T.len_a, T.out_stride_a, T.n_batch, T.batch_len, T.batch_out_stride)) return false;
     if (T.n_peers > 1) {
@@ -507,29 +397,12 @@ static bool launch_transpose_tma(const TransposePlan& T, void* out, cudaStream_t
     return es == 4 ? launch_tma1<4, 1>(sm, dm, A, stream) : launch_tma1<8, 1>(sm, dm, A, stream);
 }
 
-// Tile shapes the planner may ask for (TransposePlan::tile_ac x tile_b).  16 chunks x 64 rows (16 KB, 256-byte runs
-// both ways) is the default; 32 x 128 (64 KB, 512-byte runs) is kept for MDIM_TR_TILE=32x128 experiments — measured
-// equal at 16384^2 (6.31 vs 6.32 TB/s) and slower at 4096^2 (5.25 vs 5.67), as are 32 x 64 and 16 x 128 (5.1 TB/s).
-#define MDIM_TR_SHAPES(X) X(16, 64) X(32, 128)
-
 const char* launch_transpose(const TransposePlan& T, void* out, int grid, cudaStream_t stream) {
     if (launch_transpose_tma(T, out, stream)) return T.n_peers > 1 ? "k_transpose_tma<peer>" : "k_transpose_tma";
     const bool vec = transpose_vec_ok(T, out);
-    if (vec && use_pipe() && T.tile_ac == 16 && T.tile_b == 64 && T.n_peers <= 1) {
-        constexpr int smem = kTrStages * 64 * 64 * 4;
-        if (T.esize == 4) launch_pdl(k_transpose_pipe<4>, dim3(grid), dim3(kTrThreads), smem, stream, T, out);
-        else launch_pdl(k_transpose_pipe<8>, dim3(grid), dim3(kTrThreads), smem, stream, T, out);
-        return "k_transpose_pipe";
-    }
-#define X(AC, B)                                                                      \
-    if (T.tile_ac == AC && T.tile_b == B) {                                           \
-        if (T.esize == 4) launch_tr<4, AC, B>(T, out, grid, vec, stream);             \
-        else launch_tr<8, AC, B>(T, out, grid, vec, stream);                          \
-        return vec ? "k_transpose<regs,vec>" : "k_transpose<regs,scalar>";            \
-    }
-    MDIM_TR_SHAPES(X)
-#undef X
-    return "k_transpose<none>";
+    if (T.esize == 4) launch_tr<4>(T, out, grid, vec, stream);
+    else launch_tr<8>(T, out, grid, vec, stream);
+    return vec ? "k_transpose<regs,vec>" : "k_transpose<regs,scalar>";
 }
 
 }  // namespace mdim

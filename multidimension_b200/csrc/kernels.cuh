@@ -12,17 +12,17 @@ constexpr int kEvalThreads = 256;
 
 // ------------------------------------------------------------------------------------------------
 // K1 / K3 / K5: the rank-N fused evaluator.  One thread = one output vector per loop trip; the
-// grid is either one trip per thread or a persistent multiple of the SM count (tunable).
+// grid has one thread per vector (more trips only past 2^31 - 1 CTAs).
 // All operands are read-only and never alias `out` (C-ABI contract), so loads use the
 // non-coherent path; stores are streaming (evict-first) because nothing re-reads the output.
 // ------------------------------------------------------------------------------------------------
-template <class Sig, class S, int V, int MAXD, bool WIDE, int MAXR, int VPT>
+template <class Sig, class S, int V, int MAXD, bool WIDE, int MAXR>
 __global__ void __launch_bounds__(kEvalThreads)
 k_eval(const __grid_constant__ Program P, void* __restrict__ out, ErrWord* __restrict__ err, uint64_t g_begin, uint64_t g_end) {
     pdl_entry((P.flags & PF_NOWAIT) != 0);
     const uint64_t step = (uint64_t)gridDim.x * kEvalThreads;
     for (uint64_t g = g_begin + (uint64_t)blockIdx.x * kEvalThreads + threadIdx.x; g < g_end; g += step)
-        eval_vector<Sig, S, V, MAXD, WIDE, MAXR, VPT>(P, out, err, g);
+        eval_vector<Sig, S, V, MAXD, WIDE, MAXR>(P, out, err, g);
 }
 
 using EvalKernel = void (*)(const Program, void*, ErrWord*, uint64_t, uint64_t);
@@ -30,7 +30,6 @@ using EvalKernel = void (*)(const Program, void*, ErrWord*, uint64_t, uint64_t);
 struct EvalVariant {
     const char* name;
     int slot_bytes, vec, max_depth, wide, maxr;  // maxr: iteration axes walked (1 = contiguous stream)
-    int vpt;                                     // vectors per thread trip
     const SigInstr* sig;  // nullptr = interpreter
     int sig_n;
     EvalKernel fn;

@@ -85,7 +85,6 @@ struct Builder {
     int64_t cstride[MDIM_MAX_NODES][kMaxRank];
     int depth = 0, max_depth = 0;
     int force_vec = 0;
-    bool no_vpt = false;
     // canonical axis g (out axes outermost-first, then reduction axes) -> device program axis:
     // the out axes are stored INNERMOST FIRST, so the vector axis is always program axis 0
     int pa(int g) const { return g < rank ? rank - 1 - g : g; }  // 0 = widest that divides the innermost axis
@@ -499,36 +498,26 @@ int Builder::emit() {
         if (e->nodes[i].kind == MDIM_NODE_IOTA && dtype_size(e->nodes[i].dtype) == 8) slot = 8;
     }
     plan->slot_bytes = slot;
-    // vector width along the innermost output axis
+    // vector width along the innermost output axis: the widest of at most 32 bytes that divides it
     int V = 1;
     if (rank > 0) {
         const int cand32[3] = {8, 4, 1}, cand64[3] = {4, 2, 1};
         const int* cand = slot == 4 ? cand32 : cand64;
-        static const int max_bytes = [] { const char* e = getenv("MDIM_MAX_VEC_BYTES"); return e ? atoi(e) : 32; }();
         for (int i = 0; i < 3; ++i)
-            if (cand[i] * slot <= max_bytes && len[rank - 1] % (uint64_t)cand[i] == 0) { V = cand[i]; break; }
+            if (len[rank - 1] % (uint64_t)cand[i] == 0) { V = cand[i]; break; }
     }
     // A fold walks its reduction axes sequentially inside one thread, so the output is the only source of
     // parallelism: prefer narrower vectors until there are enough threads to fill the machine.
     if (fold_node >= 0 && rank > 0) {
         const int cand32[3] = {8, 4, 1}, cand64[3] = {4, 2, 1};
         const int* cand = slot == 4 ? cand32 : cand64;
-        static const uint64_t min_threads = [] { const char* e = getenv("MDIM_FOLD_MIN_THREADS"); return e ? (uint64_t)atoll(e) : 40000ull; }();  // measured: 64 Ki threads x 16 B beat 256 Ki x 4 B and 32 Ki x 32 B
+        const uint64_t min_threads = 40000;  // measured: 64 Ki threads x 16 B beat 256 Ki x 4 B and 32 Ki x 32 B
         for (int i = 0; i < 3 && out_elems / (uint64_t)V < min_threads; ++i)
             if (cand[i] < V && len[rank - 1] % (uint64_t)cand[i] == 0) V = cand[i];
     }
     if (force_vec) V = force_vec;
-    // Vectors per thread trip along the vector axis.  Measured on B200 (round 1): 4 consecutive vectors per
-    // thread halve the throughput of rank-N chains (lanes 128 B apart: every warp instruction touches 32
-    // separate lines), so coalescing wins over amortising the decode; the machinery stays for experiments.
-    int VPT = 1;
-    if (rank >= 2 && V > 1 && !force_vec && !no_vpt && !(flags & MDIM_COLLECT_NO_STATIC) && getenv("MDIM_VPT4")) {
-        const uint64_t inner_vecs = len[rank - 1] / (uint64_t)V;
-        if (inner_vecs % 4 == 0 && out_elems / ((uint64_t)V * 4) >= (1ull << 16)) VPT = 4;
-    }
-    plan->vpt = VPT; P.vpt = VPT;
     plan->vec = V; P.vec = V;
-    P.n_vec = out_elems / ((uint64_t)V * (uint64_t)VPT);  // work items: one per thread trip
+    P.n_vec = out_elems / (uint64_t)V;  // work items: one per thread trip
 
     // 32-bit coordinate path needs: vectors < 2^31, every axis < 2^31, every stride in int32
     bool wide = P.n_vec >= (1ull << 31);
@@ -551,10 +540,10 @@ int Builder::emit() {
     plan->n_axes = n_axes;
     for (int g = 0; g < kMaxRank; ++g) {
         uint64_t L = 1;
-        if (g < rank) L = (g == rank - 1) ? len[g] / ((uint64_t)V * (uint64_t)VPT) : len[g];
+        if (g < rank) L = (g == rank - 1) ? len[g] / (uint64_t)V : len[g];
         const int a = g < n_axes ? pa(g) : g;
         P.dec_len[a] = L;
-        P.dec_scale[a] = (g == rank - 1) ? (uint32_t)(V * VPT) : 1u;
+        P.dec_scale[a] = (g == rank - 1) ? (uint32_t)V : 1u;
         find_divisor((uint32_t)std::min<uint64_t>(L, 0x7fffffffull), &P.div_mul[a], &P.div_shr[a]);
     }
     depth = 0; max_depth = 0;
@@ -613,19 +602,12 @@ int Builder::detect_fast_paths() {
                 T.batch_out_stride[T.n_batch] = ostride[g];
                 T.n_batch++;
             }
-            // tile shape: MDIM_TR_TILE="<chunks along A>x<rows>" overrides the default (see k_transpose.cu)
-            T.tile_ac = 16; T.tile_b = 64;
-            if (const char* ts = getenv("MDIM_TR_TILE")) {
-                int ac = 0, tb = 0;
-                if (sscanf(ts, "%dx%d", &ac, &tb) == 2 && ((ac == 16 && tb == 64) || (ac == 32 && tb == 128))) { T.tile_ac = ac; T.tile_b = tb; }
-            }
-            const uint64_t tile_a = (uint64_t)T.tile_ac * 16 / (uint64_t)es;
-            T.tiles_a = (T.len_a + tile_a - 1) / tile_a; T.tiles_b = (T.len_b + T.tile_b - 1) / T.tile_b;
+            const uint64_t tile_a = (uint64_t)kTrTileChunks * 16 / (uint64_t)es;
+            T.tiles_a = (T.len_a + tile_a - 1) / tile_a; T.tiles_b = (T.len_b + kTrTileRows - 1) / kTrTileRows;
             uint64_t nb = 1; for (int b = 0; b < T.n_batch; ++b) nb *= T.batch_len[b];
             T.n_tiles = T.tiles_a * T.tiles_b * nb;
-            { const char* ord = getenv("MDIM_TR_ORDER"); T.a_fastest = ord ? atoi(ord) : 0; }
             plan->kind = KK_TRANSPOSE;
-            snprintf(plan->describe, sizeof plan->describe, "transpose.tile%dx%d%s es%d a=%llu b=%llu batch=%llu", (int)tile_a, T.tile_b, T.n_peers > 1 ? ".peers" : "", es,
+            snprintf(plan->describe, sizeof plan->describe, "transpose.tile%dx%d%s es%d a=%llu b=%llu batch=%llu", (int)tile_a, kTrTileRows, T.n_peers > 1 ? ".peers" : "", es,
                      (unsigned long long)T.len_a, (unsigned long long)T.len_b, (unsigned long long)nb);
             return MDIM_OK;
         }
@@ -789,16 +771,9 @@ int plan_expr(const mdim_expr* e, uint32_t flags, Plan* plan, char* why_buf, siz
     plan->kind = (b->rank <= 1 && b->red_rank == 0) ? KK_STREAM : KK_GENERIC;
     const int need_maxr = plan->kind == KK_STREAM ? 1 : std::max(1, plan->n_axes);
     if (!(flags & MDIM_COLLECT_NO_STATIC))
-        plan->static_id = find_static_signature(plan->sig, plan->sig_len, plan->slot_bytes, plan->vec, plan->vpt, need_maxr, plan->wide);
-    if (plan->vpt > 1 && plan->static_id < 0) {  // several vectors per trip exist only as pre-instantiated signatures
-        b->no_vpt = true;
-        st = b->emit();
-        if (st) { delete b; return st; }
-        if (!(flags & MDIM_COLLECT_NO_STATIC))
-            plan->static_id = find_static_signature(plan->sig, plan->sig_len, plan->slot_bytes, plan->vec, plan->vpt, need_maxr, plan->wide);
-    }
-    snprintf(plan->describe, sizeof plan->describe, "%s.%s s%d v%dx%d%s rank=%d+%d depth=%d instr=%d",
-             plan->kind == KK_STREAM ? "stream" : "generic", plan->static_id >= 0 ? "static" : "interp", plan->slot_bytes * 8, plan->vec, plan->vpt,
+        plan->static_id = find_static_signature(plan->sig, plan->sig_len, plan->slot_bytes, plan->vec, need_maxr, plan->wide);
+    snprintf(plan->describe, sizeof plan->describe, "%s.%s s%d v%dx1%s rank=%d+%d depth=%d instr=%d",
+             plan->kind == KK_STREAM ? "stream" : "generic", plan->static_id >= 0 ? "static" : "interp", plan->slot_bytes * 8, plan->vec,
              plan->wide ? " wide" : "", b->rank, b->red_rank, plan->max_depth, plan->prog.n_instr);
     if (!(flags & MDIM_COLLECT_NO_FASTPATH)) {
         st = b->detect_fast_paths();

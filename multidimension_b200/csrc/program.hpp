@@ -92,8 +92,7 @@ struct Program {
     int32_t out_dtypes[MDIM_MAX_OUTS];
     void* out_more[MDIM_MAX_OUTS - 1];  // run-time: the output runs 1.. (run 0 is the kernel's `out` argument)
     int32_t vec;  // lanes per vector along the innermost output axis (program axis 0)
-    int32_t vpt;  // consecutive vectors per thread trip along that axis
-    int32_t pad0;
+    int32_t pad0; // keeps length[] and the fields after it at their offsets (moved, the evaluators compile one constant load differently)
     uint32_t flags;
     uint64_t length[kMaxRank];  // coalesced lengths: out axes then reduction axes (elements)
     uint64_t dec_len[kMaxRank];   // decode length of axis a: innermost out axis in vectors; 1 if not an out axis
@@ -128,6 +127,11 @@ enum KernelKind : int32_t {
     KK_FOLD_COLS = 5,  // sequential fold over an OUTER axis of one leaf whose result is contiguous: a column walk (k_fold_cols)
 };
 
+// The register-staged transpose's tile (k_transpose.cu): 16-byte chunks along A x source rows, 256-byte runs both ways.
+// Measured on B200: 32 x 128 equal at 16384^2 (6.31 vs 6.32 TB/s) and slower at 4096^2 (5.25 vs 5.67), as were 32 x 64
+// and 16 x 128 (5.1 TB/s).
+constexpr int kTrTileChunks = 16, kTrTileRows = 64;
+
 struct TransposePlan {
     const void* src;
     int32_t esize;
@@ -142,8 +146,6 @@ struct TransposePlan {
     int64_t src_stride_b;        // source stride along B (A has source stride 1)
     int64_t out_stride_a;        // out stride along A (B has out stride 1)
     uint64_t tiles_a, tiles_b, n_tiles;
-    int32_t tile_ac, tile_b;     // tile shape: 16-byte chunks along A (source run = 16*tile_ac bytes) x source rows
-    int32_t a_fastest;           // tile order: 1 = consecutive tiles advance along A (source-contiguous) first
     // Source sharded over peer GPUs (mdim_node.n_peers on the LEAF): element e of the whole Array lives at
     // peer[e / peer_block] + (e % peer_block).  The kernel reads the owning peer's HBM over NVLink, so the
     // all-to-all a row-sharded transpose implies happens inside the tile loads.
@@ -168,7 +170,6 @@ struct FoldRowsPlan {
     int32_t post_op;      // optional binary op applied to the fold before the epilogue (e.g. DIV)
     int32_t has_post;
     uint64_t post_imm;    // ... with this constant on the right
-    int32_t rows_per_cta;
     int32_t nowait;       // set per launch (api.cu): see launch.cuh
 };
 
@@ -230,7 +231,6 @@ struct Plan {
     uint32_t flags;      // the MDIM_COLLECT_* flags the plan was made with
     int32_t slot_bytes;  // 4 or 8: width of the value-stack slots
     int32_t vec;
-    int32_t vpt;         // vectors per thread trip
     int32_t wide;        // 64-bit coordinates/strides
     int32_t n_axes;      // rank + red_rank after canonicalisation (selects the MAXR instantiation)
     int32_t vec256_ok;   // every LEAF_VEC operand is 32-byte aligned (the output is checked at launch)
@@ -260,7 +260,7 @@ const char* status_string(int st);
 // jit.cu: a kernel specialised at run time for the plan's op sequence, or nullptr (use the interpreter)
 void* jit_kernel_for(const Plan& p, int* level = nullptr);  // level: 0 none, 1 specialised on the op sequence, 2 on ops AND shape
 
-int find_static_signature(const char* sig, int sig_len, int slot_bytes, int vec, int vpt, int need_maxr, int wide);
+int find_static_signature(const char* sig, int sig_len, int slot_bytes, int vec, int need_maxr, int wide);
 // NVRTC half of jit_kernel_for alone (needs no GPU): 0 = the specialisation compiles for sm_100a
 int jit_compile_check(const Plan& p, char* log, size_t log_len);
 #endif

@@ -52,10 +52,10 @@ def main():
     def pick(pred):
         return [(n, c) for n, c in rows if pred(n)]
     groups = [
-        ("config 2: fused contiguous elementwise `k_eval<SigMulAddCF32, …, V=8, MAXR=1>` (256-bit accesses, no FFMA)", pick(lambda n: "SigMulAddCF32" in n and "8, 4, false, 1, 1" in n)),
+        ("config 2: fused contiguous elementwise `k_eval<SigMulAddCF32, …, V=8, MAXR=1>` (256-bit accesses, no FFMA)", pick(lambda n: "SigMulAddCF32" in n and "8, 4, false, 1>" in n)),
         ("config 1: tensor-map TMA transpose `k_transpose_tma<ES, peers>`", pick(lambda n: n.startswith("k_transpose_tma"))),
-        ("config 1 fallback: register-staged transpose `k_transpose<4, vec, 16, 64, peer>`", pick(lambda n: n.startswith("k_transpose<4, true, 16, 64"))),
-        ("config 3: gather `k_eval<SigGatherF32, u64 slots, V=4>` (LTC64B = the 64-byte L2 fetch flavour)", pick(lambda n: "SigGatherF32" in n and "4, 4, false, 1, 1" in n)),
+        ("config 1 fallback: register-staged transpose `k_transpose<4, vec, peer>`", pick(lambda n: n.startswith("k_transpose<4, true,"))),
+        ("config 3: gather `k_eval<SigGatherF32, u64 slots, V=4>` (LTC64B = the 64-byte L2 fetch flavour)", pick(lambda n: "SigGatherF32" in n and "4, 4, false, 1>" in n)),
         ("config 4: row folds `k_fold_rows<FAST>` (TMA bulk) and `k_fold_regs<L, FAST>`", pick(lambda n: n.startswith("k_fold_rows") or n.startswith("k_fold_regs<2,") or n.startswith("k_fold_regs<8,"))),
         ("sharded-axis fold: `k_fold_ring<S>` (TMA row tiles + peer-memory hand-off)", pick(lambda n: n.startswith("k_fold_ring") or "k_fold_ring" in n)),
         ("column walk `k_fold_xchg<S, DT, OP, ROWS, EXCHANGE>`: f32 / u64 sums, without (`k_fold_cols`, last argument false) and with the in-kernel all-reduce",

@@ -11,14 +11,12 @@
 #include "../../multidimension_b200/csrc/plan.cpp"
 
 namespace mdim {
-// No static signatures on the host; vpt > 1 is accepted so that the several-vectors-per-trip decode is
-// exercised too (through the interpreter, which the device only instantiates with vpt == 1).
-int find_static_signature(const char*, int, int, int, int vpt, int, int wide) { return vpt > 1 && !wide ? 0 : -1; }
+// No static signatures on the host.
+int find_static_signature(const char*, int, int, int, int, int) { return -1; }
 
 template <class S, int V, int MAXD, bool WIDE, int MAXR>
 static void run_all(const Program& P, void* out, ErrWord* err, uint64_t g0, uint64_t g1) {
-    if (P.vpt == 4) { for (uint64_t g = g0; g < g1; ++g) eval_vector<NoSig, S, V, MAXD, WIDE, MAXR, 4>(P, out, err, g); }
-    else { for (uint64_t g = g0; g < g1; ++g) eval_vector<NoSig, S, V, MAXD, WIDE, MAXR, 1>(P, out, err, g); }
+    for (uint64_t g = g0; g < g1; ++g) eval_vector<NoSig, S, V, MAXD, WIDE, MAXR>(P, out, err, g);
 }
 
 // the same MAXR choices the device registry offers (variants_s32.inc / variants_s64.inc), plus the
@@ -91,7 +89,7 @@ extern "C" int mdim_emu_collect(const mdim_expr* e, void* out, uint32_t flags, m
         q.explain_pos = pos;
         memset(&err, 0, sizeof err);
         err.pos = ~0ull;
-        const uint64_t item = pos / ((uint64_t)plan->vec * (uint64_t)plan->vpt);
+        const uint64_t item = pos / (uint64_t)plan->vec;
         run(*plan, q, out, &err, item, item + 1);
         st = err.status ? err.status : MDIM_ERR_INVALID;
         if (info) {

@@ -9,7 +9,7 @@ keep those tests green and leave the old kernel untested.
 So every case here names
   * the planner route `describe()` must report (checked on the CPU),
   * the kernel `Context.last_kernel()` must report after the GPU collect, under the default launch settings and under each
-    launch knob that changes it (MDIM_TR_*, MDIM_FOLD_MODE; those are read once per process, so knobs run in a subprocess),
+    launch knob that changes it (MDIM_TR_TMA, MDIM_FOLD_MODE; those are read once per process, so knobs run in a subprocess),
   * a reference computed with numpy from the input arrays alone — no lowering, descriptor or C oracle: `np.transpose(...)`
     for transposes, an explicit left-to-right loop in the element type for folds (wrapping integers in unsigned numpy
     arithmetic), and for f32 sums also an f64 error bound, so that a wrong reference cannot hide behind bit-equality.
@@ -40,12 +40,6 @@ ORACLE_MAX_ELEMS = 1 << 20  # the CPU half checks the reference against the orac
 KNOBS = {
     "default": {},
     "tr_tma=0": {"MDIM_TR_TMA": "0"},
-    "tr_pipe": {"MDIM_TR_TMA": "0", "MDIM_TR_PIPE": "1"},
-    "tr_tile=32x128": {"MDIM_TR_TILE": "32x128"},
-    "tr_tile=32x128,tma=0": {"MDIM_TR_TILE": "32x128", "MDIM_TR_TMA": "0"},
-    "tr_order=0": {"MDIM_TR_ORDER": "0"},
-    "tr_order=1": {"MDIM_TR_ORDER": "1"},
-    "tr_order=1,tma=0": {"MDIM_TR_ORDER": "1", "MDIM_TR_TMA": "0"},
     "fold_mode=1": {"MDIM_FOLD_MODE": "1"},
     "fold_mode=2": {"MDIM_FOLD_MODE": "2"},
 }
@@ -182,21 +176,10 @@ def permuted(a, n, perm):
 
 
 def transpose_kernels(base):
-    """The kernel under every transpose knob, from the one that runs by default.  TMA takes every case whose strides and base
-    are 16-byte aligned with <= 3 batch axes; without it the register-staged kernel loads 16 bytes at a time where the case
-    is aligned (vec), else element by element (scalar); MDIM_TR_PIPE=1 swaps the aligned register-staged kernel for the
-    cp.async ring (default tile only)."""
-    out = {}
-    for knob in ["default"] + TRANSPOSE_KNOBS:
-        env = KNOBS[knob]
-        k = base
-        if base != "k_transpose<regs,scalar>":
-            if base == "k_transpose_tma" and env.get("MDIM_TR_TMA") == "0":
-                k = "k_transpose<regs,vec>"
-            if k == "k_transpose<regs,vec>" and env.get("MDIM_TR_PIPE") == "1" and "MDIM_TR_TILE" not in env:
-                k = "k_transpose_pipe"
-        out[knob] = k
-    return out
+    """The kernel by default and without TMA.  TMA takes every case whose strides and base are 16-byte aligned with <= 3
+    batch axes; without it the register-staged kernel loads 16 bytes at a time where the case is aligned (vec), else element
+    by element (scalar)."""
+    return {"default": base, "tr_tma=0": "k_transpose<regs,vec>" if base == "k_transpose_tma" else base}
 
 
 def add_transpose(id, T, shape, perm, kernel, pin=None):
@@ -244,11 +227,13 @@ for T in ("f32", "f64", "u64"):
     add_raw_transpose("negative-row-stride", T, 36, 20, 40, 16 // es)
 add_transpose("pitch-not-16B-64x66", "f32", (64, 66), (1, 0), "k_transpose<regs,scalar>")        # 264-byte rows, 4-byte-aligned output
 add_transpose("pitch-not-16B-30x64", "f32", (30, 64), (1, 0), "k_transpose<regs,scalar>")        # 120-byte output rows
+# source and output together above 512 MiB: the TMA kernel walks its tiles B-fastest instead of A-fastest
+add_transpose("8192x8256", "f32", (8192, 8256), (1, 0), "k_transpose_tma")
 
 
 # ---- fold over the last axis: k_fold_rows / k_fold_regs --------------------------------------------------------------------------
 K_FOLD_THREADS = 256        # k_fold.cu / kernels.cuh: kFoldThreads
-K_FOLD_GRID_MULT = 16       # k_fold.cu: CTAs queued per SM (MDIM_FOLD_GRID_MULT unset)
+K_FOLD_GRID_MULT = 16       # k_fold.cu: CTAs queued per SM
 K_FOLD_SMEM = 227 * 1024 - 512   # k_fold.cu: the opt-in shared memory of an SM less the mbarriers (kBarBytes)
 
 
@@ -434,7 +419,7 @@ def test_four_batch_axes_stay_four():
 
 def test_case_table_names_every_dedicated_kernel():
     named = {k for c in CASES for k in c.kernels.values()}
-    for k in ("k_transpose_tma", "k_transpose<regs,vec>", "k_transpose<regs,scalar>", "k_transpose_pipe", "k_fold_rows", "k_fold_regs", "k_fold_cols"):
+    for k in ("k_transpose_tma", "k_transpose<regs,vec>", "k_transpose<regs,scalar>", "k_fold_rows", "k_fold_regs", "k_fold_cols"):
         assert k in named, k
 
 
@@ -481,7 +466,7 @@ def test_kernel_route(case, gpu_ctx):
 @pytest.mark.parametrize("knob", TRANSPOSE_KNOBS + FOLD_KNOBS)
 def test_launch_knobs(knob):
     """The launch knobs are read once per process: each runs in a subprocess over the cases it re-routes (every transpose for
-    MDIM_TR_*, every last-axis fold for MDIM_FOLD_MODE), asserting the kernel each case must then run on."""
+    MDIM_TR_TMA, every last-axis fold for MDIM_FOLD_MODE), asserting the kernel each case must then run on."""
     group = "transpose" if knob.startswith("tr_") else "fold_rows"
     code = (f"import sys; sys.path.insert(0, 'tests'); import test_kernel_routes as K; "
             f"print('ran', K.run_group({group!r}, {knob!r}))")
