@@ -59,6 +59,11 @@ int find_static_signature(const char* sig, int sig_len, int slot_bytes, int vec,
     return -1;
 }
 
+// The instantiation's template arguments, e.g. k_eval<SigSubBcastF32,s32,v8,d4,r3> or k_eval<interp,s64,v1,d8,wide,r8>.
+static void eval_kernel_name(const EvalVariant& v, char* buf, size_t len) {
+    snprintf(buf, len, "k_eval<%s,s%d,v%d,d%d%s,r%d>", v.sig ? v.name : "interp", v.slot_bytes * 8, v.vec, v.max_depth, v.wide ? ",wide" : "", v.maxr);
+}
+
 static const EvalVariant* select_variant(const Plan& p, bool force_interp) {
     const std::vector<EvalVariant>& R = registry();
     const int need = p.kind == KK_STREAM ? 1 : std::max(1, p.n_axes);
@@ -122,8 +127,9 @@ int launch_eval(mdim_ctx* ctx, const Plan& p, void* out, ErrWord* err, bool expl
     // an op tree without a pre-built signature is specialised on first use (jit.cu); else the interpreter runs
     void* jit = nullptr;
     int jit_level = 0;
-    if (!(p.flags & (MDIM_COLLECT_NO_STATIC | MDIM_COLLECT_NO_JIT))) jit = jit_kernel_for(p, &jit_level);
-    snprintf(ctx->last_kernel, sizeof ctx->last_kernel, "%s", jit ? (jit_level == 2 ? "mdim_jit_kernel[ops+shape]" : "mdim_jit_kernel[ops]") : v->name);
+    if (!(p.flags & (MDIM_COLLECT_NO_STATIC | MDIM_COLLECT_NO_JIT))) jit = jit_kernel_for(p, &jit_level, explain);
+    if (jit) snprintf(ctx->last_kernel, sizeof ctx->last_kernel, "%s", jit_level == 2 ? "mdim_jit_kernel[ops+shape]" : "mdim_jit_kernel[ops]");
+    else eval_kernel_name(*v, ctx->last_kernel, sizeof ctx->last_kernel);
     Program q = p.prog;
     if (p.vec256_ok && ((uintptr_t)out % 32) == 0) q.flags |= PF_VEC256;
     if (nowait && !explain) q.flags |= PF_NOWAIT;

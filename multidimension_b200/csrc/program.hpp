@@ -258,7 +258,8 @@ const char* status_string(int st);
 
 // Signature registry (defined with the kernels; the planner only needs lookup by bytes).
 // jit.cu: a kernel specialised at run time for the plan's op sequence, or nullptr (use the interpreter)
-void* jit_kernel_for(const Plan& p, int* level = nullptr);  // level: 0 none, 1 specialised on the op sequence, 2 on ops AND shape
+// explain: the single-element rerun of a failed collect; it reuses a shape kernel already built but neither counts towards nor triggers one
+void* jit_kernel_for(const Plan& p, int* level = nullptr, bool explain = false);  // level: 0 none, 1 specialised on the op sequence, 2 on ops AND shape
 
 int find_static_signature(const char* sig, int sig_len, int slot_bytes, int vec, int need_maxr, int wide);
 // NVRTC half of jit_kernel_for alone (needs no GPU): 0 = the specialisation compiles for sm_100a
