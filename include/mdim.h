@@ -197,7 +197,9 @@ typedef struct mdim_ctx mdim_ctx;
 /* ---- context ---------------------------------------------------------------------------------- */
 int mdim_init(int device, mdim_ctx** ctx);
 int mdim_shutdown(mdim_ctx* ctx);
-/* Launch on a caller-owned cudaStream_t (e.g. torch's current stream); NULL = the context's own. */
+/* Launch on a caller-owned cudaStream_t (e.g. torch's current stream); NULL = the context's own.  It first waits for every collect
+ * on the old stream, so a context's collects never run on two streams at once (the scratch of the few-output integer folds,
+ * k_fold_split, relies on this: one context, one stream at a time). */
 int mdim_set_stream(mdim_ctx* ctx, void* cuda_stream);
 /* The stream collects are launched on (a cudaStream_t): the context's own unless mdim_set_stream replaced it.  Record
  * CUDA events on it to time collects.  On its OWN stream the context knows every kernel in flight, so a collect whose

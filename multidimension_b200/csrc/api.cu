@@ -101,11 +101,13 @@ bool plan_can_fail(const Plan& p) {
 // nothing it writes was touched, by a kernel that may still be running.  Either way the launch is recorded.
 bool may_skip_wait(mdim_ctx* ctx, const Plan& p, const void* out) {
     const bool usable = ctx->dep_tracking && pdl_enabled() && ctx->stream == ctx->own_stream && p.n_in_ranges >= 0;
-    mdim_ctx::Touched mine[kMaxRanges + 1];
+    mdim_ctx::Touched mine[kMaxRanges + 2];
     int n = 0;
     if (p.n_in_ranges >= 0)
         for (int i = 0; i < p.n_in_ranges; ++i) mine[n++] = {p.in_range[i].lo, p.in_range[i].hi, false};
     mine[n++] = {(uint64_t)(uintptr_t)out, (uint64_t)(uintptr_t)out + p.out_elems * (uint64_t)p.out_esize, true};
+    if (p.kind == KK_FOLD_SPLIT)  // its tickets and partials: a second split fold must wait for this one
+        mine[n++] = {(uint64_t)(uintptr_t)ctx->split_scratch, (uint64_t)(uintptr_t)ctx->split_scratch + ctx->split_scratch_bytes, true};
     bool conflict = !usable || ctx->inflight.size() + (size_t)n > 256 || p.n_out > 1;  // several output runs: simply wait
     for (size_t k = 0; k < ctx->inflight.size() && !conflict; ++k) {
         const mdim_ctx::Touched& t = ctx->inflight[k];
@@ -156,8 +158,29 @@ int launch_eval(mdim_ctx* ctx, const Plan& p, void* out, ErrWord* err, bool expl
     return MDIM_OK;
 }
 
+// Scratch for k_fold_split of at least `bytes` (tickets included).  A new allocation waits for the stream (the old one may still
+// be in use) and zeroes the tickets before any split fold reads them.
+int ensure_split_scratch(mdim_ctx* ctx, size_t bytes) {
+    if (bytes <= ctx->split_scratch_bytes) return MDIM_OK;
+    CU(ctx, cudaStreamSynchronize(ctx->stream));
+    if (ctx->split_scratch) { CU(ctx, cudaFree(ctx->split_scratch)); ctx->split_scratch = nullptr; ctx->split_scratch_bytes = 0; }
+    bytes = std::max<size_t>(bytes, (size_t)1 << 20);
+    CU(ctx, cudaMalloc((void**)&ctx->split_scratch, bytes));
+    CU(ctx, cudaMemsetAsync(ctx->split_scratch, 0, kSplitMaxOuts * sizeof(unsigned int), ctx->stream));
+    CU(ctx, cudaStreamSynchronize(ctx->stream));
+    ctx->split_scratch_bytes = bytes;
+    ctx->inflight.clear();  // the stream is idle
+    return MDIM_OK;
+}
+
 int launch_plan(mdim_ctx* ctx, const Plan& p, void* out, ErrWord* err) {
     if (p.kind == KK_EMPTY) return MDIM_OK;
+    SplitGeometry sg{};
+    if (p.kind == KK_FOLD_SPLIT) {
+        sg = fold_split_geometry(p.fs, ctx->sm_count);
+        int st = ensure_split_scratch(ctx, kSplitMaxOuts * sizeof(unsigned int) + sg.partials * 8);
+        if (st) return st;
+    }
     const bool nowait = may_skip_wait(ctx, p, out);
     switch (p.kind) {
         case KK_TRANSPOSE: {
@@ -186,6 +209,17 @@ int launch_plan(mdim_ctx* ctx, const Plan& p, void* out, ErrWord* err) {
             const char* name = launch_fold_cols(fc, out, ctx->stream);
             if (!name) return cuda_fail(ctx, cudaGetLastError(), "k_fold_cols");
             snprintf(ctx->last_kernel, sizeof ctx->last_kernel, "%s", name);
+            ctx->launches++;
+            CU(ctx, cudaGetLastError());
+            return MDIM_OK;
+        }
+        case KK_FOLD_SPLIT: {
+            FoldSplitPlan fs = p.fs;
+            fs.nowait = nowait;
+            char* scratch = ctx->split_scratch;
+            const char* name = launch_fold_split(fs, sg, out, (unsigned int*)scratch, scratch + kSplitMaxOuts * sizeof(unsigned int), ctx->stream,
+                                                 ctx->last_kernel, sizeof ctx->last_kernel);
+            if (!name) return cuda_fail(ctx, cudaGetLastError(), "k_fold_split");
             ctx->launches++;
             CU(ctx, cudaGetLastError());
             return MDIM_OK;
@@ -316,6 +350,7 @@ int mdim_shutdown(mdim_ctx* ctx) {
     if (hp.h2d) cudaStreamDestroy(hp.h2d);
     if (hp.d2h) cudaStreamDestroy(hp.d2h);
     if (hp.arena) cudaFree(hp.arena);
+    if (ctx->split_scratch) cudaFree(ctx->split_scratch);
     cudaFree(ctx->d_err);
     cudaFreeHost(ctx->h_err);
     cudaStreamDestroy(ctx->own_stream);

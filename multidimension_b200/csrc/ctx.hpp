@@ -51,6 +51,10 @@ struct mdim_ctx {
     size_t host_chunk_bytes = 128u << 20;  // measured: 8 MB 60.7, 32 MB 73.1, 128 MB 75.8, 512 MB 76.3 GB/s end to end
     mdim::Comm* comm = nullptr;  // mdim_comm_init (comm.cu)
     char last_kernel[96] = {0};  // mdim_last_kernel: what the last collect actually launched
+    // k_fold_split's scratch: kSplitMaxOuts tickets (zeroed once here; every launch leaves them at 0), then the chunks' partials.
+    // Grown on first use, freed by mdim_shutdown.  Every split fold writes it, so may_skip_wait never lets two overlap.
+    char* split_scratch = nullptr;
+    size_t split_scratch_bytes = 0;
 };
 
 namespace mdim {

@@ -63,4 +63,18 @@ int launch_fold_xchg(const FoldXchgArgs& A, int dtype, int op, int sm_count, cud
 // ... and the same column walk on one GPU, no exchange (KK_FOLD_COLS): -> name of the kernel launched, nullptr on a launch error
 const char* launch_fold_cols(const FoldColsPlan& C, void* out, cudaStream_t stream);
 
+// ------------------------------------------------------------------------------------------------
+// Integer fold with few outputs and a long reduction, the reduction cut into chunks over the whole GPU (k_fold_split.cu)
+// ------------------------------------------------------------------------------------------------
+struct SplitGeometry {
+    uint64_t units;     // RUNS: outputs; COLS: batches.  Each has one ticket.
+    uint64_t n_chunks;  // chunks per unit: the grid is units x n_chunks CTAs
+    uint64_t chunk;     // RUNS: elements per chunk; COLS: rows per chunk
+    uint64_t partials;  // slots of scratch the launch writes (each slot_bytes wide)
+};
+SplitGeometry fold_split_geometry(const FoldSplitPlan& F, int sm_count);
+// tickets: units zeroed words; partials: G.partials slots.  -> name of the instantiation launched, nullptr on a launch error
+const char* launch_fold_split(const FoldSplitPlan& F, const SplitGeometry& G, void* out, unsigned int* tickets, void* partials,
+                              cudaStream_t stream, char* name, size_t name_len);
+
 }  // namespace mdim

@@ -95,6 +95,7 @@ struct Builder {
     int gen(int ni, int mask_first, int mask_n);
     int push_instr(const Instr& in);
     int detect_fast_paths();
+    bool detect_fold_split();
 };
 
 int Builder::validate() {
@@ -612,6 +613,7 @@ int Builder::detect_fast_paths() {
             return MDIM_OK;
         }
     }
+    if (detect_fold_split()) return MDIM_OK;
     // (2) last-axis sequential fold of one contiguous f32/f64/int leaf, optionally fused with
     //     `x (eop) (fold [post_op c])` broadcast back over the folded axis (config C4)
     if (fold_node >= 0 && n_child[fold_node] == 1 && red_rank == 1 && rank <= 2 && !plan->wide && !(flags & kPlanScalarOut)) {
@@ -695,6 +697,69 @@ int Builder::detect_fast_paths() {
     }
     (void)P;
     return MDIM_OK;
+}
+
+// (0) an integer fold with few outputs and a long reduction, its body one leaf or one integer cast of one leaf: k_fold_split cuts
+//     the reduction into chunks spread over the whole GPU and combines the chunks' partials.  Every other route parallelises over
+//     the outputs only, so one thread (or a few lanes) would walk each output's reduction.
+bool Builder::detect_fold_split() {
+    const mdim_node* N = e->nodes;
+    const int root = e->n_nodes - 1;
+    if (fold_node != root || n_child[fold_node] != 1 || red_rank < 1) return false;  // an init view keeps its route
+    const mdim_node& F = N[fold_node];
+    const bool op_ok = F.op == MDIM_ADD || F.op == MDIM_SUB || F.op == MDIM_MUL || F.op == MDIM_AND || F.op == MDIM_OR || F.op == MDIM_XOR;
+    if (!op_ok || !is_int(F.dtype)) return false;
+    int lf = child[fold_node][0];
+    if (N[lf].kind == MDIM_NODE_UNARY && N[lf].op == MDIM_CAST && is_int(N[lf].src_dtype) && N[lf].dtype == F.dtype) lf = child[lf][0];
+    else if (N[lf].dtype != F.dtype) return false;
+    if (N[lf].kind != MDIM_NODE_LEAF || N[lf].n_peers > 1 || !is_int(N[lf].dtype)) return false;
+    uint64_t n_out = 1, red = 1;
+    for (int g = 0; g < rank; ++g) n_out *= len[g];
+    for (int g = rank; g < n_axes; ++g) red *= len[g];
+    if (n_out > kSplitMaxOuts || red < kSplitMinRed) return false;
+    // The operators above are associative and commutative (Sub: init - sum), so the reduction may be walked in any order: sort
+    // its axes by |stride|, flip the negative ones and merge again.  A whole transposed or reversed array then reads memory in
+    // order.  No other route may do this: a float fold, or Div, must combine in index order.
+    const int64_t* s = cstride[lf];
+    int64_t offset = N[lf].offset;
+    struct Ax { uint64_t len; int64_t stride; };
+    std::vector<Ax> ra;
+    for (int g = rank; g < n_axes; ++g) {
+        int64_t st = s[g];
+        if (st < 0) { offset += st * (int64_t)(len[g] - 1); st = -st; }
+        ra.push_back(Ax{len[g], st});
+    }
+    std::stable_sort(ra.begin(), ra.end(), [](const Ax& a, const Ax& b) { return a.stride < b.stride; });
+    std::vector<Ax> merged{ra[0]};
+    for (size_t k = 1; k < ra.size(); ++k) {
+        Ax& in = merged.back();
+        if (ra[k].stride == in.stride * (int64_t)in.len) in.len *= ra[k].len;
+        else merged.push_back(ra[k]);
+    }
+    if (merged.size() != 1) return false;
+    const int64_t rstride = merged[0].stride;
+    FoldSplitPlan& S = plan->fs;
+    memset(&S, 0, sizeof S);
+    const int src_es = dtype_size(N[lf].dtype);
+    S.src = (const char*)N[lf].data + offset * src_es;
+    S.op = F.op; S.dtype = F.dtype; S.src_dtype = N[lf].dtype;
+    S.slot_bytes = dtype_size(F.dtype) == 8 ? 8 : 4;
+    S.init = F.imm.u64;
+    S.red = red; S.n_out = n_out;
+    if (rstride == 1 && rank <= 2) {  // runs: a whole reduction, or a few rows of contiguous elements, output strides free
+        S.layout = SPLIT_RUNS;
+        S.out_len[0] = S.out_len[1] = 1;
+        for (int g = 0; g < rank; ++g) { S.out_len[2 - rank + g] = len[g]; S.out_stride[2 - rank + g] = s[g]; }
+    } else if ((rank == 1 || rank == 2) && s[rank - 1] == 1 && rstride >= (int64_t)len[rank - 1] && n_out <= kSplitMaxCols) {  // columns: the k_fold_cols layout
+        S.layout = SPLIT_COLS;
+        S.cols = len[rank - 1]; S.pitch = rstride;
+        S.n_batch = rank == 2 ? len[0] : 1; S.batch_stride = rank == 2 ? s[0] : 0;
+    } else return false;
+    static const char* const dt_name[] = {"u8", "i32", "u32", "i64", "u64"};
+    plan->kind = KK_FOLD_SPLIT;
+    snprintf(plan->describe, sizeof plan->describe, "fold_split.%s outs=%llu red=%llu slot=s%d src=%s op=%d", S.layout == SPLIT_RUNS ? "runs" : "cols",
+             (unsigned long long)n_out, (unsigned long long)red, S.slot_bytes * 8, dt_name[S.src_dtype], S.op);
+    return true;
 }
 
 }  // namespace

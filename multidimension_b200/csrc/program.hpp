@@ -125,6 +125,7 @@ enum KernelKind : int32_t {
     KK_TRANSPOSE = 3,  // tiled smem transpose of one leaf (k_transpose)
     KK_FOLD_ROWS = 4,  // last-axis sequential fold (+ fused broadcast epilogue) (k_fold_rows)
     KK_FOLD_COLS = 5,  // sequential fold over an OUTER axis of one leaf whose result is contiguous: a column walk (k_fold_cols)
+    KK_FOLD_SPLIT = 6, // integer fold with few outputs and a long reduction: the reduction cut into chunks over the whole GPU (k_fold_split)
 };
 
 // The register-staged transpose's tile (k_transpose.cu): 16-byte chunks along A x source rows, 256-byte runs both ways.
@@ -183,6 +184,31 @@ struct FoldColsPlan {
     int32_t op, dtype;
     uint64_t init;
     int32_t nowait;       // set per launch (api.cu): see launch.cuh
+};
+
+// k_fold_split.cu: an integer fold whose operator is associative and commutative (wrapping Add, Mul, BitAnd, BitOr, BitXor; Sub as
+// init - sum), so any order of combination gives the reference's bits.  Taken for at most kSplitMaxOuts outputs and a reduction
+// of at least kSplitMinRed elements (kSplitMaxCols outputs when they are columns): there the other routes leave most of the GPU
+// idle, one thread or a few walking each output.  Measured on one B200 (1000 W), u32 sums (profiles/r3_fold_split_bench.txt):
+// the split fold wins at every reduction length measured (down to 2^12) for up to 16384 runs and up to 1024 columns, and loses
+// at 4096 columns (71 against 264 GB/s for k_fold_cols: the finishing CTA's combine caps the chunks of a wide row).
+constexpr uint64_t kSplitMaxOuts = 4096, kSplitMaxCols = 1024, kSplitMinRed = 1ull << 12;
+enum SplitLayout : int32_t { SPLIT_RUNS = 0, SPLIT_COLS = 1 };
+struct FoldSplitPlan {
+    const void* src;        // element 0 of the walk (the leaf's offset and any flipped reduction axis applied)
+    int32_t layout;         // SPLIT_RUNS: each output reduces one run of `red` contiguous elements
+                            // SPLIT_COLS: each output is a column; `cols` contiguous columns per row, rows `pitch` apart
+    int32_t op;             // MDIM_ADD, SUB, MUL, AND, OR, XOR
+    int32_t dtype, src_dtype;  // the fold's dtype; the leaf's (a CAST body converts between them)
+    int32_t slot_bytes;     // 4 or 8: the accumulator width (the fold's dtype, U8 widened to 4)
+    int32_t nowait;         // set per launch (api.cu): see launch.cuh
+    uint64_t init;          // bits of the immediate init
+    uint64_t red;           // RUNS: elements per run; COLS: rows
+    uint64_t n_out;         // outputs, written contiguously
+    uint64_t out_len[2];    // RUNS: output o = i0 * out_len[1] + i1 starts at i0 * out_stride[0] + i1 * out_stride[1] (elements)
+    int64_t out_stride[2];
+    uint64_t cols, n_batch; // COLS: output o = b * cols + c reads b * batch_stride + r * pitch + c (elements)
+    int64_t pitch, batch_stride;
 };
 
 // Memory a launch reads (api.cu adds the output and decides whether the kernel may skip griddepcontrol.wait).
@@ -244,6 +270,7 @@ struct Plan {
     TransposePlan tr;
     FoldRowsPlan fr;
     FoldColsPlan fc;
+    FoldSplitPlan fs;
     char sig[kMaxInstr * 4 + 4];  // signature bytes (opc,dtype,op,aux per instruction)
     int32_t sig_len;
     char describe[192];
