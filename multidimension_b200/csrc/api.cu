@@ -10,6 +10,7 @@
 #include <string.h>
 
 #include <algorithm>
+#include <memory>
 #include <new>
 #include <vector>
 
@@ -19,72 +20,23 @@
 
 using namespace mdim;
 
-namespace mdim {
+namespace {
 
-// ---- variant registry ----------------------------------------------------------------------------
-static std::vector<EvalVariant>& registry() {
-    static std::vector<EvalVariant> all = [] {
-        std::vector<EvalVariant> v;
-        int n = 0;
-        const EvalVariant* (*parts[])(int*) = {eval_variants_s32_static, eval_variants_s64_static, eval_variants_s32_interp, eval_variants_s64_interp};
-        for (auto part : parts) {
-            const EvalVariant* a = part(&n);
-            v.insert(v.end(), a, a + n);
+// The k_eval kernel of instantiation `variant` (Plan::variant), or nullptr if the four k_eval_*.cu lists do not add up to the
+// planner's table.
+EvalKernel eval_kernel(int variant) {
+    static const std::vector<EvalKernel> all = [] {
+        std::vector<EvalKernel> v;
+        for (auto part : {eval_kernels_s32_static, eval_kernels_s64_static, eval_kernels_s32_interp, eval_kernels_s64_interp}) {
+            int n = 0;
+            const EvalKernel* k = part(&n);
+            v.insert(v.end(), k, k + n);
         }
+        if ((int)v.size() != kNumEvalVariants) v.clear();
         return v;
     }();
-    return all;
+    return variant >= 0 && variant < (int)all.size() ? all[variant] : nullptr;
 }
-
-static bool sig_matches(const EvalVariant& v, const char* sig, int sig_len) {
-    if (!v.sig || v.sig_n * 4 != sig_len) return false;
-    for (int i = 0; i < v.sig_n; ++i) {
-        const unsigned char* s = (const unsigned char*)sig + 4 * i;
-        if (v.sig[i].opc != s[0] || v.sig[i].dtype != s[1]) return false;
-        // op/aux only matter for the opcodes that read them
-        const int opc = v.sig[i].opc;
-        if ((opc == OPC_LEAF_VEC || opc == OPC_LEAF_BCAST || opc == OPC_LEAF_STRIDED) && v.sig[i].aux != s[3]) return false;  // aux: bit 0 cached, bit 1 sharded
-        if ((opc == OPC_BINARY || opc == OPC_UNARY || opc == OPC_FOLD_STEP) && (v.sig[i].op != s[2] || v.sig[i].aux != s[3])) return false;
-        if (opc == OPC_GATHER && v.sig[i].aux != s[3]) return false;
-    }
-    return true;
-}
-
-int find_static_signature(const char* sig, int sig_len, int slot_bytes, int vec, int need_maxr, int wide) {
-    if (wide) return -1;  // signatures are instantiated with 32-bit coordinates only
-    const std::vector<EvalVariant>& R = registry();
-    for (size_t i = 0; i < R.size(); ++i)
-        if (R[i].slot_bytes == slot_bytes && R[i].vec == vec && R[i].maxr >= need_maxr && !R[i].wide && sig_matches(R[i], sig, sig_len))
-            return (int)i;
-    return -1;
-}
-
-// The instantiation's template arguments, e.g. k_eval<SigSubBcastF32,s32,v8,d4,r3> or k_eval<interp,s64,v1,d8,wide,r8>.
-static void eval_kernel_name(const EvalVariant& v, char* buf, size_t len) {
-    snprintf(buf, len, "k_eval<%s,s%d,v%d,d%d%s,r%d>", v.sig ? v.name : "interp", v.slot_bytes * 8, v.vec, v.max_depth, v.wide ? ",wide" : "", v.maxr);
-}
-
-static const EvalVariant* select_variant(const Plan& p, bool force_interp) {
-    const std::vector<EvalVariant>& R = registry();
-    const int need = p.kind == KK_STREAM ? 1 : std::max(1, p.n_axes);
-    const EvalVariant* best = nullptr;
-    if (p.static_id >= 0 && !p.wide && !force_interp) {
-        for (const EvalVariant& v : R) {
-            if (v.slot_bytes != p.slot_bytes || v.vec != p.vec || v.wide || v.maxr < need || !sig_matches(v, p.sig, p.sig_len)) continue;
-            if (!best || v.maxr < best->maxr) best = &v;
-        }
-        if (best) return best;
-    }
-    for (const EvalVariant& v : R) {
-        if (v.sig || v.slot_bytes != p.slot_bytes || v.vec != p.vec || v.wide != p.wide || v.maxr < need || v.max_depth < p.max_depth) continue;
-        if (!best || v.maxr < best->maxr || (v.maxr == best->maxr && v.max_depth < best->max_depth)) best = &v;
-    }
-    return best;
-}
-
-}  // namespace mdim
-
-namespace {
 
 bool plan_can_fail(const Plan& p) {
     if (p.kind != KK_GENERIC && p.kind != KK_STREAM) return false;
@@ -122,8 +74,9 @@ bool may_skip_wait(mdim_ctx* ctx, const Plan& p, const void* out) {
 }
 
 int launch_eval(mdim_ctx* ctx, const Plan& p, void* out, ErrWord* err, bool explain, uint64_t explain_pos, bool nowait = false) {
-    const EvalVariant* v = select_variant(p, false);
-    if (!v) return set_error(ctx, MDIM_ERR_UNSUPPORTED, "no evaluator instantiation for this expression");
+    if (p.variant < 0) return set_error(ctx, MDIM_ERR_UNSUPPORTED, "no evaluator instantiation for this expression");
+    const EvalKernel fn = eval_kernel(p.variant);
+    if (!fn) return set_error(ctx, MDIM_ERR_INVALID, "the k_eval kernels do not match the planner's instantiation table");
     uint64_t g0 = 0, g1 = p.prog.n_vec;
     int grid;
     // an op tree without a pre-built signature is specialised on first use (jit.cu); else the interpreter runs
@@ -131,7 +84,7 @@ int launch_eval(mdim_ctx* ctx, const Plan& p, void* out, ErrWord* err, bool expl
     int jit_level = 0;
     if (!(p.flags & (MDIM_COLLECT_NO_STATIC | MDIM_COLLECT_NO_JIT))) jit = jit_kernel_for(p, &jit_level, explain);
     if (jit) snprintf(ctx->last_kernel, sizeof ctx->last_kernel, "%s", jit_level == 2 ? "mdim_jit_kernel[ops+shape]" : "mdim_jit_kernel[ops]");
-    else eval_kernel_name(*v, ctx->last_kernel, sizeof ctx->last_kernel);
+    else eval_variant_name(p.variant, ctx->last_kernel, sizeof ctx->last_kernel);
     Program q = p.prog;
     if (p.vec256_ok && ((uintptr_t)out % 32) == 0) q.flags |= PF_VEC256;
     if (nowait && !explain) q.flags |= PF_NOWAIT;
@@ -151,7 +104,7 @@ int launch_eval(mdim_ctx* ctx, const Plan& p, void* out, ErrWord* err, bool expl
         pdl_config(cfg, attr, dim3((unsigned)grid), dim3(kEvalThreads), 0, ctx->stream);
         CU(ctx, cudaLaunchKernelExC(&cfg, (const void*)jit, args));
     } else {
-        CU(ctx, launch_pdl(v->fn, dim3((unsigned)grid), dim3(kEvalThreads), 0, ctx->stream, q, out, err, g0, g1));
+        CU(ctx, launch_pdl(fn, dim3((unsigned)grid), dim3(kEvalThreads), 0, ctx->stream, q, out, err, g0, g1));
     }
     ctx->launches++;
     CU(ctx, cudaGetLastError());
@@ -175,57 +128,24 @@ int ensure_split_scratch(mdim_ctx* ctx, size_t bytes) {
 
 int launch_plan(mdim_ctx* ctx, const Plan& p, void* out, ErrWord* err) {
     if (p.kind == KK_EMPTY) return MDIM_OK;
-    SplitGeometry sg{};
     if (p.kind == KK_FOLD_SPLIT) {
-        sg = fold_split_geometry(p.fs, ctx->sm_count);
-        int st = ensure_split_scratch(ctx, kSplitMaxOuts * sizeof(unsigned int) + sg.partials * 8);
+        int st = ensure_split_scratch(ctx, fold_split_scratch_bytes(p.fs, ctx->sm_count));
         if (st) return st;
     }
     const bool nowait = may_skip_wait(ctx, p, out);
+    const char* name;
     switch (p.kind) {
-        case KK_TRANSPOSE: {
-            // Not persistent: far more CTAs than fit at once, so the hardware scheduler balances the tail.
-            // Measured (B200, 16384^2 f32): 8/SM (resident set) 5.71 TB/s, 64/SM 6.18, 128/SM 6.32, one CTA per tile 6.35.
-            const uint64_t cap = (uint64_t)ctx->sm_count * 128;
-            const int grid = (int)std::min<uint64_t>(p.tr.n_tiles, std::max<uint64_t>(cap, 1));
-            TransposePlan tr = p.tr;
-            tr.nowait = nowait;
-            snprintf(ctx->last_kernel, sizeof ctx->last_kernel, "%s", launch_transpose(tr, out, grid, ctx->stream));
-            ctx->launches++;
-            CU(ctx, cudaGetLastError());
-            return MDIM_OK;
-        }
-        case KK_FOLD_ROWS: {
-            FoldRowsPlan fr = p.fr;
-            fr.nowait = nowait;
-            snprintf(ctx->last_kernel, sizeof ctx->last_kernel, "%s", launch_fold_rows(fr, out, ctx->sm_count, ctx->stream));
-            ctx->launches++;
-            CU(ctx, cudaGetLastError());
-            return MDIM_OK;
-        }
-        case KK_FOLD_COLS: {
-            FoldColsPlan fc = p.fc;
-            fc.nowait = nowait;
-            const char* name = launch_fold_cols(fc, out, ctx->stream);
-            if (!name) return cuda_fail(ctx, cudaGetLastError(), "k_fold_cols");
-            snprintf(ctx->last_kernel, sizeof ctx->last_kernel, "%s", name);
-            ctx->launches++;
-            CU(ctx, cudaGetLastError());
-            return MDIM_OK;
-        }
-        case KK_FOLD_SPLIT: {
-            FoldSplitPlan fs = p.fs;
-            fs.nowait = nowait;
-            char* scratch = ctx->split_scratch;
-            const char* name = launch_fold_split(fs, sg, out, (unsigned int*)scratch, scratch + kSplitMaxOuts * sizeof(unsigned int), ctx->stream,
-                                                 ctx->last_kernel, sizeof ctx->last_kernel);
-            if (!name) return cuda_fail(ctx, cudaGetLastError(), "k_fold_split");
-            ctx->launches++;
-            CU(ctx, cudaGetLastError());
-            return MDIM_OK;
-        }
+        case KK_TRANSPOSE: name = launch_transpose(p, out, nowait, ctx->stream, ctx->sm_count); break;
+        case KK_FOLD_ROWS: name = launch_fold_rows(p, out, nowait, ctx->stream, ctx->sm_count); break;
+        case KK_FOLD_COLS: name = launch_fold_cols(p, out, nowait, ctx->stream, ctx->sm_count); break;
+        case KK_FOLD_SPLIT: name = launch_fold_split(p, out, nowait, ctx->stream, ctx->sm_count, ctx->split_scratch); break;
         default: return launch_eval(ctx, p, out, err, false, 0, nowait);
     }
+    if (!name) return cuda_fail(ctx, cudaGetLastError(), "kernel launch");
+    snprintf(ctx->last_kernel, sizeof ctx->last_kernel, "%s", name);
+    ctx->launches++;
+    CU(ctx, cudaGetLastError());
+    return MDIM_OK;
 }
 
 // Fill ctx->last from a failed collect: rerun the failing element alone with PF_EXPLAIN.
@@ -239,25 +159,12 @@ int explain(mdim_ctx* ctx, const Plan& p, void* out, int slot, uint64_t pos) {
     if (st) return st;
     CU(ctx, cudaMemcpyAsync(h, d, sizeof *h, cudaMemcpyDeviceToHost, ctx->stream));
     CU(ctx, cudaStreamSynchronize(ctx->stream));
-    mdim_error_info& L = ctx->last;
-    memset(&L, 0, sizeof L);
-    L.status = h->status ? h->status : MDIM_ERR_INVALID;
-    L.node = h->status ? h->node : -1;
-    L.position = pos;
-    L.value = h->value;
-    L.bound = h->bound;
-    L.component = h->component;
-    if (L.status == MDIM_ERR_OOB)  // src/int.rs:17
-        snprintf(L.message, sizeof L.message, "Index %llu is out of bounds for size %llu", (unsigned long long)L.value, (unsigned long long)L.bound);
-    else if (L.status == MDIM_ERR_ARITH)
-        snprintf(L.message, sizeof L.message, "attempt to divide by zero or with overflow");
-    else
-        snprintf(L.message, sizeof L.message, "device reported a failure at position %llu", (unsigned long long)pos);
+    explain_failure(*h, pos, &ctx->last);
     // reset the slot for reuse
     h->pos = ~0ull; h->status = 0;
     CU(ctx, cudaMemcpyAsync(d, h, sizeof *h, cudaMemcpyHostToDevice, ctx->stream));
     CU(ctx, cudaStreamSynchronize(ctx->stream));
-    return L.status;
+    return ctx->last.status;
 }
 
 // Wait for the stream and resolve every pending (fallible) collect in submission order.
@@ -473,80 +380,51 @@ static int collect_planned(mdim_ctx* ctx, Plan* plan, void* out_device, uint32_t
     return drain(ctx);
 }
 
-int mdim_collect(mdim_ctx* ctx, const mdim_expr* e, void* out_device, uint32_t flags) {
-    if (!ctx) return MDIM_ERR_INVALID;
-    Plan* plan = new (std::nothrow) Plan();
+// Plan, then launch on the context's device.  One Plan is several KB: it lives on the heap.
+static int collect(mdim_ctx* ctx, const mdim_expr* e, void* const* outs, int n_outs, uint32_t flags) {
+    std::unique_ptr<Plan> plan(new (std::nothrow) Plan());
     if (!plan) return MDIM_ERR_NOMEM;
     char why[160];
-    int st = plan_expr(e, flags, plan, why, sizeof why);
-    if (st) { delete plan; return set_error(ctx, st, why); }
-    if (plan->kind != KK_EMPTY && !out_device) { delete plan; return set_error(ctx, MDIM_ERR_INVALID, "null output buffer"); }
-    if (plan->kind != KK_EMPTY && plan->n_out > 1) { delete plan; return set_error(ctx, MDIM_ERR_INVALID, "a tuple-typed root needs mdim_collect_tuple (one output run per scalar leaf)"); }
-    if (plan->kind != KK_EMPTY && ((uintptr_t)out_device % (uintptr_t)plan->out_esize) != 0) { delete plan; return set_error(ctx, MDIM_ERR_INVALID, "output buffer is not aligned to its element size"); }
-    if (plan->kind != KK_EMPTY && ((uintptr_t)out_device % 16) != 0 && (plan->vec > 1 || plan->kind == KK_FOLD_ROWS || plan->kind == KK_FOLD_COLS)) {
-        // an element-aligned output (a slice of a caller's tensor): plan again with scalar stores
-        st = plan_expr(e, flags | kPlanScalarOut, plan, why, sizeof why);
-        if (st) { delete plan; return set_error(ctx, st, why); }
-    }
+    int st = plan_collect(e, flags, outs, n_outs, plan.get(), why, sizeof why);
+    if (st) return set_error(ctx, st, why);
+    if (plan->kind == KK_EMPTY) return MDIM_OK;
     cudaError_t ce = cudaSetDevice(ctx->device);
-    if (ce != cudaSuccess) { delete plan; return cuda_fail(ctx, ce, "cudaSetDevice"); }
-    st = collect_planned(ctx, plan, out_device, flags);
-    delete plan;
-    return st;
+    if (ce != cudaSuccess) return cuda_fail(ctx, ce, "cudaSetDevice");
+    return collect_planned(ctx, plan.get(), outs[0], flags);
+}
+
+int mdim_collect(mdim_ctx* ctx, const mdim_expr* e, void* out_device, uint32_t flags) {
+    if (!ctx) return MDIM_ERR_INVALID;
+    return collect(ctx, e, &out_device, 1, flags);
 }
 
 int mdim_collect_tuple(mdim_ctx* ctx, const mdim_expr* e, void* const* outs_device, int n_outs, uint32_t flags) {
     if (!ctx || !outs_device || n_outs < 1 || n_outs > MDIM_MAX_OUTS) return MDIM_ERR_INVALID;
-    Plan* plan = new (std::nothrow) Plan();
-    if (!plan) return MDIM_ERR_NOMEM;
-    char why[160];
-    int st = plan_expr(e, flags, plan, why, sizeof why);
-    if (st) { delete plan; return set_error(ctx, st, why); }
-    if (plan->kind == KK_EMPTY) { delete plan; return MDIM_OK; }
-    if (plan->n_out != n_outs) { delete plan; return set_error(ctx, MDIM_ERR_INVALID, "the number of output runs does not match the TUPLE root"); }
-    bool aligned16 = true;
-    for (int k = 0; k < n_outs; ++k) {
-        if (!outs_device[k] || ((uintptr_t)outs_device[k] % (uintptr_t)plan->out_esizes[k]) != 0) { delete plan; return set_error(ctx, MDIM_ERR_INVALID, "null or misaligned output run"); }
-        aligned16 = aligned16 && ((uintptr_t)outs_device[k] % 16) == 0;
-    }
-    if (!aligned16 && plan->vec > 1) {
-        st = plan_expr(e, flags | kPlanScalarOut, plan, why, sizeof why);
-        if (st) { delete plan; return set_error(ctx, st, why); }
-    }
-    for (int k = 1; k < n_outs; ++k) plan->prog.out_more[k - 1] = outs_device[k];
-    cudaError_t ce = cudaSetDevice(ctx->device);
-    if (ce != cudaSuccess) { delete plan; return cuda_fail(ctx, ce, "cudaSetDevice"); }
-    st = collect_planned(ctx, plan, outs_device[0], flags);
-    delete plan;
-    return st;
+    return collect(ctx, e, outs_device, n_outs, flags);
 }
 
 int mdim_plan_describe_nodevice(const mdim_expr* e, uint32_t flags, char* buf, size_t buf_len) {
     if (!buf || !buf_len) return MDIM_ERR_INVALID;
-    Plan* plan = new (std::nothrow) Plan();
+    std::unique_ptr<Plan> plan(new (std::nothrow) Plan());
     if (!plan) return MDIM_ERR_NOMEM;
     char why[160];
-    int st = plan_expr(e, flags, plan, why, sizeof why);
+    int st = plan_expr(e, flags, plan.get(), why, sizeof why);
     if (st) snprintf(buf, buf_len, "%s", why);
-    else {
-        const EvalVariant* v = (plan->kind == KK_GENERIC || plan->kind == KK_STREAM) ? select_variant(*plan, false) : nullptr;
+    else if ((plan->kind == KK_GENERIC || plan->kind == KK_STREAM) && plan->variant >= 0) {
         const bool may_jit = plan->static_id < 0 && !(flags & (MDIM_COLLECT_NO_STATIC | MDIM_COLLECT_NO_JIT));
-        if (v) snprintf(buf, buf_len, "%s [%s r%d%s]", plan->describe, v->name, v->maxr, may_jit ? ", specialised on first use" : "");
-        else snprintf(buf, buf_len, "%s", plan->describe);
-    }
-    delete plan;
+        const EvalVariant& v = kEvalVariants[plan->variant];
+        snprintf(buf, buf_len, "%s [%s r%d%s]", plan->describe, v.name, v.maxr, may_jit ? ", specialised on first use" : "");
+    } else snprintf(buf, buf_len, "%s", plan->describe);
     return st;
 }
 
 int mdim_jit_check_nodevice(const mdim_expr* e, uint32_t flags, char* log, size_t log_len) {
-    Plan* plan = new (std::nothrow) Plan();
+    std::unique_ptr<Plan> plan(new (std::nothrow) Plan());
     if (!plan) return MDIM_ERR_NOMEM;
     char why[160];
-    int st = plan_expr(e, flags, plan, why, sizeof why);
-    if (st) { if (log && log_len) snprintf(log, log_len, "%s", why); delete plan; return st; }
-    st = jit_compile_check(*plan, log, log_len);
-    delete plan;
-    return st;
+    int st = plan_expr(e, flags, plan.get(), why, sizeof why);
+    if (st) { if (log && log_len) snprintf(log, log_len, "%s", why); return st; }
+    return jit_compile_check(*plan, log, log_len);
 }
 
 int mdim_plan_describe(mdim_ctx* ctx, const mdim_expr* e, uint32_t flags, char* buf, size_t buf_len) {
@@ -599,63 +477,6 @@ struct HostBuf {       // one distinct host operand (several nodes may view the 
     char* stage[2];    // staging (chunked)
 };
 
-struct NodeRange { int64_t lo, hi; };  // [lo, hi) over all coordinates, relative to element 0 of the buffer
-
-// Per node, the coordinate range [lo, hi) of every iteration axis over which the node is evaluated: the
-// whole axis, except under a CONCAT, whose V side sees [0, len(V)) and whose W side [len(V), end).
-struct AxisRange { uint64_t lo[MDIM_MAX_RANK], hi[MDIM_MAX_RANK]; };
-
-void node_axis_ranges(const mdim_expr* e, std::vector<AxisRange>& out) {
-    const int total = e->rank + e->red_rank;
-    out.assign(e->n_nodes, AxisRange{});
-    std::vector<std::vector<int>> kids(e->n_nodes);
-    std::vector<int> stack;
-    for (int i = 0; i < e->n_nodes; ++i) {
-        const mdim_node& n = e->nodes[i];
-        int k = 0;
-        switch (n.kind) {
-            case MDIM_NODE_UNARY: case MDIM_NODE_DIAG: case MDIM_NODE_FOLD: k = 1; break;
-            case MDIM_NODE_BINARY: case MDIM_NODE_CONCAT: k = 2; break;
-            case MDIM_NODE_GATHER: k = n.n_comp; break;
-            default: k = 0;
-        }
-        for (int c = 0; c < k; ++c) kids[i].push_back(stack[stack.size() - k + c]);
-        stack.resize(stack.size() - k);
-        stack.push_back(i);
-    }
-    for (int a = 0; a < total; ++a) { out[e->n_nodes - 1].lo[a] = 0; out[e->n_nodes - 1].hi[a] = e->length[a]; }
-    for (int i = e->n_nodes - 1; i >= 0; --i) {  // parents before children in reverse post-order
-        const mdim_node& n = e->nodes[i];
-        for (size_t c = 0; c < kids[i].size(); ++c) {
-            AxisRange r = out[i];
-            if (n.kind == MDIM_NODE_CONCAT) {
-                const int a = n.axis_a[0];
-                if (c == 0) r.hi[a] = std::min<uint64_t>(r.hi[a], n.axis_c[0]);
-                else r.lo[a] = std::max<uint64_t>(r.lo[a], n.axis_c[0]);
-            }
-            out[kids[i][c]] = r;
-        }
-    }
-}
-
-// reach of offset + sum(coord[a] * stride[a]) over axes [first, total) (+ gather components)
-NodeRange node_reach(const mdim_expr* e, const mdim_node& n, const AxisRange& r, int first) {
-    int64_t lo = n.offset, hi = n.offset;
-    const int total = e->rank + e->red_rank;
-    for (int a = first; a < total; ++a) {
-        if (r.hi[a] <= r.lo[a]) continue;  // never evaluated along this axis: contributes nothing
-        const int64_t s0 = (int64_t)r.lo[a] * n.stride[a], s1 = (int64_t)(r.hi[a] - 1) * n.stride[a];
-        lo += std::min(s0, s1); hi += std::max(s0, s1);
-    }
-    if (n.kind == MDIM_NODE_GATHER)
-        for (int c = 0; c < n.n_comp; ++c) {
-            if (n.bound[c] == 0) continue;
-            const int64_t span = (int64_t)(n.bound[c] - 1) * n.gstride[c];
-            if (span > 0) hi += span; else lo += span;
-        }
-    return NodeRange{lo, hi + 1};
-}
-
 int ensure_pipe(mdim_ctx* ctx, size_t arena_bytes) {
     HostPipe& hp = ctx->pipe;
     if (!hp.h2d) {
@@ -681,15 +502,14 @@ size_t align_up(size_t x, size_t a) { return (x + a - 1) / a * a; }
 
 extern "C" int mdim_collect_host(mdim_ctx* ctx, const mdim_expr* e, void* out_host, uint32_t flags) {
     if (!ctx) return MDIM_ERR_INVALID;
-    Plan* plan = new (std::nothrow) Plan();
+    std::unique_ptr<Plan> plan(new (std::nothrow) Plan());  // validates the descriptor here, then plans each chunk
     if (!plan) return MDIM_ERR_NOMEM;
     char why[160];
-    int st = plan_expr(e, flags, plan, why, sizeof why);  // validates the descriptor
-    if (st) { delete plan; return set_error(ctx, st, why); }
-    const bool empty = plan->kind == KK_EMPTY;
-    delete plan;
-    if (empty) return MDIM_OK;
+    int st = plan_expr(e, flags, plan.get(), why, sizeof why);
+    if (st) return set_error(ctx, st, why);
+    if (plan->kind == KK_EMPTY) return MDIM_OK;
     if (!out_host) return set_error(ctx, MDIM_ERR_INVALID, "null output buffer");
+    if (plan->n_out > 1) return set_error(ctx, MDIM_ERR_INVALID, "a tuple-typed root in a host collect (mdim_collect_tuple collects its runs)");
     CU(ctx, cudaSetDevice(ctx->device));
     st = drain(ctx);
     if (st) return st;
@@ -705,8 +525,8 @@ extern "C" int mdim_collect_host(mdim_ctx* ctx, const mdim_expr* e, void* out_ho
     std::vector<HostBuf> bufs;
     std::vector<int> node_buf(e->n_nodes, -1);
     bool can_chunk = e->rank >= 1 && n0 >= 2;
-    std::vector<AxisRange> ranges;
-    node_axis_ranges(e, ranges);
+    std::vector<AxisRange> ranges(e->n_nodes);
+    node_axis_ranges(e, ranges.data());
     for (int i = 0; i < e->n_nodes; ++i) {
         const mdim_node& n = e->nodes[i];
         if (n.kind == MDIM_NODE_CONCAT && n.axis_a[0] == 0) can_chunk = false;  // range test on the chunked coordinate
@@ -717,12 +537,12 @@ extern "C" int mdim_collect_host(mdim_ctx* ctx, const mdim_expr* e, void* out_ho
         }
         if (n.kind != MDIM_NODE_LEAF && n.kind != MDIM_NODE_GATHER) continue;
         if (n.n_peers > 1) return set_error(ctx, MDIM_ERR_INVALID, "peer-sharded source in a host collect");
-        const NodeRange all = node_reach(e, n, ranges[i], 0);
+        const ElemRange all = operand_reach(e, n, ranges[i], 0);
         int b = -1;
         for (size_t k = 0; k < bufs.size(); ++k) if (bufs[k].base == (const char*)n.data) b = (int)k;
         const int es = dtype_size(n.dtype);
         const bool slabbed = n.kind == MDIM_NODE_LEAF && n.stride[0] > 0;
-        NodeRange slab = slabbed ? node_reach(e, n, ranges[i], 1) : NodeRange{0, 0};
+        const ElemRange slab = slabbed ? operand_reach(e, n, ranges[i], 1) : ElemRange{0, 0};
         bool disjoint = slabbed && slab.hi - slab.lo <= n.stride[0];
         for (int a = 1; a < total && disjoint; ++a) if (n.stride[a] < 0) disjoint = false;
         if (b < 0) {
@@ -819,14 +639,12 @@ extern "C" int mdim_collect_host(mdim_ctx* ctx, const mdim_expr* e, void* out_ho
         char* out_dev = hp.arena + sets_at + set_bytes * s + off_out;
         CU(ctx, cudaStreamWaitEvent(compute, hp.up[s], 0));
         if (pipelined && c >= (uint64_t)n_sets) CU(ctx, cudaStreamWaitEvent(compute, hp.down[s], 0));
-        Plan* p = new (std::nothrow) Plan();
-        if (!p) return MDIM_ERR_NOMEM;
-        int rc = plan_expr(&sub, flags, p, why, sizeof why);
-        if (rc) { delete p; return set_error(ctx, rc, why); }
+        void* outs[1] = {out_dev};
+        int rc = plan_collect(&sub, flags, outs, 1, plan.get(), why, sizeof why);
+        if (rc) return set_error(ctx, rc, why);
         ctx->pos_base = r0 * row_elems;
-        rc = collect_planned(ctx, p, out_dev, pipelined ? (flags | MDIM_COLLECT_ASYNC) : (flags & ~MDIM_COLLECT_ASYNC));
+        rc = collect_planned(ctx, plan.get(), out_dev, pipelined ? (flags | MDIM_COLLECT_ASYNC) : (flags & ~MDIM_COLLECT_ASYNC));
         ctx->pos_base = 0;
-        delete p;
         if (rc) return rc;
         CU(ctx, cudaEventRecord(hp.done[s], compute));
         CU(ctx, cudaStreamWaitEvent(hp.d2h, hp.done[s], 0));

@@ -314,7 +314,8 @@ __global__ void __launch_bounds__(256) k_fold_regs(const __grid_constant__ FoldR
     }
 }
 
-template <bool FAST> static bool launch_regs(const FoldRowsPlan& R, void* out, cudaStream_t stream) {
+// -> false: the register form does not take this row length or row count (*e: the launch's result otherwise)
+template <bool FAST> static bool launch_regs(const FoldRowsPlan& R, void* out, cudaStream_t stream, cudaError_t* e) {
     const uint32_t L = R.row_len / 32;  // row_len = 4 elements x 8 chunks x L lanes
     if (R.row_len % 32 != 0 || L < 1 || L > 32 || (L & (L - 1)) != 0) return false;
     const uint64_t warps = (R.n_rows + (32 / L) - 1) / (32 / L);
@@ -322,19 +323,21 @@ template <bool FAST> static bool launch_regs(const FoldRowsPlan& R, void* out, c
     if (ctas > 0x7fffffffull) return false;
     const dim3 grid((unsigned)ctas), block(256);
     switch (L) {
-        case 1: launch_pdl(k_fold_regs<1, FAST>, grid, block, 0, stream, R, out); break;
-        case 2: launch_pdl(k_fold_regs<2, FAST>, grid, block, 0, stream, R, out); break;
-        case 4: launch_pdl(k_fold_regs<4, FAST>, grid, block, 0, stream, R, out); break;
-        case 8: launch_pdl(k_fold_regs<8, FAST>, grid, block, 0, stream, R, out); break;
-        case 16: launch_pdl(k_fold_regs<16, FAST>, grid, block, 0, stream, R, out); break;
-        default: launch_pdl(k_fold_regs<32, FAST>, grid, block, 0, stream, R, out); break;
+        case 1: *e = launch_pdl(k_fold_regs<1, FAST>, grid, block, 0, stream, R, out); break;
+        case 2: *e = launch_pdl(k_fold_regs<2, FAST>, grid, block, 0, stream, R, out); break;
+        case 4: *e = launch_pdl(k_fold_regs<4, FAST>, grid, block, 0, stream, R, out); break;
+        case 8: *e = launch_pdl(k_fold_regs<8, FAST>, grid, block, 0, stream, R, out); break;
+        case 16: *e = launch_pdl(k_fold_regs<16, FAST>, grid, block, 0, stream, R, out); break;
+        default: *e = launch_pdl(k_fold_regs<32, FAST>, grid, block, 0, stream, R, out); break;
     }
     return true;
 }
 
 }  // namespace
 
-const char* launch_fold_rows(const FoldRowsPlan& R, void* out, int sm_count, cudaStream_t stream) {
+const char* launch_fold_rows(const Plan& p, void* out, bool nowait, cudaStream_t stream, int sm_count) {
+    FoldRowsPlan R = p.fr;
+    R.nowait = nowait;
     // column chunk: the whole row when a 32-row tile of it fits 64 KB (and always for the fused form,
     // which needs the whole row resident); else 256 columns per item
     int ch = (int)R.row_len;
@@ -361,7 +364,8 @@ const char* launch_fold_rows(const FoldRowsPlan& R, void* out, int sm_count, cud
     // the TMA / shared-memory form for the fold alone (config 4a: 6.28 vs 5.66 TB/s).
     static const int mode = [] { const char* e = getenv("MDIM_FOLD_MODE"); return e ? atoi(e) : 0; }();  // 1 = always smem, 2 = always registers
     const bool want_regs = mode == 2 || (mode == 0 && R.epilogue != 0);
-    if (want_regs && (fast ? launch_regs<true>(R, out, stream) : launch_regs<false>(R, out, stream))) return "k_fold_regs";
+    cudaError_t e = cudaSuccess;
+    if (want_regs && (fast ? launch_regs<true>(R, out, stream, &e) : launch_regs<false>(R, out, stream, &e))) return e == cudaSuccess ? "k_fold_regs" : nullptr;
     // i / q4 for the flat epilogue walk: umulhi(i, mul) >> shr, exact for i < 2^31 (q4 >= 2 here)
     uint32_t q4 = (uint32_t)ch / 4, lg = 0;
     while ((1u << lg) < q4) ++lg;
@@ -369,10 +373,10 @@ const char* launch_fold_rows(const FoldRowsPlan& R, void* out, int sm_count, cud
     const uint32_t q4_mul = (uint32_t)(((1ull << (31 + lg)) + q4 - 1) / q4);
     auto go = [&](auto kern) {
         cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
-        launch_pdl(kern, dim3(grid), dim3(kFoldThreads), smem, stream, R, out, n_warps, stages, ch, skew, q4_mul, q4_shr);
+        return launch_pdl(kern, dim3(grid), dim3(kFoldThreads), smem, stream, R, out, n_warps, stages, ch, skew, q4_mul, q4_shr);
     };
-    if (fast) go(k_fold_rows<true>); else go(k_fold_rows<false>);
-    return "k_fold_rows";
+    e = fast ? go(k_fold_rows<true>) : go(k_fold_rows<false>);
+    return e == cudaSuccess ? "k_fold_rows" : nullptr;
 }
 
 }  // namespace mdim

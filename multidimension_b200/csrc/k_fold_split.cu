@@ -271,7 +271,14 @@ SplitKernel pick_src(int es, int op, int layout) {
 
 }  // namespace
 
-SplitGeometry fold_split_geometry(const FoldSplitPlan& F, int sm_count) {
+struct SplitGeometry {
+    uint64_t units;     // RUNS: outputs; COLS: batches.  Each has one ticket.
+    uint64_t n_chunks;  // chunks per unit: the grid is units x n_chunks CTAs
+    uint64_t chunk;     // RUNS: elements per chunk; COLS: rows per chunk
+    uint64_t partials;  // slots of scratch the launch writes (each slot_bytes wide)
+};
+
+static SplitGeometry fold_split_geometry(const FoldSplitPlan& F, int sm_count) {
     SplitGeometry G;
     const uint64_t target = (uint64_t)std::max(sm_count, 1) * kSplitCtasPerSm;
     const int es = dtype_size(F.src_dtype);
@@ -295,17 +302,24 @@ SplitGeometry fold_split_geometry(const FoldSplitPlan& F, int sm_count) {
     return G;
 }
 
+size_t fold_split_scratch_bytes(const FoldSplitPlan& F, int sm_count) {
+    return kSplitMaxOuts * sizeof(unsigned int) + fold_split_geometry(F, sm_count).partials * 8;
+}
+
 static const char* const kOpName[] = {"add", "mul", "and", "or", "xor"};
 
-const char* launch_fold_split(const FoldSplitPlan& F, const SplitGeometry& G, void* out, unsigned int* tickets, void* partials,
-                              cudaStream_t stream, char* name, size_t name_len) {
+const char* launch_fold_split(const Plan& p, void* out, bool nowait, cudaStream_t stream, int sm_count, char* scratch) {
+    FoldSplitPlan F = p.fs;
+    F.nowait = nowait;
+    const SplitGeometry G = fold_split_geometry(F, sm_count);
     const int op = F.op == MDIM_MUL ? SOP_MUL : F.op == MDIM_AND ? SOP_AND : F.op == MDIM_OR ? SOP_OR : F.op == MDIM_XOR ? SOP_XOR : SOP_ADD;
     const int es = dtype_size(F.src_dtype);
     const SplitKernel k = F.slot_bytes == 8 ? pick_src<unsigned long long>(es, op, F.layout) : pick_src<unsigned int>(es, op, F.layout);
-    const cudaError_t e = launch_pdl(k, dim3((unsigned)(G.units * G.n_chunks)), dim3(kSplitThreads), 0, stream, F, out, tickets, partials,
-                                     (uint64_t)G.chunk, (uint32_t)G.n_chunks);
+    const cudaError_t e = launch_pdl(k, dim3((unsigned)(G.units * G.n_chunks)), dim3(kSplitThreads), 0, stream, F, out, (unsigned int*)scratch,
+                                     (void*)(scratch + kSplitMaxOuts * sizeof(unsigned int)), (uint64_t)G.chunk, (uint32_t)G.n_chunks);
     if (e != cudaSuccess) return nullptr;
-    snprintf(name, name_len, "k_fold_split<u%d,src=u%d,%s,%s>", F.slot_bytes * 8, es * 8, kOpName[op], F.layout == SPLIT_RUNS ? "runs" : "cols");
+    static thread_local char name[48];
+    snprintf(name, sizeof name, "k_fold_split<u%d,src=u%d,%s,%s>", F.slot_bytes * 8, es * 8, kOpName[op], F.layout == SPLIT_RUNS ? "runs" : "cols");
     return name;
 }
 

@@ -317,13 +317,14 @@ int launch_fold_xchg(const FoldXchgArgs& A, int dtype, int op, int sm_count, cud
 }
 
 // The column walk on one GPU (KK_FOLD_COLS, planned in plan.cpp): no packets, no co-residency requirement.
-const char* launch_fold_cols(const FoldColsPlan& C, void* out, cudaStream_t stream) {
+const char* launch_fold_cols(const Plan& p, void* out, bool nowait, cudaStream_t stream, int) {
+    const FoldColsPlan& C = p.fc;
     XchgKernel fn = pick_kernel<false>(C.dtype, C.op);
     if (!fn) return nullptr;
     FoldXchgArgs A;
     memset(&A, 0, sizeof A);
     A.n_rows = C.n_rows; A.row_bytes = C.row_bytes; A.pitch_bytes = C.pitch_bytes;
-    A.world = 1; A.start = C.init; A.rows = C.src; A.out = out; A.nowait = C.nowait;
+    A.world = 1; A.start = C.init; A.rows = C.src; A.out = out; A.nowait = nowait;
     A.n_batch = C.n_batch ? C.n_batch : 1; A.batch_pitch_bytes = C.batch_pitch_bytes;
     A.wide = !(((uintptr_t)C.src & 31) || (C.pitch_bytes & 31) || (A.n_batch > 1 && (C.batch_pitch_bytes & 31)));
     const uint64_t n_groups = (C.row_bytes + 31) / 32 * A.n_batch, n_slices = (n_groups + kXThreads - 1) / kXThreads;

@@ -27,31 +27,28 @@ k_eval(const __grid_constant__ Program P, void* __restrict__ out, ErrWord* __res
 
 using EvalKernel = void (*)(const Program, void*, ErrWord*, uint64_t, uint64_t);
 
-struct EvalVariant {
-    const char* name;
-    int slot_bytes, vec, max_depth, wide, maxr;  // maxr: iteration axes walked (1 = contiguous stream)
-    const SigInstr* sig;  // nullptr = interpreter
-    int sig_n;
-    EvalKernel fn;
-};
+// The kernels of the variants_*.inc lists, in list order, defined in k_eval_{s32,s64}_{interp,static}.cu (four translation units:
+// the build parallelises over them).  Concatenated s32 static, s64 static, s32 interp, s64 interp they follow kEvalVariants.
+const EvalKernel* eval_kernels_s32_interp(int* n);
+const EvalKernel* eval_kernels_s32_static(int* n);
+const EvalKernel* eval_kernels_s64_interp(int* n);
+const EvalKernel* eval_kernels_s64_static(int* n);
 
-// defined in k_eval_{s32,s64}_{interp,static}.cu (four translation units: the build parallelises over them)
-const EvalVariant* eval_variants_s32_interp(int* n);
-const EvalVariant* eval_variants_s32_static(int* n);
-const EvalVariant* eval_variants_s64_interp(int* n);
-const EvalVariant* eval_variants_s64_static(int* n);
+// The launchers of the dedicated kernels (KK_TRANSPOSE, KK_FOLD_ROWS, KK_FOLD_COLS, KK_FOLD_SPLIT) share one shape: each launches its
+// plan's kernel on `stream`, without griddepcontrol.wait if `nowait` (launch.cuh), and returns the name of the kernel launched,
+// nullptr on a launch error.
 
 // ------------------------------------------------------------------------------------------------
 // K2: tiled transpose of one leaf (see k_transpose.cu)
 // ------------------------------------------------------------------------------------------------
 constexpr int kTrThreads = 256;
-const char* launch_transpose(const TransposePlan& T, void* out, int grid, cudaStream_t stream);  // -> name of the kernel launched
+const char* launch_transpose(const Plan& p, void* out, bool nowait, cudaStream_t stream, int sm_count);
 
 // ------------------------------------------------------------------------------------------------
 // K4: sequential-order last-axis fold, optionally fused with a broadcast epilogue (k_fold.cu)
 // ------------------------------------------------------------------------------------------------
 constexpr int kFoldThreads = 256;
-const char* launch_fold_rows(const FoldRowsPlan& R, void* out, int sm_count, cudaStream_t stream);  // -> name of the kernel launched
+const char* launch_fold_rows(const Plan& p, void* out, bool nowait, cudaStream_t stream, int sm_count);
 
 // ------------------------------------------------------------------------------------------------
 // Fold over the SHARDED axis, bit-exact, pipelined through the ranks over NVLink (k_fold_ring.cu)
@@ -60,21 +57,14 @@ int launch_fold_ring(const FoldRingArgs& A, const void* rows, int sm_count, cuda
 
 // Fold over the SHARDED axis, blocked by rank + in-kernel all-reduce in rank order over NVLink (k_fold_xchg.cu)
 int launch_fold_xchg(const FoldXchgArgs& A, int dtype, int op, int sm_count, cudaStream_t stream);
-// ... and the same column walk on one GPU, no exchange (KK_FOLD_COLS): -> name of the kernel launched, nullptr on a launch error
-const char* launch_fold_cols(const FoldColsPlan& C, void* out, cudaStream_t stream);
+// ... and the same column walk on one GPU, no exchange (KK_FOLD_COLS)
+const char* launch_fold_cols(const Plan& p, void* out, bool nowait, cudaStream_t stream, int sm_count);
 
 // ------------------------------------------------------------------------------------------------
 // Integer fold with few outputs and a long reduction, the reduction cut into chunks over the whole GPU (k_fold_split.cu)
 // ------------------------------------------------------------------------------------------------
-struct SplitGeometry {
-    uint64_t units;     // RUNS: outputs; COLS: batches.  Each has one ticket.
-    uint64_t n_chunks;  // chunks per unit: the grid is units x n_chunks CTAs
-    uint64_t chunk;     // RUNS: elements per chunk; COLS: rows per chunk
-    uint64_t partials;  // slots of scratch the launch writes (each slot_bytes wide)
-};
-SplitGeometry fold_split_geometry(const FoldSplitPlan& F, int sm_count);
-// tickets: units zeroed words; partials: G.partials slots.  -> name of the instantiation launched, nullptr on a launch error
-const char* launch_fold_split(const FoldSplitPlan& F, const SplitGeometry& G, void* out, unsigned int* tickets, void* partials,
-                              cudaStream_t stream, char* name, size_t name_len);
+// Its scratch holds kSplitMaxOuts tickets, zeroed before first use and left at zero by every launch, then the chunks' partials.
+size_t fold_split_scratch_bytes(const FoldSplitPlan& F, int sm_count);
+const char* launch_fold_split(const Plan& p, void* out, bool nowait, cudaStream_t stream, int sm_count, char* scratch);
 
 }  // namespace mdim

@@ -4,8 +4,9 @@
 // a run-time descriptor: it validates the post-order node array, canonicalises the iteration
 // space (drops length-1 axes, merges jointly-contiguous neighbours — `Iso`/`Coat` regroupings
 // and contiguous arrays of any rank collapse to rank 1), picks the vector width and per-leaf load
-// mode, emits the postfix device program, and recognises the shapes that have a dedicated kernel
-// (tiled transpose, last-axis fold).  Host-only code; no CUDA calls.
+// mode, emits the postfix device program, selects the k_eval instantiation that runs it, and
+// recognises the shapes that have a dedicated kernel (tiled transpose, folds).  It also checks a
+// collect's output runs (plan_collect).  Host-only code; no CUDA calls.
 #include <stdarg.h>
 #include <stdio.h>
 #include <stdlib.h>
@@ -15,6 +16,7 @@
 #include <vector>
 
 #include "program.hpp"
+#include "sigs.hpp"
 
 namespace mdim {
 
@@ -55,6 +57,114 @@ static int node_arity(const mdim_node& n) {
         case MDIM_NODE_TUPLE: return n.n_comp;
     }
     return -1;
+}
+
+void node_axis_ranges(const mdim_expr* e, AxisRange* out) {
+    int parent[MDIM_MAX_NODES], side[MDIM_MAX_NODES], stack[MDIM_MAX_NODES], sp = 0;
+    for (int i = 0; i < e->n_nodes; ++i) {  // a validated descriptor: every node finds its operands on the stack
+        const int k = node_arity(e->nodes[i]);
+        sp -= k;
+        for (int c = 0; c < k; ++c) { parent[stack[sp + c]] = i; side[stack[sp + c]] = c; }
+        stack[sp++] = i;
+    }
+    AxisRange& root = out[e->n_nodes - 1];
+    root = AxisRange{};
+    for (int a = 0; a < e->rank + e->red_rank; ++a) root.hi[a] = e->length[a];
+    for (int i = e->n_nodes - 2; i >= 0; --i) {  // post-order: a parent comes after its children
+        const mdim_node& p = e->nodes[parent[i]];
+        out[i] = out[parent[i]];
+        if (p.kind == MDIM_NODE_CONCAT) {
+            const int a = p.axis_a[0];
+            if (side[i] == 0) out[i].hi[a] = std::min<uint64_t>(out[i].hi[a], p.axis_c[0]);
+            else out[i].lo[a] = std::max<uint64_t>(out[i].lo[a], p.axis_c[0]);
+        }
+    }
+}
+
+ElemRange operand_reach(const mdim_expr* e, const mdim_node& n, const AxisRange& r, int first_axis) {
+    int64_t lo = n.offset, hi = n.offset;
+    for (int a = first_axis; a < e->rank + e->red_rank; ++a) {
+        if (r.hi[a] <= r.lo[a]) continue;  // never evaluated along this axis: contributes nothing
+        const int64_t s0 = (int64_t)r.lo[a] * n.stride[a], s1 = (int64_t)(r.hi[a] - 1) * n.stride[a];
+        lo += std::min(s0, s1); hi += std::max(s0, s1);
+    }
+    if (n.kind == MDIM_NODE_GATHER)
+        for (int c = 0; c < n.n_comp; ++c) {
+            if (n.bound[c] == 0) continue;
+            const int64_t span = (int64_t)(n.bound[c] - 1) * n.gstride[c];
+            if (span > 0) hi += span; else lo += span;
+        }
+    return ElemRange{lo, hi + 1};
+}
+
+void explain_failure(const ErrWord& w, uint64_t pos, mdim_error_info* info) {
+    memset(info, 0, sizeof *info);
+    info->status = w.status ? w.status : MDIM_ERR_INVALID;
+    info->node = w.status ? w.node : -1;
+    info->position = pos;
+    info->value = w.value;
+    info->bound = w.bound;
+    info->component = w.component;
+    if (info->status == MDIM_ERR_OOB)  // src/int.rs:17
+        snprintf(info->message, sizeof info->message, "Index %llu is out of bounds for size %llu", (unsigned long long)info->value, (unsigned long long)info->bound);
+    else if (info->status == MDIM_ERR_ARITH)
+        snprintf(info->message, sizeof info->message, "attempt to divide by zero or with overflow");
+    else
+        snprintf(info->message, sizeof info->message, "device reported a failure at position %llu", (unsigned long long)pos);
+}
+
+// ---- evaluator instantiations ------------------------------------------------------------------
+template <class Sig> constexpr const SigInstr* sig_code() { if constexpr (Sig::n > 0) return Sig::code; else return nullptr; }
+
+const EvalVariant kEvalVariants[] = {
+#define X(Sig, S, V, MAXD, WIDE, MAXR) {#Sig, (int)sizeof(S), V, MAXD, WIDE ? 1 : 0, MAXR, sig_code<Sig>(), Sig::n},
+#include "variants_s32_static.inc"
+#include "variants_s64_static.inc"
+#include "variants_s32_interp.inc"
+#include "variants_s64_interp.inc"
+#undef X
+};
+const int kNumEvalVariants = (int)(sizeof(kEvalVariants) / sizeof(kEvalVariants[0]));
+
+void eval_variant_name(int variant, char* buf, size_t len) {
+    const EvalVariant& v = kEvalVariants[variant];
+    snprintf(buf, len, "k_eval<%s,s%d,v%d,d%d%s,r%d>", v.sig ? v.name : "interp", v.slot_bytes * 8, v.vec, v.max_depth, v.wide ? ",wide" : "", v.maxr);
+}
+
+static bool sig_matches(const EvalVariant& v, const char* sig, int sig_len) {
+    if (!v.sig || v.sig_n * 4 != sig_len) return false;
+    for (int i = 0; i < v.sig_n; ++i) {
+        const unsigned char* s = (const unsigned char*)sig + 4 * i;
+        if (v.sig[i].opc != s[0] || v.sig[i].dtype != s[1]) return false;
+        // op/aux only matter for the opcodes that read them
+        const int opc = v.sig[i].opc;
+        if ((opc == OPC_LEAF_VEC || opc == OPC_LEAF_BCAST || opc == OPC_LEAF_STRIDED) && v.sig[i].aux != s[3]) return false;  // aux: bit 0 cached, bit 1 sharded
+        if ((opc == OPC_BINARY || opc == OPC_UNARY || opc == OPC_FOLD_STEP) && (v.sig[i].op != s[2] || v.sig[i].aux != s[3])) return false;
+        if (opc == OPC_GATHER && v.sig[i].aux != s[3]) return false;
+    }
+    return true;
+}
+
+// A pre-built signature's smallest MAXR that covers the plan's axes (signatures have 32-bit coordinates only), else the
+// interpreter's smallest MAXR, then its smallest depth.  -1: no instantiation runs the plan.
+static int select_variant(const Plan& p, uint32_t flags) {
+    const int need = p.kind == KK_STREAM ? 1 : std::max(1, p.n_axes);
+    int best = -1;
+    if (!p.wide && !(flags & MDIM_COLLECT_NO_STATIC)) {
+        for (int i = 0; i < kNumEvalVariants; ++i) {
+            const EvalVariant& v = kEvalVariants[i];
+            if (v.slot_bytes != p.slot_bytes || v.vec != p.vec || v.wide || v.maxr < need || !sig_matches(v, p.sig, p.sig_len)) continue;
+            if (best < 0 || v.maxr < kEvalVariants[best].maxr) best = i;
+        }
+        if (best >= 0) return best;
+    }
+    for (int i = 0; i < kNumEvalVariants; ++i) {
+        const EvalVariant& v = kEvalVariants[i];
+        if (v.sig || v.slot_bytes != p.slot_bytes || v.vec != p.vec || v.wide != p.wide || v.maxr < need || v.max_depth < p.max_depth) continue;
+        const EvalVariant* b = best >= 0 ? &kEvalVariants[best] : nullptr;
+        if (!b || v.maxr < b->maxr || (v.maxr == b->maxr && v.max_depth < b->max_depth)) best = i;
+    }
+    return best;
 }
 
 namespace {
@@ -571,7 +681,6 @@ int Builder::emit() {
 
 // ---- fast paths -------------------------------------------------------------------------------
 int Builder::detect_fast_paths() {
-    Program& P = plan->prog;
     const mdim_node* N = e->nodes;
     const int root = e->n_nodes - 1;
     if (N[root].kind == MDIM_NODE_TUPLE) return MDIM_OK;  // several outputs: the evaluator only
@@ -621,11 +730,10 @@ int Builder::detect_fast_paths() {
         const int fc = child[fold_node][0];
         const uint64_t row_len = len[n_axes - 1];
         const int es = dtype_size(F.dtype);
-        auto rows_leaf = [&](int ni, bool with_red, int out_rank_expected) -> bool {
+        auto rows_leaf = [&](int ni, bool with_red) -> bool {
             // contiguous (rows, row_len) leaf: red stride 1 (if with_red) and row stride row_len
             if (N[ni].kind != MDIM_NODE_LEAF || N[ni].dtype != F.dtype || N[ni].n_peers > 1) return false;
             const int64_t* s = cstride[ni];
-            (void)out_rank_expected;
             if (with_red && s[n_axes - 1] != 1) return false;
             return true;
         };
@@ -637,7 +745,7 @@ int Builder::detect_fast_paths() {
             R.row_len = (uint32_t)row_len; R.op = F.op; R.dtype = F.dtype; R.init = F.imm.u64 & 0xffffffffull;
             const bool src_aligned = (((uintptr_t)N[fc].data + (uintptr_t)(N[fc].offset * es)) % 16) == 0;
             // (2a) fold only: out rank 1 (rows), leaf strides (row_len | 1)
-            if (root == fold_node && rank == 1 && rows_leaf(fc, true, 1) && cstride[fc][0] == (int64_t)row_len && src_aligned) {
+            if (root == fold_node && rank == 1 && rows_leaf(fc, true) && cstride[fc][0] == (int64_t)row_len && src_aligned) {
                 R.src = N[fc].data; R.src_offset = N[fc].offset; R.n_rows = len[0]; R.epilogue = 0;
                 plan->kind = KK_FOLD_ROWS;
                 snprintf(plan->describe, sizeof plan->describe, "fold_rows rows=%llu len=%u op=%d", (unsigned long long)R.n_rows, R.row_len, R.op);
@@ -695,7 +803,6 @@ int Builder::detect_fast_paths() {
             }
         }
     }
-    (void)P;
     return MDIM_OK;
 }
 
@@ -773,28 +880,18 @@ static void input_ranges(const mdim_expr* e, Plan* plan) {
         if (plan->n_in_ranges == kMaxRanges) { plan->n_in_ranges = -1; return; }
         plan->in_range[plan->n_in_ranges++] = MemRange{lo, hi};
     };
-    const int n_axes = e->rank + e->red_rank;
+    AxisRange whole{};
+    for (int a = 0; a < e->rank + e->red_rank; ++a) whole.hi[a] = e->length[a];
     for (int i = 0; i < e->n_nodes; ++i) {
         const mdim_node& n = e->nodes[i];
         if (n.kind != MDIM_NODE_LEAF && n.kind != MDIM_NODE_GATHER) continue;
-        const uint64_t es = (uint64_t)dtype_size(n.dtype);
+        const int64_t es = dtype_size(n.dtype);
         if (n.n_peers > 1) {
             for (int p = 0; p < n.n_peers; ++p) push((uint64_t)(uintptr_t)n.peer[p], (uint64_t)(uintptr_t)n.peer[p] + n.peer_block * es);
             continue;
         }
-        int64_t lo = n.offset, hi = n.offset;
-        for (int a = 0; a < n_axes; ++a) {
-            if (e->length[a] == 0) continue;
-            const int64_t ext = n.stride[a] * (int64_t)(e->length[a] - 1);
-            if (ext > 0) hi += ext; else lo += ext;
-        }
-        if (n.kind == MDIM_NODE_GATHER)
-            for (int c = 0; c < n.n_comp; ++c) {
-                if (n.bound[c] == 0) continue;
-                const int64_t ext = n.gstride[c] * (int64_t)(n.bound[c] - 1);
-                if (ext > 0) hi += ext; else lo += ext;
-            }
-        push((uint64_t)((int64_t)(uintptr_t)n.data + lo * (int64_t)es), (uint64_t)((int64_t)(uintptr_t)n.data + (hi + 1) * (int64_t)es));
+        const ElemRange r = operand_reach(e, n, whole, 0);
+        push((uint64_t)((int64_t)(uintptr_t)n.data + r.lo * es), (uint64_t)((int64_t)(uintptr_t)n.data + r.hi * es));
     }
 }
 
@@ -803,7 +900,7 @@ int plan_expr(const mdim_expr* e, uint32_t flags, Plan* plan, char* why_buf, siz
     b->e = e; b->flags = flags; b->plan = plan; b->why = Why{why_buf, why_len};
     if (why_buf && why_len) why_buf[0] = 0;
     memset(plan, 0, sizeof *plan);
-    plan->static_id = -1;
+    plan->variant = plan->static_id = -1;
     plan->flags = flags;
     int st = b->validate();
     if (st) { delete b; return st; }
@@ -834,9 +931,9 @@ int plan_expr(const mdim_expr* e, uint32_t flags, Plan* plan, char* why_buf, siz
         if (st) { delete b; return st; }
     }
     plan->kind = (b->rank <= 1 && b->red_rank == 0) ? KK_STREAM : KK_GENERIC;
-    const int need_maxr = plan->kind == KK_STREAM ? 1 : std::max(1, plan->n_axes);
-    if (!(flags & MDIM_COLLECT_NO_STATIC))
-        plan->static_id = find_static_signature(plan->sig, plan->sig_len, plan->slot_bytes, plan->vec, need_maxr, plan->wide);
+    // chosen before the fast paths, so that every plan names the instantiation that would run its program
+    plan->variant = select_variant(*plan, flags);
+    if (plan->variant >= 0 && kEvalVariants[plan->variant].sig) plan->static_id = plan->variant;
     snprintf(plan->describe, sizeof plan->describe, "%s.%s s%d v%dx1%s rank=%d+%d depth=%d instr=%d",
              plan->kind == KK_STREAM ? "stream" : "generic", plan->static_id >= 0 ? "static" : "interp", plan->slot_bytes * 8, plan->vec,
              plan->wide ? " wide" : "", b->rank, b->red_rank, plan->max_depth, plan->prog.n_instr);
@@ -846,6 +943,28 @@ int plan_expr(const mdim_expr* e, uint32_t flags, Plan* plan, char* why_buf, siz
     }
     if (gather_big) plan->prog.flags |= PF_GATHER_BIG;
     delete b;
+    return MDIM_OK;
+}
+
+int plan_collect(const mdim_expr* e, uint32_t flags, void* const* outs, int n_outs, Plan* plan, char* why_buf, size_t why_len) {
+    int st = plan_expr(e, flags, plan, why_buf, why_len);
+    if (st || plan->kind == KK_EMPTY) return st;
+    Why why{why_buf, why_len};
+    if (plan->n_out != n_outs)
+        return why.fail(MDIM_ERR_INVALID, n_outs == 1 ? "a tuple-typed root needs mdim_collect_tuple (one output run per scalar leaf)"
+                                                      : "the number of output runs does not match the TUPLE root");
+    bool aligned16 = true;
+    for (int k = 0; k < n_outs; ++k) {
+        if (!outs[k]) return why.fail(MDIM_ERR_INVALID, "null output buffer");
+        if ((uintptr_t)outs[k] % (uintptr_t)plan->out_esizes[k]) return why.fail(MDIM_ERR_INVALID, "output buffer is not aligned to its element size");
+        aligned16 = aligned16 && (uintptr_t)outs[k] % 16 == 0;
+    }
+    if (!aligned16 && (plan->vec > 1 || plan->kind == KK_FOLD_ROWS || plan->kind == KK_FOLD_COLS)) {
+        // an element-aligned output (a slice of a caller's tensor): plan again with scalar stores
+        st = plan_expr(e, flags | kPlanScalarOut, plan, why_buf, why_len);
+        if (st) return st;
+    }
+    for (int k = 1; k < n_outs; ++k) plan->prog.out_more[k - 1] = outs[k];
     return MDIM_OK;
 }
 

@@ -154,7 +154,7 @@ struct TransposePlan {
     float peer_inv;              // 1 / peer_block (quotient estimate, corrected exactly in the kernel)
     uint64_t peer_block;
     const void* peer[MDIM_MAX_PEERS];
-    int32_t nowait;              // set per launch (api.cu): see launch.cuh
+    int32_t nowait;              // set per launch by its launcher: see launch.cuh
 };
 
 struct FoldRowsPlan {
@@ -171,7 +171,7 @@ struct FoldRowsPlan {
     int32_t post_op;      // optional binary op applied to the fold before the epilogue (e.g. DIV)
     int32_t has_post;
     uint64_t post_imm;    // ... with this constant on the right
-    int32_t nowait;       // set per launch (api.cu): see launch.cuh
+    int32_t nowait;       // set per launch by its launcher: see launch.cuh
 };
 
 struct FoldColsPlan {
@@ -183,7 +183,6 @@ struct FoldColsPlan {
     uint64_t batch_pitch_bytes;  // bytes between consecutive blocks (multiple of 16)
     int32_t op, dtype;
     uint64_t init;
-    int32_t nowait;       // set per launch (api.cu): see launch.cuh
 };
 
 // k_fold_split.cu: an integer fold whose operator is associative and commutative (wrapping Add, Mul, BitAnd, BitOr, BitXor; Sub as
@@ -201,7 +200,7 @@ struct FoldSplitPlan {
     int32_t op;             // MDIM_ADD, SUB, MUL, AND, OR, XOR
     int32_t dtype, src_dtype;  // the fold's dtype; the leaf's (a CAST body converts between them)
     int32_t slot_bytes;     // 4 or 8: the accumulator width (the fold's dtype, U8 widened to 4)
-    int32_t nowait;         // set per launch (api.cu): see launch.cuh
+    int32_t nowait;         // set per launch by its launcher: see launch.cuh
     uint64_t init;          // bits of the immediate init
     uint64_t red;           // RUNS: elements per run; COLS: rows
     uint64_t n_out;         // outputs, written contiguously
@@ -261,7 +260,8 @@ struct Plan {
     int32_t n_axes;      // rank + red_rank after canonicalisation (selects the MAXR instantiation)
     int32_t vec256_ok;   // every LEAF_VEC operand is 32-byte aligned (the output is checked at launch)
     int32_t max_depth;
-    int32_t static_id;   // index into the signature registry, -1 = interpreted
+    int32_t variant;     // the k_eval instantiation that serves the evaluator's program (index into kEvalVariants), -1 = none
+    int32_t static_id;   // = variant when that instantiation runs a pre-built signature, else -1 (interpreted)
     uint64_t out_elems;
     int32_t out_esize;
     int32_t n_out;                        // > 1: tuple-typed root
@@ -280,15 +280,40 @@ struct Plan {
 
 #ifndef __CUDACC_RTC__  // host-side declarations (this header is also compiled by NVRTC, see jit.cu)
 int plan_expr(const mdim_expr* e, uint32_t flags, Plan* plan, char* why, size_t why_len);
+// plan_expr for a collect into the output runs outs[0 .. n_outs) (one per scalar leaf of a TUPLE root, else one): checks each run
+// (not null, aligned to its element), plans again with scalar stores when a run is only element-aligned, and fills out_more[]
+int plan_collect(const mdim_expr* e, uint32_t flags, void* const* outs, int n_outs, Plan* plan, char* why, size_t why_len);
 int dtype_size(int dt);
 const char* status_string(int st);
+// mdim_error_info for a device-side failure at output position `pos`, from the error word of its PF_EXPLAIN rerun
+void explain_failure(const ErrWord& w, uint64_t pos, mdim_error_info* info);
 
-// Signature registry (defined with the kernels; the planner only needs lookup by bytes).
+// Every k_eval instantiation (kernels.cuh), as the planner selects among them: the variants_*.inc lists in the order s32 static,
+// s64 static, s32 interp, s64 interp, which is also the order of the kernels k_eval_*.cu export.
+struct SigInstr;
+struct EvalVariant {
+    const char* name;
+    int slot_bytes, vec, max_depth, wide, maxr;  // maxr: iteration axes walked (1 = contiguous stream)
+    const SigInstr* sig;  // nullptr = interpreter
+    int sig_n;
+};
+extern const EvalVariant kEvalVariants[];
+extern const int kNumEvalVariants;
+// the instantiation's template arguments, e.g. k_eval<SigSubBcastF32,s32,v8,d4,r3> or k_eval<interp,s64,v1,d8,wide,r8>
+void eval_variant_name(int variant, char* buf, size_t len);
+
+// Per iteration axis, the coordinates [lo, hi) over which a node is evaluated, and the elements [lo, hi) an operand reaches over
+// them, relative to its data pointer (offset + sum of stride * coordinate, plus the gathered components over [0, bound)).
+struct AxisRange { uint64_t lo[MDIM_MAX_RANK], hi[MDIM_MAX_RANK]; };
+struct ElemRange { int64_t lo, hi; };
+// the whole axes at the root, narrowed under a CONCAT: its V side sees [0, len(V)), its W side [len(V), end)
+void node_axis_ranges(const mdim_expr* e, AxisRange* out);  // out: e->n_nodes entries
+ElemRange operand_reach(const mdim_expr* e, const mdim_node& n, const AxisRange& r, int first_axis);  // axes [first_axis, rank + red_rank)
+
 // jit.cu: a kernel specialised at run time for the plan's op sequence, or nullptr (use the interpreter)
 // explain: the single-element rerun of a failed collect; it reuses a shape kernel already built but neither counts towards nor triggers one
 void* jit_kernel_for(const Plan& p, int* level = nullptr, bool explain = false);  // level: 0 none, 1 specialised on the op sequence, 2 on ops AND shape
 
-int find_static_signature(const char* sig, int sig_len, int slot_bytes, int vec, int need_maxr, int wide);
 // NVRTC half of jit_kernel_for alone (needs no GPU): 0 = the specialisation compiles for sm_100a
 int jit_compile_check(const Plan& p, char* log, size_t log_len);
 #endif

@@ -16,9 +16,9 @@ So every case here names
     nothing is fused), fancy indexing for strides and gathers, and the sequential fold of test_kernel_routes.
 
 The cases are hand-built descriptors (the C ABI the evaluator serves), so that every stride, offset, alignment and
-predicate is explicit.  On the CPU the host form of the same instantiation (tests/emu, which now builds every line of the
-`.inc` lists and picks one by the library's rules) must report the same kernel and, with the C oracle, equal the reference bit
-for bit.
+predicate is explicit.  On the CPU the host form of the same instantiation (tests/emu: the library's planner, which selects and
+names the instantiation, over a host build of every line of the `.inc` lists) must report the same kernel and, with the C
+oracle, equal the reference bit for bit.
 """
 import ctypes as C
 import functools
@@ -73,8 +73,8 @@ def _parse(name):
 
 
 def instantiation(sig, slot, vec, depth, wide, need):
-    """select_variant (api.cu) over the registry: the signature's smallest MAXR >= need, else the interpreter's smallest MAXR
-    and depth that cover the plan."""
+    """The selection rule, restated independently of the library's select_variant (plan.cpp): the signature's smallest
+    MAXR >= need, else the interpreter's smallest MAXR and depth that cover the plan."""
     cands = [(_parse(n), n) for n in registry()]
     if sig and not wide:
         ok = [(p["maxr"], n) for p, n in cands if p["sig"] == sig and p["slot"] == slot and p["vec"] == vec and p["maxr"] >= need]
