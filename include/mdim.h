@@ -68,7 +68,10 @@ typedef enum mdim_dtype {
     MDIM_U64 = 4,
     MDIM_F32 = 5,
     MDIM_F64 = 6,
-    MDIM_DTYPE_COUNT = 7
+    MDIM_I8 = 7,  /* 1- and 2-byte integers: a slot holds the raw bits, zero-extended (exec.cuh, "value semantics") */
+    MDIM_I16 = 8,
+    MDIM_U16 = 9,
+    MDIM_DTYPE_COUNT = 10
 } mdim_dtype;
 
 /* ---- binary operator vocabulary = the reference's uninstantiable enums, src/ops.rs:23-129 ---- */
@@ -125,6 +128,9 @@ typedef union mdim_scalar {
     uint32_t u32;
     int32_t i32;
     uint8_t u8;
+    int8_t i8;
+    int16_t i16;
+    uint16_t u16;
 } mdim_scalar;
 
 /*
@@ -272,7 +278,8 @@ int mdim_comm_destroy(mdim_ctx* ctx);
 int mdim_comm_info(mdim_ctx* ctx, int* rank, int* world, int* nccl_version);
 int mdim_allgather(mdim_ctx* ctx, const void* send_device, void* recv_device, size_t block_bytes); /* async, rank-major */
 int mdim_allreduce(mdim_ctx* ctx, void* data_device, size_t n, int dtype, int op);       /* async, in place; op: MDIM_ADD,
-                                                                                             MDIM_MUL, MDIM_REDUCE_MIN/MAX */
+                                                                                             MDIM_MUL, MDIM_REDUCE_MIN/MAX; NCCL has no
+                                                                                             16-bit integer: I16 / U16 are UNSUPPORTED */
 int mdim_barrier(mdim_ctx* ctx);                                                          /* + waits for the stream */
 int mdim_peer_table(mdim_ctx* ctx, void* local_device, size_t block_bytes, void* peers[MDIM_MAX_PEERS]);
 int mdim_peer_table_close(mdim_ctx* ctx);                                                 /* unmaps every peer block */

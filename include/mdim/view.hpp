@@ -143,6 +143,9 @@ template <> struct DType<uint32_t> { static constexpr int v = MDIM_U32; };
 template <> struct DType<int64_t> { static constexpr int v = MDIM_I64; };
 template <> struct DType<uint64_t> { static constexpr int v = MDIM_U64; };
 template <> struct DType<uint8_t> { static constexpr int v = MDIM_U8; };
+template <> struct DType<int8_t> { static constexpr int v = MDIM_I8; };
+template <> struct DType<int16_t> { static constexpr int v = MDIM_I16; };
+template <> struct DType<uint16_t> { static constexpr int v = MDIM_U16; };
 template <> struct DType<bool> { static constexpr int v = MDIM_U8; };
 template <class T> mdim_scalar scalar_of(T x) { mdim_scalar s; s.u64 = 0; std::memcpy(&s, &x, sizeof(T)); return s; }
 

@@ -20,9 +20,9 @@ COMM_ID_BYTES = 128
 REDUCE_MIN, REDUCE_MAX = 100, 101
 
 # dtypes (mdim_dtype)
-U8, I32, U32, I64, U64, F32, F64 = range(7)
-DTYPE_SIZE = {U8: 1, I32: 4, U32: 4, I64: 8, U64: 8, F32: 4, F64: 8}
-DTYPE_NAME = {U8: "u8", I32: "i32", U32: "u32", I64: "i64", U64: "u64", F32: "f32", F64: "f64"}
+U8, I32, U32, I64, U64, F32, F64, I8, I16, U16 = range(10)
+DTYPE_SIZE = {U8: 1, I32: 4, U32: 4, I64: 8, U64: 8, F32: 4, F64: 8, I8: 1, I16: 2, U16: 2}
+DTYPE_NAME = {U8: "u8", I32: "i32", U32: "u32", I64: "i64", U64: "u64", F32: "f32", F64: "f64", I8: "i8", I16: "i16", U16: "u16"}
 
 # binary ops (mdim_binary_op) — reference src/ops.rs:23-129
 ADD, SUB, MUL, DIV, REM, AND, OR, XOR, SHL, SHR = range(10)
@@ -38,7 +38,7 @@ IPC_HANDLE_BYTES = 64
 
 class Scalar(C.Union):
     _fields_ = [("u64", C.c_uint64), ("i64", C.c_int64), ("f64", C.c_double), ("f32", C.c_float),
-                ("u32", C.c_uint32), ("i32", C.c_int32), ("u8", C.c_uint8)]
+                ("u32", C.c_uint32), ("i32", C.c_int32), ("u8", C.c_uint8), ("i8", C.c_int8), ("i16", C.c_int16), ("u16", C.c_uint16)]
 
 
 class Node(C.Structure):

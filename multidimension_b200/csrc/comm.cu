@@ -219,6 +219,8 @@ int mdim_allreduce(mdim_ctx* ctx, void* data_device, size_t n, int dtype, int op
     int nt, no;
     switch (dtype) {
         case MDIM_U8: nt = kNcclUint8; break;
+        case MDIM_I8: nt = kNcclInt8; break;
+        case MDIM_I16: case MDIM_U16: return set_error(ctx, MDIM_ERR_UNSUPPORTED, "all-reduce: NCCL has no 16-bit integer type");
         case MDIM_I32: nt = kNcclInt32; break;
         case MDIM_U32: nt = kNcclUint32; break;
         case MDIM_I64: nt = kNcclInt64; break;

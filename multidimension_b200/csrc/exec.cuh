@@ -69,7 +69,14 @@ MDIM_FN double d_mul(double a, double b) { volatile double r = a * b; return r; 
 MDIM_FN double d_div(double a, double b) { volatile double r = a / b; return r; }
 #endif
 
-MDIM_FN int esize_of(int dt) { return dt == MDIM_U8 ? 1 : (dt == MDIM_I32 || dt == MDIM_U32 || dt == MDIM_F32) ? 4 : 8; }
+// The 1- and 2-byte integers besides U8.  No pre-built signature has one, so a kernel whose signature has none (SMALL = false)
+// skips their tests where a dtype is only known at run time (the output's, a gather source's), and keeps the code it had before
+// they existed.  The interpreter (SMALL = true) serves every program.
+MDIM_CE bool is_small_int(int dt) { return dt == MDIM_I8 || dt == MDIM_I16 || dt == MDIM_U16; }
+template <bool SMALL = true> MDIM_FN int esize_of(int dt) {
+    if constexpr (SMALL) return dtype_size(dt);
+    else return dt == MDIM_U8 ? 1 : (dt == MDIM_I32 || dt == MDIM_U32 || dt == MDIM_F32) ? 4 : 8;
+}
 
 // ------------------------------------------------------------------------------------------------
 // global memory access.  Streaming vector loads bypass L1 (read once); scalar broadcast / strided /
@@ -122,6 +129,9 @@ MDIM_FN uint64_t ld64(const void* p) { return __ldg((const unsigned long long*)p
 MDIM_FN uint32_t ld32_big(const void* p) { uint32_t a; asm volatile("ld.global.nc.L2::64B.u32 %0, [%1];" : "=r"(a) : "l"(p)); return a; }
 MDIM_FN uint64_t ld64_big(const void* p) { unsigned long long a; asm volatile("ld.global.nc.L2::64B.u64 %0, [%1];" : "=l"(a) : "l"(p)); return a; }
 MDIM_FN uint32_t ld8(const void* p) { return __ldg((const uint8_t*)p); }
+MDIM_FN uint32_t ld16(const void* p) { return __ldg((const unsigned short*)p); }
+MDIM_FN uint32_t ld16_stream(const void* p) { unsigned short a; asm volatile("ld.global.nc.L1::no_allocate.u16 %0, [%1];" : "=h"(a) : "l"(p)); return a; }
+MDIM_FN uint32_t ld16_big(const void* p) { unsigned short a; asm volatile("ld.global.nc.L2::64B.u16 %0, [%1];" : "=h"(a) : "l"(p)); return a; }
 MDIM_FN void st128(void* p, uint32_t a, uint32_t b, uint32_t c, uint32_t d, bool cs) {
     if (cs) asm volatile("st.global.cs.v4.u32 [%0], {%1,%2,%3,%4};" ::"l"(p), "r"(a), "r"(b), "r"(c), "r"(d) : "memory");
     else asm volatile("st.global.v4.u32 [%0], {%1,%2,%3,%4};" ::"l"(p), "r"(a), "r"(b), "r"(c), "r"(d) : "memory");
@@ -130,6 +140,7 @@ MDIM_FN void st64(void* p, uint32_t a, uint32_t b) {
     asm volatile("st.global.v2.u32 [%0], {%1,%2};" ::"l"(p), "r"(a), "r"(b) : "memory");
 }
 MDIM_FN void st32(void* p, uint32_t a) { *(uint32_t*)p = a; }
+MDIM_FN void st16(void* p, uint32_t a) { *(uint16_t*)p = (uint16_t)a; }
 MDIM_FN void st8(void* p, uint32_t a) { *(uint8_t*)p = (uint8_t)a; }
 MDIM_FN void err_min(unsigned long long* p, unsigned long long v) { atomicMin(p, v); }
 #else
@@ -147,9 +158,13 @@ MDIM_FN uint64_t ld64(const void* p) { return *(const uint64_t*)p; }
 MDIM_FN uint32_t ld32_big(const void* p) { return *(const uint32_t*)p; }
 MDIM_FN uint64_t ld64_big(const void* p) { return *(const uint64_t*)p; }
 MDIM_FN uint32_t ld8(const void* p) { return *(const uint8_t*)p; }
+MDIM_FN uint32_t ld16(const void* p) { return *(const uint16_t*)p; }
+MDIM_FN uint32_t ld16_stream(const void* p) { return *(const uint16_t*)p; }
+MDIM_FN uint32_t ld16_big(const void* p) { return *(const uint16_t*)p; }
 MDIM_FN void st128(void* p, uint32_t a, uint32_t b, uint32_t c, uint32_t d, bool) { uint32_t* q = (uint32_t*)p; q[0] = a; q[1] = b; q[2] = c; q[3] = d; }
 MDIM_FN void st64(void* p, uint32_t a, uint32_t b) { uint32_t* q = (uint32_t*)p; q[0] = a; q[1] = b; }
 MDIM_FN void st32(void* p, uint32_t a) { *(uint32_t*)p = a; }
+MDIM_FN void st16(void* p, uint32_t a) { *(uint16_t*)p = (uint16_t)a; }
 MDIM_FN void st8(void* p, uint32_t a) { *(uint8_t*)p = (uint8_t)a; }
 MDIM_FN void err_min(unsigned long long* p, unsigned long long v) { if (v < *p) *p = v; }
 #endif
@@ -158,16 +173,20 @@ template <bool CACHED> MDIM_FN void ld128(const void* p, uint32_t& a, uint32_t& 
     if constexpr (CACHED) ld128_cached(p, a, b, c, d); else ld128_stream(p, a, b, c, d);
 }
 
-template <class S> MDIM_FN S ld_scalar_big(const void* base, int64_t idx, int esize) {
+template <class S, bool SMALL = true> MDIM_FN S ld_scalar_big(const void* base, int64_t idx, int esize) {
     if (esize == 4) return (S)ld32_big((const char*)base + idx * 4);
     if (esize == 1) return (S)ld8((const char*)base + idx);
+    if constexpr (SMALL)
+        if (esize == 2) return (S)ld16_big((const char*)base + idx * 2);
     if (sizeof(S) == 8) return (S)ld64_big((const char*)base + idx * 8);
     return 0;
 }
 
-template <class S> MDIM_FN S ld_scalar(const void* base, int64_t idx, int esize) {
+template <class S, bool SMALL = true> MDIM_FN S ld_scalar(const void* base, int64_t idx, int esize) {
     if (esize == 4) return (S)ld32((const char*)base + idx * 4);
     if (esize == 1) return (S)ld8((const char*)base + idx);
+    if constexpr (SMALL)
+        if (esize == 2) return (S)ld16((const char*)base + idx * 2);
     if (sizeof(S) == 8) return (S)ld64((const char*)base + idx * 8);
     return 0;
 }
@@ -216,6 +235,22 @@ template <class S, int V, bool CACHED> MDIM_FN void ld_vector(const void* base, 
                 uint32_t a, b; ld64_stream(p, a, b); d[0] = (S)a | ((S)b << 32);
             }
         }
+    } else if (esize == 2) {  // 8 lanes: one 128-bit access, 4 lanes: one 64-bit access
+        const char* p = (const char*)base + idx * 2;
+        if constexpr (V == 8) {
+            uint32_t w[4];
+            ld128<CACHED>(p, w[0], w[1], w[2], w[3]);
+#pragma unroll
+            for (int i = 0; i < 4; ++i) { d[2 * i] = w[i] & 0xffffu; d[2 * i + 1] = w[i] >> 16; }
+        } else if constexpr (V == 4) {
+            uint32_t a, b; ld64_stream(p, a, b);
+            d[0] = a & 0xffffu; d[1] = a >> 16; d[2] = b & 0xffffu; d[3] = b >> 16;
+        } else if constexpr (V == 2) {
+            const uint32_t a = ld32_stream(p);
+            d[0] = a & 0xffffu; d[1] = a >> 16;
+        } else {
+            d[0] = (S)ld16_stream(p);
+        }
     } else {
         const char* p = (const char*)base + idx;
         if constexpr (V == 8) {
@@ -234,7 +269,7 @@ template <class S, int V, bool CACHED> MDIM_FN void ld_vector(const void* base, 
 }
 
 // Wide stores are streaming (st.global.cs, evict-first): nothing re-reads the output.
-template <class S, int V> MDIM_FN void st_vector(void* base, uint64_t idx, int esize, const S (&d)[V], bool w256 = false) {
+template <class S, int V, bool SMALL = true> MDIM_FN void st_vector(void* base, uint64_t idx, int esize, const S (&d)[V], bool w256 = false) {
     if constexpr (V * sizeof(S) == 32 && (sizeof(S) == 4 || sizeof(S) == 8)) {
         if (w256 && esize == (int)sizeof(S)) {
             uint32_t r[8];
@@ -270,6 +305,13 @@ template <class S, int V> MDIM_FN void st_vector(void* base, uint64_t idx, int e
                 st64(p, (uint32_t)d[0], (uint32_t)(d[0] >> 32));
             }
         }
+    } else if (SMALL && esize == 2) {
+        char* p = (char*)base + idx * 2;
+        auto pair = [&](int i) { return ((uint32_t)d[i] & 0xffffu) | ((uint32_t)d[i + 1] << 16); };
+        if constexpr (V == 8) st128(p, pair(0), pair(2), pair(4), pair(6), true);
+        else if constexpr (V == 4) st64(p, pair(0), pair(2));
+        else if constexpr (V == 2) st32(p, pair(0));
+        else st16(p, (uint32_t)d[0]);
     } else {
         char* p = (char*)base + idx;
         if constexpr (V == 8) {
@@ -293,8 +335,45 @@ template <class S, int V> MDIM_FN void st_vector(void* base, uint64_t idx, int e
 // value semantics.  A slot holds the raw bits of one value, zero-extended to the slot width.
 // Integer semantics follow Rust RELEASE builds: add/sub/mul wrap, shift amounts are masked,
 // x/0 and MIN/-1 panic in every build mode (→ arith error).  Floats are IEEE, never fused.
+// The 1- and 2-byte integers (U8, I8, I16, U16; w = 8 or 16) keep that layout: every result is masked back to w bits.
+// Add, Sub, Mul, Neg and Not wrap mod 2^w and Abs(MIN) = MIN; Div and Rem truncate toward zero, x / 0, x % 0, MIN / -1 and
+// MIN % -1 are arith errors; a shift takes the rhs's own bits masked by w - 1, and Shr is arithmetic on I8 / I16.  Signed
+// values are sign-extended from bit w - 1 wherever the sign matters (Shr, Div, Rem, Abs, casts).
 // ------------------------------------------------------------------------------------------------
-template <class S> MDIM_FN S bin_op(int dt, int op, int rdt, S a, S b, bool& arith) {
+MDIM_FN int32_t sext(uint32_t x, int bits) { return (int32_t)(x << (32 - bits)) >> (32 - bits); }
+
+MDIM_FN uint32_t small_bin_op(int dt, int op, uint32_t x, uint32_t y, bool& arith) {
+    const int bits = 8 * dtype_size(dt);
+    const bool sgn = is_signed(dt);
+    const int32_t sx = sgn ? sext(x, bits) : (int32_t)x, sy = sgn ? sext(y, bits) : (int32_t)y;  // exact values (y: the rhs's own width)
+    uint32_t r = 0;
+    switch (op) {
+        case MDIM_ADD: r = x + y; break;
+        case MDIM_SUB: r = x - y; break;
+        case MDIM_MUL: r = x * y; break;
+        case MDIM_AND: r = x & y; break;
+        case MDIM_OR: r = x | y; break;
+        case MDIM_XOR: r = x ^ y; break;
+        case MDIM_SHL: r = x << (y & (uint32_t)(bits - 1)); break;
+        case MDIM_SHR: r = (uint32_t)(sx >> (y & (uint32_t)(bits - 1))); break;  // sx >= 0 when unsigned: logical
+        case MDIM_DIV:
+        case MDIM_REM:
+            if (y == 0 || (sgn && sx == -(1 << (bits - 1)) && sy == -1)) { arith = true; r = 0; }
+            else r = (uint32_t)(op == MDIM_DIV ? sx / sy : sx % sy);
+            break;
+    }
+    return r & ((1u << bits) - 1u);
+}
+// One out-of-line copy for the interpreter, which expands bin_op at every stack depth: its code (and the instruction cache it
+// runs from) then grows by a call per depth instead of the whole operator.  A signature's kernel inlines the operator it names.
+#if defined(__CUDACC__)
+static __device__ __noinline__
+#else
+static
+#endif
+uint32_t small_bin_op_shared(int dt, int op, uint32_t x, uint32_t y, bool& arith) { return small_bin_op(dt, op, x, y, arith); }
+
+template <class S, bool SMALL = true> MDIM_FN S bin_op(int dt, int op, int rdt, S a, S b, bool& arith) {
     if (dt == MDIM_F32) {
         float x = as_f32((uint32_t)a), y = as_f32((uint32_t)b), r = 0.f;
         switch (op) {
@@ -306,6 +385,8 @@ template <class S> MDIM_FN S bin_op(int dt, int op, int rdt, S a, S b, bool& ari
         }
         return (S)f32_bits(r);
     }
+    if constexpr (SMALL)
+        if (is_small_int(dt)) return (S)small_bin_op(dt, op, (uint32_t)a, (uint32_t)b, arith);  // (a shift's rhs: its low bits suffice)
     if (dt == MDIM_I32 || dt == MDIM_U32 || dt == MDIM_U8) {
         uint32_t x = (uint32_t)a, y = (uint32_t)b, r = 0;
         const uint32_t bits = dt == MDIM_U8 ? 8u : 32u;
@@ -379,8 +460,13 @@ MDIM_FN uint64_t sat_u64(double f, uint64_t hi) {
     return (uint64_t)f;
 }
 
-template <class S> MDIM_FN S cast_val(int from, int to, S a) {
+template <class S> MDIM_FN S small_cast(int from, int to, S a);
+
+// SMALL = false: a cast between the 4- and 8-byte types and U8 only (see is_small_int)
+template <class S, bool SMALL = true> MDIM_FN S cast_val(int from, int to, S a) {
     if (from == to) return a;
+    if constexpr (SMALL)
+        if (is_small_int(from) || is_small_int(to)) return small_cast<S>(from, to, a);
     const bool from_f = from == MDIM_F32 || from == MDIM_F64;
     if (from_f) {
         double d;
@@ -415,8 +501,29 @@ template <class S> MDIM_FN S cast_val(int from, int to, S a) {
     return 0;
 }
 
-template <class S> MDIM_FN S un_op(int op, int dt, int src_dt, S a) {
-    if (op == MDIM_CAST) return cast_val<S>(src_dt, dt, a);
+// A cast with an I8 / I16 / U16 side.  A 1- or 2-byte source is exactly an i32 (I8, I16: sign-extended) or a u32 (U16) value,
+// so a cast to a wider type is that type's cast; a 1- or 2-byte destination takes the low bits of an integer (wrapping) and
+// the saturated value of a float.
+template <class S> MDIM_FN S small_cast(int from, int to, S a) {
+    if (is_small_int(from)) {
+        const uint32_t x = is_signed(from) ? (uint32_t)sext((uint32_t)a, 8 * dtype_size(from)) : (uint32_t)a;
+        if (!is_small_int(to)) return cast_val<S, false>(is_signed(from) ? MDIM_I32 : MDIM_U32, to, (S)x);
+        return (S)(x & ((1u << (8 * dtype_size(to))) - 1u));
+    }
+    const uint32_t mask = (1u << (8 * dtype_size(to))) - 1u;
+    if (from == MDIM_F32 || from == MDIM_F64) {
+        double d;
+        if (from == MDIM_F32) d = (double)as_f32((uint32_t)a);
+        else { if constexpr (sizeof(S) == 8) d = as_f64(a); else d = 0.; }
+        if (is_signed(to)) return (S)((uint32_t)sat_i64(d, -(int64_t)(mask >> 1) - 1, (int64_t)(mask >> 1)) & mask);
+        return (S)sat_u64(d, mask);
+    }
+    return (S)((uint32_t)a & mask);  // int -> int: the low bits
+}
+
+// SMALL = false: an op on the 4- and 8-byte types and U8 only
+template <class S, bool SMALL = true> MDIM_FN S un_op(int op, int dt, int src_dt, S a) {
+    if (op == MDIM_CAST) return cast_val<S, SMALL>(src_dt, dt, a);
     if (dt == MDIM_F32) {
         float x = as_f32((uint32_t)a);
         switch (op) {
@@ -447,6 +554,17 @@ template <class S> MDIM_FN S un_op(int op, int dt, int src_dt, S a) {
         return a;
     }
     uint32_t x = (uint32_t)a, r = x;
+    if constexpr (SMALL) {
+        if (is_small_int(dt)) {
+            const int bits = 8 * dtype_size(dt);
+            switch (op) {
+                case MDIM_NEG: r = 0u - x; break;
+                case MDIM_NOT: r = ~x; break;
+                case MDIM_ABS: r = is_signed(dt) && sext(x, bits) < 0 ? 0u - x : x; break;
+            }
+            return (S)(r & ((1u << bits) - 1u));
+        }
+    }
     switch (op) {
         case MDIM_NEG: r = 0u - x; break;
         case MDIM_NOT: r = ~x; break;
@@ -455,6 +573,13 @@ template <class S> MDIM_FN S un_op(int op, int dt, int src_dt, S a) {
     if (dt == MDIM_U8) r &= 0xffu;
     return (S)r;
 }
+// The interpreter's one out-of-line copy of the unary ops and casts with a 1- or 2-byte side (see small_bin_op_shared)
+#if defined(__CUDACC__)
+template <class S> static __device__ __noinline__
+#else
+template <class S> static
+#endif
+S un_op_shared(int op, int dt, int src_dt, S a) { return un_op<S, true>(op, dt, src_dt, a); }
 
 // ------------------------------------------------------------------------------------------------
 // per-thread state.  MAXR = number of iteration axes this instantiation walks (the planner picks the
@@ -542,13 +667,13 @@ MDIM_FN int depth_delta(int opc, int aux) {
 // Compose::at = w.at(v.at(i)) (src/view.rs:905,911); each component is bounds-checked like
 // usize::to_usize (src/int.rs:16-19) in component order; inactive (off-diagonal) lanes neither
 // load nor report, because Diagonal::at never evaluates its inner view there (src/view.rs:854-856).
-template <int D, int NC, class S, int V, int MAXD, bool WIDE, int MAXR>
+template <int D, int NC, class S, int V, int MAXD, bool WIDE, int MAXR, bool SMALL>
 MDIM_FN void exec_gather(const Program& P, ErrWord* err, const Instr& I, int slot, S (&st)[MAXD][V], const ThreadState<WIDE, MAXR>& ts) {
     if constexpr (sizeof(S) == 8 && D >= NC && NC >= 1) {
         const Addr& A = MDIM_SHAPE_OF(P).addr[slot];  // gstride / bound / n_peers: shape-like; the pointer is read from P
         const int64_t base = (int64_t)addr_offset<WIDE, MAXR>(P, slot, ts);
         const int64_t s_in = inner_stride(P, slot);
-        const int es = esize_of(I.dtype);
+        const int es = esize_of<SMALL>(I.dtype);
 #pragma unroll
         for (int l = 0; l < V; ++l) {
             int64_t idx = base + (int64_t)l * s_in;
@@ -566,11 +691,11 @@ MDIM_FN void exec_gather(const Program& P, ErrWord* err, const Instr& I, int slo
             if (ok) {
                 if (A.n_peers > 1) {
                     const uint64_t p = (uint64_t)idx / P.peers.block;
-                    v = ld_scalar<S>(P.peers.peer[p], (int64_t)((uint64_t)idx - p * P.peers.block), es);
+                    v = ld_scalar<S, SMALL>(P.peers.peer[p], (int64_t)((uint64_t)idx - p * P.peers.block), es);
                 } else if (P.flags & PF_GATHER_BIG) {
-                    v = ld_scalar_big<S>(P.addr[slot].ptr, idx, es);
+                    v = ld_scalar_big<S, SMALL>(P.addr[slot].ptr, idx, es);
                 } else {
-                    v = ld_scalar<S>(P.addr[slot].ptr, idx, es);
+                    v = ld_scalar<S, SMALL>(P.addr[slot].ptr, idx, es);
                 }
             }
             st[D - NC][l] = v;
@@ -602,6 +727,31 @@ template <bool WIDE, int MAXR> MDIM_FN void advance_red(const Program& P, Thread
 // A LEAF whose Array is sharded over the GPUs of the box (instruction aux bit 1; mdim_node.n_peers): element `off`
 // of the whole Array lives at peers.peer[off / block] + off % block.  Vectors never straddle two blocks (the
 // planner only vectorises when block boundaries are vector-aligned).
+// The 32-bit-slot interpreter, whose code grows most with them (8 lanes at every depth), runs the 1- and 2-byte operators and casts
+// through one shared out-of-line copy; the 64-bit-slot one inlines them (a call's saved registers would spill there).
+template <bool INTERP, class S> constexpr bool kShareSmall = INTERP && sizeof(S) == 4;
+
+// x (op) y on every lane, for a BINARY or a FOLD_STEP: an integer error is reported at the lane's position when the lane is active.
+// The interpreter branches once per instruction to its shared copy of the 1- and 2-byte operators.
+template <bool SMALL, bool INTERP, class S, int V, bool WIDE, int MAXR>
+MDIM_FN void binary_lanes(const Program& P, ErrWord* err, int node, int dt, int op, int rdt, S (&x)[V], const S (&y)[V], const ThreadState<WIDE, MAXR>& ts) {
+    if (kShareSmall<INTERP, S> && is_small_int(dt)) {
+#pragma unroll
+        for (int l = 0; l < V; ++l) {
+            bool arith = false;
+            x[l] = (S)small_bin_op_shared(dt, op, (uint32_t)x[l], (uint32_t)y[l], arith);  // (a shift's rhs: its low bits suffice)
+            if (arith && ((ts.mask >> l) & 1u)) report(P, err, ts.pos0 + l, MDIM_ERR_ARITH, node, 0, (uint64_t)y[l], 0);
+        }
+    } else {
+#pragma unroll
+        for (int l = 0; l < V; ++l) {
+            bool arith = false;
+            x[l] = bin_op<S, SMALL && !kShareSmall<INTERP, S>>(dt, op, rdt, x[l], y[l], arith);
+            if (arith && ((ts.mask >> l) & 1u)) report(P, err, ts.pos0 + l, MDIM_ERR_ARITH, node, 0, (uint64_t)y[l], 0);
+        }
+    }
+}
+
 template <bool WIDE> MDIM_FN const void* leaf_base(const Program& P, int slot, int aux, int64_t& off) {
     if (aux & 2) {
         uint64_t p;
@@ -613,7 +763,8 @@ template <bool WIDE> MDIM_FN const void* leaf_base(const Program& P, int slot, i
     return P.addr[slot].ptr;
 }
 
-template <int D, class S, int V, int MAXD, bool WIDE, int MAXR, int SLOTK = -1>
+// INTERP: called by the interpreter (every opcode and dtype at every depth), not by a signature's compile-time instruction stream.
+template <int D, class S, int V, int MAXD, bool WIDE, int MAXR, int SLOTK = -1, bool SMALL = true, bool INTERP = true>
 MDIM_FN int exec_instr(const Program& P, ErrWord* err, int opc, int dtype, int op, int aux, int pc,
                        S (&st)[MAXD][V], ThreadState<WIDE, MAXR>& ts) {
     const Instr& I = MDIM_SHAPE_OF(P).instr[pc];  // opcode operands (slot, n, source node) are shape-like ...
@@ -663,8 +814,8 @@ MDIM_FN int exec_instr(const Program& P, ErrWord* err, int opc, int dtype, int o
 #pragma unroll
                 for (int l = 0; l < V; ++l) {
                     const uint64_t x = (uint64_t)(off + (int64_t)l * s_in);
-                    if constexpr (sizeof(S) == 8) st[D][l] = cast_val<S>(MDIM_U64, dtype, x);
-                    else st[D][l] = dtype == MDIM_F32 ? (S)f32_bits((float)x) : dtype == MDIM_U8 ? (S)(x & 0xffu) : (S)(uint32_t)x;
+                    if constexpr (sizeof(S) == 8) st[D][l] = cast_val<S, SMALL>(MDIM_U64, dtype, x);
+                    else st[D][l] = dtype == MDIM_F32 ? (S)f32_bits((float)x) : dtype_size(dtype) < 4 ? (S)(x & ((1u << (8 * dtype_size(dtype))) - 1u)) : (S)(uint32_t)x;
                 }
             }
             break;
@@ -676,18 +827,18 @@ MDIM_FN int exec_instr(const Program& P, ErrWord* err, int opc, int dtype, int o
             break;
         case OPC_UNARY:  // Map::at = f(v.at(i)) (src/view.rs:888), closed op set
             if constexpr (D >= 1) {
+                if (kShareSmall<INTERP, S> && (is_small_int(dtype) || is_small_int(aux))) {
 #pragma unroll
-                for (int l = 0; l < V; ++l) st[D - 1][l] = un_op<S>(op, dtype, aux, st[D - 1][l]);
+                    for (int l = 0; l < V; ++l) st[D - 1][l] = un_op_shared<S>(op, dtype, aux, st[D - 1][l]);
+                } else {
+#pragma unroll
+                    for (int l = 0; l < V; ++l) st[D - 1][l] = un_op<S, SMALL && !kShareSmall<INTERP, S>>(op, dtype, aux, st[D - 1][l]);
+                }
             }
             break;
         case OPC_BINARY:  // Zip::at = B::call(v.at(vi), w.at(wi)) (src/view.rs:1194-1197)
             if constexpr (D >= 2) {
-#pragma unroll
-                for (int l = 0; l < V; ++l) {
-                    bool arith = false;
-                    st[D - 2][l] = bin_op<S>(dtype, op, aux, st[D - 2][l], st[D - 1][l], arith);
-                    if (arith && ((ts.mask >> l) & 1u)) report(P, err, ts.pos0 + l, MDIM_ERR_ARITH, I.n, 0, (uint64_t)st[D - 1][l], 0);
-                }
+                binary_lanes<SMALL, INTERP>(P, err, I.n, dtype, op, aux, st[D - 2], st[D - 1], ts);
             }
             break;
         case OPC_MASK:
@@ -708,9 +859,9 @@ MDIM_FN int exec_instr(const Program& P, ErrWord* err, int opc, int dtype, int o
             }
             break;
         case OPC_GATHER:
-            if (aux == 1) exec_gather<D, 1, S, V, MAXD, WIDE, MAXR>(P, err, I, slot, st, ts);
-            else if (aux == 2) exec_gather<D, 2, S, V, MAXD, WIDE, MAXR>(P, err, I, slot, st, ts);
-            else if (aux == 3) exec_gather<D, 3, S, V, MAXD, WIDE, MAXR>(P, err, I, slot, st, ts);
+            if (aux == 1) exec_gather<D, 1, S, V, MAXD, WIDE, MAXR, SMALL>(P, err, I, slot, st, ts);
+            else if (aux == 2) exec_gather<D, 2, S, V, MAXD, WIDE, MAXR, SMALL>(P, err, I, slot, st, ts);
+            else if (aux == 3) exec_gather<D, 3, S, V, MAXD, WIDE, MAXR, SMALL>(P, err, I, slot, st, ts);
             break;
         case OPC_FOLD_BEGIN:  // let mut s = init;  (the closure of rows().map(..), SURVEY.md fact 3)
             if constexpr (D < MAXD) {
@@ -728,12 +879,7 @@ MDIM_FN int exec_instr(const Program& P, ErrWord* err, int opc, int dtype, int o
             break;
         case OPC_FOLD_STEP:  // row.each(|x| s = s (op) x): sequential, index order (src/view.rs:250-252)
             if constexpr (D >= 2) {
-#pragma unroll
-                for (int l = 0; l < V; ++l) {
-                    bool arith = false;
-                    st[D - 2][l] = bin_op<S>(dtype, op, aux, st[D - 2][l], st[D - 1][l], arith);
-                    if (arith && ((ts.mask >> l) & 1u)) report(P, err, ts.pos0 + l, MDIM_ERR_ARITH, I.n, 0, (uint64_t)st[D - 1][l], 0);
-                }
+                binary_lanes<SMALL, INTERP>(P, err, I.n, dtype, op, aux, st[D - 2], st[D - 1], ts);
                 advance_red<WIDE, MAXR>(P, ts);
                 ts.red_k += 1;
                 if (ts.red_k < MDIM_SHAPE_OF(P).red_count) next = I.slot;
@@ -767,6 +913,15 @@ template <class Sig> MDIM_CE int sig_addr_slot(int pc) {
         if (sig_is_addressed(Sig::code[i])) ++k;
     return sig_is_addressed(Sig::code[pc]) ? k : -1;
 }
+// a signature with a value of a 1- or 2-byte type besides U8 (every value's type is some instruction's dtype)
+template <class Sig> MDIM_CE bool sig_small() {
+    if constexpr (Sig::n == 0) return true;  // the interpreter: any program
+    else {
+        for (int i = 0; i < Sig::n; ++i)
+            if (is_small_int(Sig::code[i].dtype)) return true;
+        return false;
+    }
+}
 MDIM_CE int sig_depth_after(SigInstr I, int d) {
     return d + (I.opc == OPC_LEAF_VEC || I.opc == OPC_LEAF_BCAST || I.opc == OPC_LEAF_STRIDED || I.opc == OPC_IOTA || I.opc == OPC_CONST ||
                         (I.opc == OPC_FOLD_BEGIN && I.aux != 1) ? 1
@@ -784,7 +939,7 @@ MDIM_FN void run_static(const Program& P, ErrWord* err, S (&st)[MAXD][V], Thread
         if constexpr (I.opc == OPC_FOLD_BEGIN) {
             constexpr int END = sig_fold_end<Sig>(PC);
             constexpr int B = I.aux == 1 ? D - 1 : D;  // stack slot of the accumulator (aux 1: the init view's value, already pushed)
-            exec_instr<D, S, V, MAXD, WIDE, MAXR>(P, err, I.opc, I.dtype, I.op, I.aux, PC, st, ts);
+            exec_instr<D, S, V, MAXD, WIDE, MAXR, -1, sig_small<Sig>(), false>(P, err, I.opc, I.dtype, I.op, I.aux, PC, st, ts);
             constexpr SigInstr E = Sig::code[END < Sig::n ? END : PC];
             // Outer loop: the slower reduction axes (coordinates in c[], rare).  Inner loop: the fastest one,
             // where every coordinate in c[] is loop-invariant, so an operand's address is base + rk * rstride;
@@ -809,7 +964,7 @@ MDIM_FN void run_static(const Program& P, ErrWord* err, S (&st)[MAXD][V], Thread
             }
             run_static<Sig, END + 1, B + 1, STOP, S, V, MAXD, WIDE, MAXR>(P, err, st, ts);
         } else {
-            exec_instr<D, S, V, MAXD, WIDE, MAXR, sig_addr_slot<Sig>(PC)>(P, err, I.opc, I.dtype, I.op, I.aux, PC, st, ts);
+            exec_instr<D, S, V, MAXD, WIDE, MAXR, sig_addr_slot<Sig>(PC), sig_small<Sig>(), false>(P, err, I.opc, I.dtype, I.op, I.aux, PC, st, ts);
             run_static<Sig, PC + 1, sig_depth_after(I, D), STOP, S, V, MAXD, WIDE, MAXR>(P, err, st, ts);
         }
     }
@@ -873,12 +1028,13 @@ MDIM_FN void eval_vector(const Program& P, void* out, ErrWord* err, uint64_t g) 
     S st[MAXD][V];
     if constexpr (Sig::n > 0) run_static<Sig, 0, 0, Sig::n, S, V, MAXD, WIDE, MAXR>(P, err, st, ts);
     else run_interp<S, V, MAXD, WIDE, MAXR>(P, err, st, ts);
-    st_vector<S, V>(out, ts.pos0, esize_of(MDIM_SHAPE_OF(P).out_dtype), st[0], (P.flags & PF_VEC256) != 0);
+    constexpr bool SMALL = sig_small<Sig>();
+    st_vector<S, V, SMALL>(out, ts.pos0, esize_of<SMALL>(MDIM_SHAPE_OF(P).out_dtype), st[0], (P.flags & PF_VEC256) != 0);
     if (MDIM_SHAPE_OF(P).n_out > 1) {  // a tuple-typed root: value k of the final stack is scalar leaf k, stored to its own run
 #pragma unroll
         for (int k = 1; k < MDIM_MAX_OUTS; ++k)
             if (k < MAXD && k < MDIM_SHAPE_OF(P).n_out)
-                st_vector<S, V>(P.out_more[k - 1], ts.pos0, esize_of(MDIM_SHAPE_OF(P).out_dtypes[k]), st[k < MAXD ? k : 0]);
+                st_vector<S, V, SMALL>(P.out_more[k - 1], ts.pos0, esize_of<SMALL>(MDIM_SHAPE_OF(P).out_dtypes[k]), st[k < MAXD ? k : 0]);
     }
 }
 

@@ -68,7 +68,7 @@ __device__ __forceinline__ float apply_f32(int op, float a, float b) {
 __device__ __forceinline__ uint32_t apply_any(int dtype, int op, uint32_t a, uint32_t b) {
     if (dtype == MDIM_F32) return __float_as_uint(apply_f32(op, __uint_as_float(a), __uint_as_float(b)));
     bool arith = false;
-    return bin_op<uint32_t>(dtype, op, dtype, a, b, arith);
+    return bin_op<uint32_t, false>(dtype, op, dtype, a, b, arith);  // (4-byte types only)
 }
 
 constexpr int kRowsPerTile = 32;  // one row per lane

@@ -83,7 +83,7 @@ __device__ __forceinline__ void fold_tile(S (&acc)[4], uint32_t p, uint32_t rows
             asm volatile("ld.shared.v2.u64 {%0,%1}, [%2];" : "=l"(x[2]), "=l"(x[3]) : "r"(p + r * SC * ES + 16));
         }
 #pragma unroll
-        for (int e = 0; e < 4; ++e) { bool arith = false; acc[e] = bin_op<S>(DT, OP, DT, acc[e], x[e], arith); }
+        for (int e = 0; e < 4; ++e) { bool arith = false; acc[e] = bin_op<S, false>(DT, OP, DT, acc[e], x[e], arith); }
     }
 }
 template <class S, int DT>

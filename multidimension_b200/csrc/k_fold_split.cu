@@ -41,9 +41,11 @@ template <int OP, class S> __device__ __forceinline__ S combine(S a, S b) {
     else if constexpr (OP == SOP_OR) return a | b;
     else return a ^ b;
 }
-// one source element (its ES bytes in the low bits of x) into a slot
-template <class S, int ES> __device__ __forceinline__ S extend(uint64_t x, bool sgn) {
-    if constexpr (ES == 1) return (S)(x & 0xffu);  // U8 is the only 1-byte integer: unsigned
+// one source element (its ES bytes in the low bits of x) into a slot.  The sign of a 1- or 2-byte source is a template
+// argument (SGN: I8, I16), that of a 4- or 8-byte one a run-time flag (sgn: I32, I64).
+template <class S, int ES, bool SGN> __device__ __forceinline__ S extend(uint64_t x, bool sgn) {
+    if constexpr (ES == 1) return SGN ? (S)(int8_t)(uint8_t)x : (S)(x & 0xffu);
+    else if constexpr (ES == 2) return SGN ? (S)(int16_t)(uint16_t)x : (S)(x & 0xffffu);
     else if constexpr (ES == 4) {
         if constexpr (sizeof(S) == 8) return sgn ? (S)(int64_t)(int32_t)(uint32_t)x : (S)(uint32_t)x;
         else return (S)(uint32_t)x;
@@ -59,38 +61,56 @@ __device__ __forceinline__ void ld128(const void* p, uint32_t (&r)[4]) {
 }
 template <int ES> __device__ __forceinline__ uint64_t ld_elem(const char* p) {
     if constexpr (ES == 1) return *(const uint8_t*)p;
+    else if constexpr (ES == 2) return __ldg((const unsigned short*)p);
     else if constexpr (ES == 4) return __ldg((const unsigned int*)p);
     else return __ldg((const unsigned long long*)p);
 }
 // element k of a vector of N 32-bit words
 template <int ES, int N> __device__ __forceinline__ uint64_t elem_of(const uint32_t (&r)[N], int k) {
     if constexpr (ES == 1) return (r[k >> 2] >> ((k & 3) * 8)) & 0xffu;
+    else if constexpr (ES == 2) return (r[k >> 1] >> ((k & 1) * 16)) & 0xffffu;
     else if constexpr (ES == 4) return r[k];
     else return (uint64_t)r[2 * k] | ((uint64_t)r[2 * k + 1] << 32);
 }
 
-// Fold a whole 32-byte vector into acc.  Bytes: Add sums the vector in 32 bits first (at most 32 x 255); the bit operations
-// combine whole words into `wacc`, each byte lane apart, and fold its four lanes into acc once at the end (bytes_into); Mul goes
-// element by element.
-template <int ES, int OP> constexpr bool kByteLanes = ES == 1 && (OP == SOP_AND || OP == SOP_OR || OP == SOP_XOR);
-template <class S, int ES, int OP> __device__ __forceinline__ void fold_vec(S& acc, uint32_t& wacc, const uint32_t (&r)[8], bool sgn) {
-    if constexpr (ES == 1 && OP == SOP_ADD) {
+// Fold a whole 32-byte vector into acc.  Bytes and 2-byte words: Add sums the vector in 32 bits first (at most 32 x 255, or
+// 16 x 65535; signed: the same bounds around 0), and the sum is extended to the slot once: extension commutes with wrapping
+// addition.  The bit operations on 1- and 2-byte elements combine whole words into `wacc`, each lane apart, and fold its lanes
+// into acc once at the end (lanes_into): bitwise operations commute with sign extension too.  Mul goes element by element.
+template <int ES, int OP> constexpr bool kWordLanes = ES < 4 && (OP == SOP_AND || OP == SOP_OR || OP == SOP_XOR);
+template <class S, int ES, int OP, bool SGN> __device__ __forceinline__ void fold_vec(S& acc, uint32_t& wacc, const uint32_t (&r)[8], bool sgn) {
+    if constexpr (ES == 1 && OP == SOP_ADD && SGN) {  // x = (x ^ 0x80) - 128 read unsigned: the unsigned sum less 32 x 128
+        uint32_t t = 0;
+#pragma unroll
+        for (int w = 0; w < 8; ++w) t = __dp4a(r[w] ^ 0x80808080u, 0x01010101u, t);
+        acc += (S)(long long)((int)t - 32 * 128);
+    } else if constexpr (ES == 1 && OP == SOP_ADD) {
         uint32_t t = 0;
 #pragma unroll
         for (int w = 0; w < 8; ++w) t = __dp4a(r[w], 0x01010101u, t);
         acc += (S)t;
-    } else if constexpr (kByteLanes<ES, OP>) {
+    } else if constexpr (ES == 2 && OP == SOP_ADD && SGN) {
+        int t = 0;
+#pragma unroll
+        for (int w = 0; w < 8; ++w) t += ((int)(r[w] << 16) >> 16) + ((int)r[w] >> 16);
+        acc += (S)(long long)t;
+    } else if constexpr (ES == 2 && OP == SOP_ADD) {
+        uint32_t t = 0;
+#pragma unroll
+        for (int w = 0; w < 8; ++w) t += (r[w] & 0xffffu) + (r[w] >> 16);
+        acc += (S)t;
+    } else if constexpr (kWordLanes<ES, OP>) {
 #pragma unroll
         for (int w = 0; w < 8; ++w) wacc = combine<OP>(wacc, r[w]);
     } else {
 #pragma unroll
-        for (int k = 0; k < 32 / ES; ++k) acc = combine<OP>(acc, extend<S, ES>(elem_of<ES, 8>(r, k), sgn));
+        for (int k = 0; k < 32 / ES; ++k) acc = combine<OP>(acc, extend<S, ES, SGN>(elem_of<ES, 8>(r, k), sgn));
     }
 }
-template <class S, int OP> __device__ __forceinline__ S bytes_into(S acc, uint32_t t) {
+template <class S, int ES, int OP, bool SGN> __device__ __forceinline__ S lanes_into(S acc, uint32_t t) {
     t = combine<OP>(t, t >> 16);
-    t = combine<OP>(t, t >> 8);
-    return combine<OP>(acc, (S)(t & 0xffu));
+    if constexpr (ES == 1) t = combine<OP>(t, t >> 8);
+    return combine<OP>(acc, extend<S, ES, SGN>(t, false));
 }
 
 template <int OP, class S> __device__ __forceinline__ S warp_combine(S v) {
@@ -116,6 +136,7 @@ template <int OP, class S> __device__ __forceinline__ S cta_combine(S v, S* red)
 
 template <class S> __device__ __forceinline__ void store_out(void* out, uint64_t o, int es, S v) {
     if (es == 1) ((uint8_t*)out)[o] = (uint8_t)v;
+    else if (es == 2) ((uint16_t*)out)[o] = (uint16_t)v;
     else if (es == 4) ((uint32_t*)out)[o] = (uint32_t)v;
     else ((uint64_t*)out)[o] = (uint64_t)v;
 }
@@ -134,8 +155,9 @@ __device__ __forceinline__ bool take_ticket(unsigned int* ticket, uint32_t n_chu
     return *last;
 }
 
-// S: slot type; ES: source bytes; OP: SplitOp; LAYOUT: SPLIT_RUNS / SPLIT_COLS.  grid = units x n_chunks, unit-major.
-template <class S, int ES, int OP, int LAYOUT>
+// S: slot type; ES: source bytes; OP: SplitOp; LAYOUT: SPLIT_RUNS / SPLIT_COLS; SGN: a signed 1- or 2-byte source.
+// grid = units x n_chunks, unit-major.
+template <class S, int ES, int OP, int LAYOUT, bool SGN>
 __global__ void __launch_bounds__(kSplitThreads, kSplitCtasPerSm)
 k_fold_split(const __grid_constant__ FoldSplitPlan F, void* __restrict__ out, unsigned int* __restrict__ tickets, void* __restrict__ partials_v,
              uint64_t chunk, uint32_t n_chunks) {
@@ -143,11 +165,11 @@ k_fold_split(const __grid_constant__ FoldSplitPlan F, void* __restrict__ out, un
     S* __restrict__ partials = (S*)partials_v;
     __shared__ S red[kSplitWarps];
     __shared__ bool last;
-    const bool sgn = F.src_dtype == MDIM_I32 || F.src_dtype == MDIM_I64;
+    const bool sgn = is_signed(F.src_dtype);
     const uint64_t unit = blockIdx.x / n_chunks;
     const uint32_t j = blockIdx.x % n_chunks;
     const int tid = threadIdx.x;
-    const int out_es = F.dtype == MDIM_U8 ? 1 : (F.dtype == MDIM_I32 || F.dtype == MDIM_U32) ? 4 : 8;
+    const int out_es = dtype_size(F.dtype);
     if constexpr (LAYOUT == SPLIT_RUNS) {
         // ---- one run: elements [k0, k1) of output `unit` -------------------------------------------------------------------
         const uint64_t i0 = unit / F.out_len[1], i1 = unit % F.out_len[1];
@@ -161,8 +183,8 @@ k_fold_split(const __grid_constant__ FoldSplitPlan F, void* __restrict__ out, un
         const uint64_t tail0 = head + nv * VE;
         S acc = identity<S, OP>();
         uint32_t wacc = identity<uint32_t, OP>();
-        if ((uint64_t)tid < head) acc = combine<OP>(acc, extend<S, ES>(ld_elem<ES>(p + (uint64_t)tid * ES), sgn));
-        if ((uint64_t)tid < n - tail0) acc = combine<OP>(acc, extend<S, ES>(ld_elem<ES>(p + (tail0 + tid) * ES), sgn));
+        if ((uint64_t)tid < head) acc = combine<OP>(acc, extend<S, ES, SGN>(ld_elem<ES>(p + (uint64_t)tid * ES), sgn));
+        if ((uint64_t)tid < n - tail0) acc = combine<OP>(acc, extend<S, ES, SGN>(ld_elem<ES>(p + (tail0 + tid) * ES), sgn));
         const char* body = p + head * ES;
         uint64_t v = tid;
         for (; v + 3 * kSplitThreads < nv; v += 4 * kSplitThreads) {  // four 256-bit loads in flight
@@ -170,15 +192,15 @@ k_fold_split(const __grid_constant__ FoldSplitPlan F, void* __restrict__ out, un
 #pragma unroll
             for (int u = 0; u < 4; ++u) ld256(body + (v + (uint64_t)u * kSplitThreads) * 32, r[u]);
 #pragma unroll
-            for (int u = 0; u < 4; ++u) fold_vec<S, ES, OP>(acc, wacc, r[u], sgn);
+            for (int u = 0; u < 4; ++u) fold_vec<S, ES, OP, SGN>(acc, wacc, r[u], sgn);
         }
         for (; v < nv; v += kSplitThreads) {
             uint32_t r[8];
             ld256(body + v * 32, r);
-            fold_vec<S, ES, OP>(acc, wacc, r, sgn);
+            fold_vec<S, ES, OP, SGN>(acc, wacc, r, sgn);
         }
-        if constexpr (kByteLanes<ES, OP>)
-            if ((uint64_t)tid < nv) acc = bytes_into<S, OP>(acc, wacc);  // (only lanes that saw a byte: for And, (S)0xff is no identity)
+        if constexpr (kWordLanes<ES, OP>)
+            if ((uint64_t)tid < nv) acc = lanes_into<S, ES, OP, SGN>(acc, wacc);  // (only lanes that saw an element: for And, (S)0xff is no identity)
         acc = cta_combine<OP>(acc, red);
         if (tid == 0) partials[unit * n_chunks + j] = acc;
         if (!take_ticket(&tickets[unit], n_chunks, &last)) return;
@@ -217,14 +239,14 @@ k_fold_split(const __grid_constant__ FoldSplitPlan F, void* __restrict__ out, un
                         uint32_t q[4];
                         ld128(colp + r * pitch, q);
 #pragma unroll
-                        for (int w = 0; w < W; ++w) acc[w] = combine<OP>(acc[w], extend<S, ES>(elem_of<ES, 4>(q, w), sgn));
+                        for (int w = 0; w < W; ++w) acc[w] = combine<OP>(acc[w], extend<S, ES, SGN>(elem_of<ES, 4>(q, w), sgn));
                     }
                 } else {
                     const int nw = (int)umin64((uint64_t)W, cols - c0);
                     for (uint64_t r = r0 + ri; r < r1; r += (uint64_t)rl)
 #pragma unroll
                         for (int w = 0; w < W; ++w)
-                            if (w < nw) acc[w] = combine<OP>(acc[w], extend<S, ES>(ld_elem<ES>(colp + r * pitch + (uint64_t)w * ES), sgn));
+                            if (w < nw) acc[w] = combine<OP>(acc[w], extend<S, ES, SGN>(ld_elem<ES>(colp + r * pitch + (uint64_t)w * ES), sgn));
                 }
             }
             __syncthreads();  // part[] is free again
@@ -250,23 +272,29 @@ k_fold_split(const __grid_constant__ FoldSplitPlan F, void* __restrict__ out, un
 
 using SplitKernel = void (*)(const FoldSplitPlan, void*, unsigned int*, void*, uint64_t, uint32_t);
 
-template <class S, int ES, int OP>
+template <class S, int ES, int OP, bool SGN>
 SplitKernel pick_layout(int layout) {
-    return layout == SPLIT_RUNS ? k_fold_split<S, ES, OP, SPLIT_RUNS> : k_fold_split<S, ES, OP, SPLIT_COLS>;
+    return layout == SPLIT_RUNS ? k_fold_split<S, ES, OP, SPLIT_RUNS, SGN> : k_fold_split<S, ES, OP, SPLIT_COLS, SGN>;
 }
-template <class S, int ES>
+template <class S, int ES, bool SGN = false>
 SplitKernel pick_op(int op, int layout) {
     switch (op) {
-        case SOP_MUL: return pick_layout<S, ES, SOP_MUL>(layout);
-        case SOP_AND: return pick_layout<S, ES, SOP_AND>(layout);
-        case SOP_OR: return pick_layout<S, ES, SOP_OR>(layout);
-        case SOP_XOR: return pick_layout<S, ES, SOP_XOR>(layout);
-        default: return pick_layout<S, ES, SOP_ADD>(layout);
+        case SOP_MUL: return pick_layout<S, ES, SOP_MUL, SGN>(layout);
+        case SOP_AND: return pick_layout<S, ES, SOP_AND, SGN>(layout);
+        case SOP_OR: return pick_layout<S, ES, SOP_OR, SGN>(layout);
+        case SOP_XOR: return pick_layout<S, ES, SOP_XOR, SGN>(layout);
+        default: return pick_layout<S, ES, SOP_ADD, SGN>(layout);
     }
 }
 template <class S>
-SplitKernel pick_src(int es, int op, int layout) {
-    return es == 1 ? pick_op<S, 1>(op, layout) : es == 4 ? pick_op<S, 4>(op, layout) : pick_op<S, 8>(op, layout);
+SplitKernel pick_src(int src_dtype, int op, int layout) {
+    const bool sgn = is_signed(src_dtype);
+    switch (dtype_size(src_dtype)) {
+        case 1: return sgn ? pick_op<S, 1, true>(op, layout) : pick_op<S, 1>(op, layout);
+        case 2: return sgn ? pick_op<S, 2, true>(op, layout) : pick_op<S, 2>(op, layout);
+        case 4: return pick_op<S, 4>(op, layout);
+        default: return pick_op<S, 8>(op, layout);
+    }
 }
 
 }  // namespace
@@ -314,7 +342,7 @@ const char* launch_fold_split(const Plan& p, void* out, bool nowait, cudaStream_
     const SplitGeometry G = fold_split_geometry(F, sm_count);
     const int op = F.op == MDIM_MUL ? SOP_MUL : F.op == MDIM_AND ? SOP_AND : F.op == MDIM_OR ? SOP_OR : F.op == MDIM_XOR ? SOP_XOR : SOP_ADD;
     const int es = dtype_size(F.src_dtype);
-    const SplitKernel k = F.slot_bytes == 8 ? pick_src<unsigned long long>(es, op, F.layout) : pick_src<unsigned int>(es, op, F.layout);
+    const SplitKernel k = F.slot_bytes == 8 ? pick_src<unsigned long long>(F.src_dtype, op, F.layout) : pick_src<unsigned int>(F.src_dtype, op, F.layout);
     const cudaError_t e = launch_pdl(k, dim3((unsigned)(G.units * G.n_chunks)), dim3(kSplitThreads), 0, stream, F, out, (unsigned int*)scratch,
                                      (void*)(scratch + kSplitMaxOuts * sizeof(unsigned int)), (uint64_t)G.chunk, (uint32_t)G.n_chunks);
     if (e != cudaSuccess) return nullptr;

@@ -109,7 +109,7 @@ __global__ void __launch_bounds__(kXThreads, EXCHANGE ? 4 : 6) k_fold_xchg(const
     do {                                                                                                       \
         S v[EPT];                                                                                              \
         unpack<S>(x[u], v);                                                                                    \
-        _Pragma("unroll") for (int e = 0; e < EPT; ++e) { bool arith = false; acc[e] = bin_op<S>(DT, OP, DT, acc[e], v[e], arith); } \
+        _Pragma("unroll") for (int e = 0; e < EPT; ++e) { bool arith = false; acc[e] = bin_op<S, false>(DT, OP, DT, acc[e], v[e], arith); } \
     } while (0)
 #pragma unroll
             for (int u = 0; u < ROWS; ++u) MDIM_LOAD_ROW(u, (uint64_t)u);
@@ -136,7 +136,7 @@ __global__ void __launch_bounds__(kXThreads, EXCHANGE ? 4 : 6) k_fold_xchg(const
             S v[EPT];
             unpack<S>(x, v);
 #pragma unroll
-            for (int e = 0; e < EPT; ++e) { bool arith = false; acc[e] = bin_op<S>(DT, OP, DT, acc[e], v[e], arith); }
+            for (int e = 0; e < EPT; ++e) { bool arith = false; acc[e] = bin_op<S, false>(DT, OP, DT, acc[e], v[e], arith); }
         }
         // ---- exchange.  Two ranks: everybody sends to everybody and combines (one hop).  More: the columns have an OWNER (warp-
         //      granular, round robin) that collects the partial values, combines them in rank order and sends the result to
@@ -208,7 +208,7 @@ __global__ void __launch_bounds__(kXThreads, EXCHANGE ? 4 : 6) k_fold_xchg(const
 #pragma unroll
                     for (int e = 0; e < EPT; ++e) {
                         bool arith = false;
-                        tot[e] = q == 0 ? v[e] : bin_op<S>(DT, OP, DT, tot[e], v[e], arith);
+                        tot[e] = q == 0 ? v[e] : bin_op<S, false>(DT, OP, DT, tot[e], v[e], arith);
                     }
                 }
             if (!one_shot) {  // the result goes to everybody else's result area

@@ -20,15 +20,6 @@
 
 namespace mdim {
 
-int dtype_size(int dt) {
-    switch (dt) {
-        case MDIM_U8: return 1;
-        case MDIM_I32: case MDIM_U32: case MDIM_F32: return 4;
-        case MDIM_I64: case MDIM_U64: case MDIM_F64: return 8;
-    }
-    return 0;
-}
-
 const char* status_string(int st) {
     switch (st) {
         case MDIM_OK: return "ok";
@@ -44,7 +35,6 @@ const char* status_string(int st) {
     return "unknown status";
 }
 
-static bool is_int(int dt) { return dt == MDIM_U8 || dt == MDIM_I32 || dt == MDIM_U32 || dt == MDIM_I64 || dt == MDIM_U64; }
 static bool is_float(int dt) { return dt == MDIM_F32 || dt == MDIM_F64; }
 
 static int node_arity(const mdim_node& n) {
@@ -446,8 +436,7 @@ int Builder::gen(int ni, int mask_first, int mask_n) {
         }
         case MDIM_NODE_CONST:
             in.opc = OPC_CONST; in.imm = n.imm.u64;
-            if (dtype_size(n.dtype) == 4) in.imm &= 0xffffffffull;
-            if (dtype_size(n.dtype) == 1) in.imm &= 0xffull;
+            if (dtype_size(n.dtype) < 8) in.imm &= (1ull << (8 * dtype_size(n.dtype))) - 1;
             return push_instr(in);
         case MDIM_NODE_UNARY: {
             int st = gen(child[ni][0], mask_first, mask_n); if (st) return st;
@@ -489,8 +478,7 @@ int Builder::gen(int ni, int mask_first, int mask_n) {
             }
             int st = gen(child[ni][0], r0, mask_n + own_n); if (st) return st;
             in.opc = OPC_SELECT; in.slot = (uint16_t)own0; in.n = (uint16_t)own_n; in.imm = n.imm.u64;
-            if (dtype_size(n.dtype) == 4) in.imm &= 0xffffffffull;
-            if (dtype_size(n.dtype) == 1) in.imm &= 0xffull;
+            if (dtype_size(n.dtype) < 8) in.imm &= (1ull << (8 * dtype_size(n.dtype))) - 1;
             st = push_instr(in); if (st) return st;
             if (lazy) {
                 Instr m; memset(&m, 0, sizeof m);
@@ -552,8 +540,7 @@ int Builder::gen(int ni, int mask_first, int mask_n) {
                 in.aux = 1;
             }
             in.opc = OPC_FOLD_BEGIN; in.imm = n.imm.u64;
-            if (dtype_size(n.dtype) == 4) in.imm &= 0xffffffffull;
-            if (dtype_size(n.dtype) == 1) in.imm &= 0xffull;
+            if (dtype_size(n.dtype) < 8) in.imm &= (1ull << (8 * dtype_size(n.dtype))) - 1;
             int st = push_instr(in); if (st) return st;
             const int begin_pc = P.n_instr - 1;
             const int body_pc = P.n_instr;
@@ -862,7 +849,7 @@ bool Builder::detect_fold_split() {
         S.cols = len[rank - 1]; S.pitch = rstride;
         S.n_batch = rank == 2 ? len[0] : 1; S.batch_stride = rank == 2 ? s[0] : 0;
     } else return false;
-    static const char* const dt_name[] = {"u8", "i32", "u32", "i64", "u64"};
+    static const char* const dt_name[MDIM_DTYPE_COUNT] = {"u8", "i32", "u32", "i64", "u64", "f32", "f64", "i8", "i16", "u16"};
     plan->kind = KK_FOLD_SPLIT;
     snprintf(plan->describe, sizeof plan->describe, "fold_split.%s outs=%llu red=%llu slot=s%d src=%s op=%d", S.layout == SPLIT_RUNS ? "runs" : "cols",
              (unsigned long long)n_out, (unsigned long long)red, S.slot_bytes * 8, dt_name[S.src_dtype], S.op);

@@ -20,6 +20,24 @@ constexpr int kMaxPred = 16;
 constexpr int kMaxComp = 4;
 constexpr int kMaxDepth = 8;  // deepest value stack any instantiation supports
 
+#if defined(__CUDACC__)
+#define MDIM_HD __host__ __device__
+#else
+#define MDIM_HD
+#endif
+// Element type facts, shared by the planner, the evaluator and the dedicated kernels.
+MDIM_HD constexpr int dtype_size(int dt) {
+    switch (dt) {
+        case MDIM_U8: case MDIM_I8: return 1;
+        case MDIM_I16: case MDIM_U16: return 2;
+        case MDIM_I32: case MDIM_U32: case MDIM_F32: return 4;
+        case MDIM_I64: case MDIM_U64: case MDIM_F64: return 8;
+    }
+    return 0;
+}
+MDIM_HD constexpr bool is_int(int dt) { return dtype_size(dt) != 0 && dt != MDIM_F32 && dt != MDIM_F64; }
+MDIM_HD constexpr bool is_signed(int dt) { return dt == MDIM_I8 || dt == MDIM_I16 || dt == MDIM_I32 || dt == MDIM_I64; }
+
 enum Opc : uint8_t {
     OPC_LEAF_VEC = 0,   // contiguous along the vector axis, aligned: 128-bit loads
     OPC_LEAF_BCAST,     // stride 0 along the vector axis: one scalar load, replicated
@@ -199,7 +217,7 @@ struct FoldSplitPlan {
                             // SPLIT_COLS: each output is a column; `cols` contiguous columns per row, rows `pitch` apart
     int32_t op;             // MDIM_ADD, SUB, MUL, AND, OR, XOR
     int32_t dtype, src_dtype;  // the fold's dtype; the leaf's (a CAST body converts between them)
-    int32_t slot_bytes;     // 4 or 8: the accumulator width (the fold's dtype, U8 widened to 4)
+    int32_t slot_bytes;     // 4 or 8: the accumulator width (the fold's dtype, 1- and 2-byte types widened to 4)
     int32_t nowait;         // set per launch by its launcher: see launch.cuh
     uint64_t init;          // bits of the immediate init
     uint64_t red;           // RUNS: elements per run; COLS: rows
@@ -283,7 +301,6 @@ int plan_expr(const mdim_expr* e, uint32_t flags, Plan* plan, char* why, size_t 
 // plan_expr for a collect into the output runs outs[0 .. n_outs) (one per scalar leaf of a TUPLE root, else one): checks each run
 // (not null, aligned to its element), plans again with scalar stores when a run is only element-aligned, and fills out_more[]
 int plan_collect(const mdim_expr* e, uint32_t flags, void* const* outs, int n_outs, Plan* plan, char* why, size_t why_len);
-int dtype_size(int dt);
 const char* status_string(int st);
 // mdim_error_info for a device-side failure at output position `pos`, from the error word of its PF_EXPLAIN rerun
 void explain_failure(const ErrWord& w, uint64_t pos, mdim_error_info* info);

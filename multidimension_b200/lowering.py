@@ -183,7 +183,7 @@ def rename(table):
 
 
 # ---- packing immediates -----------------------------------------------------------------------
-_PACK = {F.U8: "<B", F.I32: "<i", F.U32: "<I", F.I64: "<q", F.U64: "<Q", F.F32: "<f", F.F64: "<d"}
+_PACK = {F.U8: "<B", F.I32: "<i", F.U32: "<I", F.I64: "<q", F.U64: "<Q", F.F32: "<f", F.F64: "<d", F.I8: "<b", F.I16: "<h", F.U16: "<H"}
 
 
 def imm_bits(dtype, value):

@@ -13,7 +13,8 @@ import numpy as np
 
 from . import _ffi as F
 
-NP_OF = {F.U8: np.uint8, F.I32: np.int32, F.U32: np.uint32, F.I64: np.int64, F.U64: np.uint64, F.F32: np.float32, F.F64: np.float64}
+NP_OF = {F.U8: np.uint8, F.I32: np.int32, F.U32: np.uint32, F.I64: np.int64, F.U64: np.uint64, F.F32: np.float32, F.F64: np.float64,
+         F.I8: np.int8, F.I16: np.int16, F.U16: np.uint16}
 
 
 class Context:

@@ -21,9 +21,11 @@ Panic = F.Panic
 Unsupported = L.Unsupported
 
 # ---- element types ------------------------------------------------------------------------------
-_DT_OF_NAME = {"u8": F.U8, "i32": F.I32, "u32": F.U32, "i64": F.I64, "u64": F.U64, "f32": F.F32, "f64": F.F64}
+_DT_OF_NAME = {"u8": F.U8, "i32": F.I32, "u32": F.U32, "i64": F.I64, "u64": F.U64, "f32": F.F32, "f64": F.F64,
+               "i8": F.I8, "i16": F.I16, "u16": F.U16}
 _NAME_OF_NP = {np.dtype(np.uint8): "u8", np.dtype(np.int32): "i32", np.dtype(np.uint32): "u32", np.dtype(np.int64): "i64",
-               np.dtype(np.uint64): usize, np.dtype(np.float32): "f32", np.dtype(np.float64): "f64", np.dtype(np.bool_): bool}
+               np.dtype(np.uint64): usize, np.dtype(np.float32): "f32", np.dtype(np.float64): "f64", np.dtype(np.bool_): bool,
+               np.dtype(np.int8): "i8", np.dtype(np.int16): "i16", np.dtype(np.uint16): "u16"}
 
 
 def dtype_of(T):

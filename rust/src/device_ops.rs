@@ -24,6 +24,7 @@ device_elem! {
     u8 => ffi::U8, |x: u8| x as u64;   i32 => ffi::I32, |x: i32| x as u32 as u64;   u32 => ffi::U32, |x: u32| x as u64;
     i64 => ffi::I64, |x: i64| x as u64;   u64 => ffi::U64, |x: u64| x;   usize => ffi::U64, |x: usize| x as u64;
     f32 => ffi::F32, |x: f32| x.to_bits() as u64;   f64 => ffi::F64, |x: f64| x.to_bits();
+    i8 => ffi::I8, |x: i8| x as u8 as u64;   i16 => ffi::I16, |x: i16| x as u16 as u64;   u16 => ffi::U16, |x: u16| x as u64;
 }
 impl DeviceElem for bool { const DTYPE: i32 = ffi::U8; const IS_BOOL: bool = true; fn bits(self) -> u64 { self as u64 } }
 

@@ -26,6 +26,7 @@ pub const MDIM_ERR_NCCL: i32 = 8;
 // mdim_dtype (usize = U64, bool = U8)
 pub const U8: i32 = 0; pub const I32: i32 = 1; pub const U32: i32 = 2; pub const I64: i32 = 3;
 pub const U64: i32 = 4; pub const F32: i32 = 5; pub const F64: i32 = 6;
+pub const I8: i32 = 7; pub const I16: i32 = 8; pub const U16: i32 = 9;
 // mdim_binary_op = the enums of src/ops.rs:23-129
 pub const ADD: i32 = 0; pub const SUB: i32 = 1; pub const MUL: i32 = 2; pub const DIV: i32 = 3; pub const REM: i32 = 4;
 pub const AND: i32 = 5; pub const OR: i32 = 6; pub const XOR: i32 = 7; pub const SHL: i32 = 8; pub const SHR: i32 = 9;
@@ -39,7 +40,7 @@ pub const DIAG: i32 = 5; pub const GATHER: i32 = 6; pub const FOLD: i32 = 7; pub
 pub const COLLECT_ASYNC: u32 = 1; pub const COLLECT_NO_FASTPATH: u32 = 2; pub const COLLECT_NO_STATIC: u32 = 4; pub const COLLECT_NO_JIT: u32 = 8;
 
 #[repr(C)] #[derive(Copy, Clone)]
-pub union MdimScalar { pub u64_: u64, pub i64_: i64, pub f64_: f64, pub f32_: f32, pub u32_: u32, pub i32_: i32, pub u8_: u8 }
+pub union MdimScalar { pub u64_: u64, pub i64_: i64, pub f64_: f64, pub f32_: f32, pub u32_: u32, pub i32_: i32, pub u8_: u8, pub i8_: i8, pub i16_: i16, pub u16_: u16 }
 
 #[repr(C)] #[derive(Copy, Clone)]
 pub struct MdimNode {
